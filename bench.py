@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path (N>1: under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference algorithm on the host CPU
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's results as DIR/<name>.npy
 
 Workload (BASELINE.json configs[2], the largest single-GPU configuration): 360-node synthetic
 Watts-Strogatz connectomes, batch 4096 subjects per GPU, hidden 64, 3 layers, dropout 0.3.
@@ -23,6 +24,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "connectome-gnn-suite_b200")):
     if _p not in sys.path:
@@ -58,10 +60,17 @@ def parse():
     ap.add_argument("--no-peer-collectives", action="store_true",
                     help="N > 1: SyncBN statistics through NCCL collectives instead of the peer-memory exchange kernel (A/B)")
     ap.add_argument("--dp-per-rank", type=int, default=48, help="subjects per rank in the data-parallel parity step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (losses, correct counts, trained parameters, their "
+                         "gradients and BatchNorm statistics) as DIR/<name>.npy, rank 0 only")
     a = ap.parse_args()
     a.legs = tuple(x for x in a.legs.split(",") if x)
     if not a.legs or any(x not in LEGS for x in a.legs):
         ap.error(f"--legs takes a subset of {LEGS}")
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the sm_100a arm (--impl b200)")
     return a
 
 
@@ -186,7 +195,7 @@ PKG_DIR = os.path.join(ROOT, "connectome-gnn-suite_b200")
 
 
 def reference_legs(a, steps, warmup):
-    """Times the UNMODIFIED reference (oracle/_ref, copied from /root/reference by oracle/make_ref.py): its own
+    """Times the UNMODIFIED reference (oracle/_ref, copied from a checkout of it by oracle/make_ref.py): its own
     generate_dataset, ConnectomeDataLoader, GCNConnectome / GraphSAGEConnectome and Trainer.train_epoch / evaluate on the
     host cores, one batch of `cpu_sample` subjects per leg and step.  Only called in a process that has not imported
     this repo's package (the two share the name `connectome_gnn`)."""
@@ -333,19 +342,22 @@ def run_b200(a):
     order_gen = torch.Generator().manual_seed(99 + rank)
 
     def leg(name, st):
+        """What the step hands its caller: (loss,) for training, (loss, correct count) for inference."""
         kind, mode = name.split("_")
         tr = trainers[kind]
         ids = torch.randperm(a.batch, generator=order_gen).numpy()
         batch = st.collate(ids, prepare_for=kind, backward=(mode == "train"), **meta)
         if mode == "train":
             tr.model.train()
-            return tr.train_step(batch)
+            return (tr.train_step(batch),)
         tr.model.eval()
-        return tr.eval_step(batch)[0]
+        return tr.eval_step(batch)
+
+    last = {}   # the latest resident step's results per leg (--dump-outputs)
 
     def step_resident():
         for name in a.legs:
-            leg(name, store)
+            last[name] = leg(name, store)
 
     streaming = StreamingStore(pinned, dev, depth=3)
     streaming.prefetch(pinned)   # primes the pipeline (two sets ahead) once, before any timed region
@@ -359,7 +371,7 @@ def run_b200(a):
         for name in a.legs:
             st = streaming.next()
             streaming.prefetch(pinned)
-            losses.append(leg(name, st).reshape(()))
+            losses.append(leg(name, st)[0].reshape(()))
             st.release()                             # the arena may be refilled once this leg's kernels have run
         return torch.stack(losses).cpu().tolist()    # the step's four losses read back to the host
 
@@ -398,6 +410,8 @@ def run_b200(a):
     launches = lib.cgnn_kernel_launches() - launches0
     graphs_per_step = len(a.legs) * a.batch * world
     value = graphs_per_step * a.steps / (ms / 1e3)
+    if a.dump_outputs is not None and rank == 0:   # before anything else runs a step: the models hold its results
+        dump_outputs(a.dump_outputs, last, trainers)
 
     # ---- per-leg device time (CUDA events on the launching stream) -------------------------------------
     leg_ms = {}
@@ -474,6 +488,46 @@ def run_b200(a):
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BUDGET = 60 << 20   # bytes of array data: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, last, trainers, budget=DUMP_BUDGET):
+    """Write what the last timed step handed its caller as ``out_dir/<name>.npy``: per leg its loss (inference legs also
+    the argmax-correct count), and for every training leg the model as the step left it - ``state_dict`` entries
+    (parameters, BatchNorm running statistics) and parameter gradients.  Floating tensors keep their dtype, integers
+    become float64.  Above ``budget`` bytes in all, every array is cut to the same fraction of its entries, chosen by a
+    fixed seed, so that two builds run with the same arguments still compare entry for entry."""
+    arrays = {}
+    for name, out in last.items():
+        kind, mode = name.split("_")
+        arrays[f"{name}.loss"] = out[0]
+        if mode == "infer":
+            arrays[f"{name}.correct"] = out[1]
+            continue
+        model = trainers[kind].model
+        for k, v in model.state_dict().items():
+            arrays[f"{name}.{k}"] = v
+        for k, p in model.named_parameters():
+            if p.grad is not None:
+                arrays[f"{name}.grad.{k}"] = p.grad
+    host = {}
+    for k, v in arrays.items():
+        v = v.detach().cpu()
+        host[k] = v.numpy() if v.dtype in (torch.float32, torch.float64) else v.double().numpy()
+    total = sum(v.nbytes for v in host.values())
+    if total > budget:
+        rng = np.random.default_rng(0)
+        for k, v in host.items():
+            keep = max(1, v.size * budget // total)
+            if keep < v.size:
+                host[k] = v.reshape(-1)[np.sort(rng.choice(v.size, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    print(f"bench.py: {len(host)} arrays ({sum(v.nbytes for v in host.values()) / 1e6:.2f} MB) written to {out_dir}",
+          file=sys.stderr)
 
 
 def eager_step_only(a, graphs, dev, subjects=2048):

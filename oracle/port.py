@@ -3,7 +3,7 @@
 Nothing under ``connectome-gnn-suite_b200/`` imports this module.  It is used by ``tests/``
 (as the checker), by ``__graft_entry__.smoke()`` (as the checker) and by ``bench.py`` for the
 ``cpu_baseline`` leg / ``--impl reference`` arm (as the thing timed on the host cores, because the
-Python reference under /root/reference cannot travel to the GPU box).
+Python reference itself is not part of this repository).
 
 What it restates (danieleschmidt/connectome-gnn-suite, all arithmetic delegated - like the
 reference - to PyTorch 2.11 CPU ATen kernels, the reference's un-pinned ``torch>=2.0`` dependency):
@@ -19,7 +19,7 @@ reference - to PyTorch 2.11 CPU ATen kernels, the reference's un-pinned ``torch>
 Parity is PINNED: ``tests/test_oracle.py`` checks every function here against fixtures produced
 by importing the unmodified reference (``tests/golden/make_golden.py``, outputs committed under
 ``tests/golden/``) - bit-exact for collate / degrees and for every float tensor (same op sequence
-on the same ATen build), and, when /root/reference is present, against the live reference.
+on the same ATen build), and, when CGNN_REFERENCE names a checkout of it, against the live reference.
 
 Parameters are plain ``dict[str, Tensor]`` with the reference's ``state_dict`` keys
 (``convs.i.linear.weight``, ``convs.i.bias`` | ``convs.i.linear.bias``,

@@ -1,11 +1,11 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures in this directory FROM THE UNMODIFIED REFERENCE.
 
-Run in the build container (the reference tree does not exist on the GPU box):
+Run with a checkout of the reference first on the import path:
 
-    PYTHONDONTWRITEBYTECODE=1 PYTHONPATH=/root/reference python tests/golden/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 PYTHONPATH=<reference checkout> python tests/golden/make_golden.py
 
-It imports ``connectome_gnn`` from /root/reference (never the package in this repo), runs the
+It imports ``connectome_gnn`` from that checkout (never the package in this repo), runs the
 reference's own collate / models / Trainer on seeded synthetic inputs and stores inputs + outputs
 as small ``.npz`` / ``.json`` files.  The oracle (``oracle/``) is pinned against these files by
 ``tests/test_oracle.py``; the CUDA path is compared against them (and the oracle) by the
@@ -24,7 +24,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 import connectome_gnn  # noqa: E402  (must resolve to the reference)
 
-assert "/root/reference" in os.path.abspath(connectome_gnn.__file__), connectome_gnn.__file__
+# this package (in this tree or installed anywhere) sets BACKEND; the reference has no such attribute
+assert not hasattr(connectome_gnn, "BACKEND"), f"{connectome_gnn.__file__} is this package, not the reference"
 from connectome_gnn.graph import ConnectomeDataLoader, ConnectomeGraph, collate_graphs  # noqa: E402
 from connectome_gnn.models import GCNConnectome, GraphSAGEConnectome  # noqa: E402
 from connectome_gnn.synthetic import REGION_NAMES, generate_connectome, generate_dataset  # noqa: E402

@@ -23,6 +23,7 @@ from oracle import port
 META = json.load(open(os.path.join(helpers.GOLDEN, "ref_meta.json")))
 SAME_BUILD = torch.__version__ == META["made_with"]["torch"]
 FIXTURES = ["ref_small.npz", "ref_ragged.npz", "ref_c1.npz", "ref_c3.npz", "ref_c5.npz"]
+REFERENCE = os.environ.get("CGNN_REFERENCE", "")   # optional checkout of the reference, for the live comparison
 
 
 @pytest.fixture(autouse=True)
@@ -221,13 +222,14 @@ def test_generator_matches_reference_fingerprints():
             (ref["edge_index"], ref["node_features"], ref["label"], ref["subject_id"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/connectome_gnn"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "connectome_gnn"))),
+                    reason="needs CGNN_REFERENCE: a checkout of the reference, which is not part of this repository")
 def test_oracle_against_live_reference():
     """Run the reference itself (separate process: it shares the import name with the package) on a fresh
     random case and compare the port on the same inputs."""
     code = r'''
 import sys, json, torch, numpy as np
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, sys.argv[1])
 from connectome_gnn.synthetic import generate_dataset
 from connectome_gnn.graph import collate_graphs
 from connectome_gnn.models import GCNConnectome, GraphSAGEConnectome
@@ -241,7 +243,7 @@ for kind, cls in (("gcn", GCNConnectome), ("sage", GraphSAGEConnectome)):
                  "grads": {k: p.grad.tolist() for k, p in m.named_parameters()}}
 print(json.dumps(out))
 '''
-    res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, check=True,
+    res = subprocess.run([sys.executable, "-c", code, REFERENCE], capture_output=True, text=True, check=True,
                          env={**os.environ, "PYTHONDONTWRITEBYTECODE": "1", "PYTHONPATH": ""})
     ref = json.loads(res.stdout)
     from connectome_gnn.synthetic import generate_dataset
