@@ -106,9 +106,11 @@ class Engine:
 
     # -- K0 ---------------------------------------------------------------------------------
     def new_csr(self, rows: int, edges: int, graphs: int) -> dict:
-        e = self.empty
+        # a batch without a single edge still gets one (unused) element per edge array: the C side reads a NULL array as
+        # "not materialised" (a lean batch), and the data_ptr() of an empty tensor - even a view - is NULL
+        e = lambda n, dtype=torch.float32: self.empty(max(n, 1), dtype)
         return dict(
-            graph_meta=e((graphs, 4), torch.int32),
+            graph_meta=self.empty((graphs, 4), torch.int32),
             in_rowptr=e(rows + 1, torch.int32), in_col=e(edges, torch.int32), in_w=e(edges), in_wn=e(edges),
             out_rowptr=e(rows + 1, torch.int32), out_col=e(edges, torch.int32), out_w=e(edges), out_wn=e(edges),
             deg=e(rows), dinv=e(rows), wsum=e(rows))
