@@ -114,11 +114,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
   rt::ChanQuad cq;
   rt::chan_quad_init(cq, p.act, c0, C);
   const rt::RowKey rk = rt::row_key(p.act);
-  rt::BnBwdDev bn;
-  bn.scale = p.bn_scale; bn.mean = p.bn_mean; bn.rstd = p.bn_rstd; bn.s1 = p.bn_s1; bn.s2 = p.bn_s2; bn.sums64 = p.bn_sums64;
-  bn.inv_count = p.inv_count; bn.train = p.bn_train; bn.has = p.has_bn;
   rt::BnQuad bq;
-  if (MODE == GATHER_GCN_BWD) rt::bn_quad_init(bq, bn, c0, C);
+  if (MODE == GATHER_GCN_BWD) rt::bn_quad_init(bq, p.bn, c0, C);
   float pmean[4] = {0.f, 0.f, 0.f, 0.f}, prstd[4] = {0.f, 0.f, 0.f, 0.f};
   if (MODE == GATHER_SAGE_BWD && p.want_prev) {
 #pragma unroll
@@ -171,7 +168,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
           float4 o = a[u];
           if (MODE == GATHER_SAGE_FWD || MODE == GATHER_GCN_FWD) o = rt::act_fwd4(p.act, cq, a[u], rk, (uint32_t)(nb + rr));
           if (MODE == GATHER_GCN_BWD) {
-            o = rt::bn_bwd4(bn, bq, a[u], rt::act_bwd4(p.act, cq, a[u], b[MODE == GATHER_GCN_BWD ? u : 0], rk, (uint32_t)(nb + rr)));
+            o = rt::bn_bwd4(p.bn, bq, a[u], rt::act_bwd4(p.act, cq, a[u], b[MODE == GATHER_GCN_BWD ? u : 0], rk, (uint32_t)(nb + rr)));
             if (!VEC) o = rt::mask_quad(o, c0, C);
             s1[0] += o.x; s1[1] += o.y; s1[2] += o.z; s1[3] += o.w;
           }
@@ -249,8 +246,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
   (void)RP;
 }
 
-#endif  // CGNN_EMU
-
 // ---- host side -------------------------------------------------------------------------------------------------
 static bool gather_shape(int C, int max_nodes, int max_edges, int* lpr, int* nslab, size_t* smem) {
   if (C <= 0 || C > 256) return false;
@@ -272,15 +267,11 @@ bool gather_supported(int C, int max_nodes, int max_edges) {
 
 // Launches one gather kernel; returns the grid through *grid_out (the caller reduces `partials` over it).
 int launch_gather(int mode, GatherArgs& a, int* grid_out, cudaStream_t stream) {
-#ifdef CGNN_EMU
-  (void)mode; (void)a; (void)grid_out; (void)stream;
-  return -1;
-#else
   const DeviceInfo dev = device_info();
   int LPR = 0, nslab = 0;
   size_t smem = 0;
   if (a.max_nodes < 1) a.max_nodes = 1;
-  if (!gather_shape(a.C, a.max_nodes, a.max_edges, &LPR, &nslab, &smem)) return -1;
+  if (!gather_shape(a.C, a.max_nodes, a.max_edges, &LPR, &nslab, &smem)) return CGNN_ERR_INVALID_ARG;
   a.nslab = nslab;
   const int C = a.C;
   auto al16 = [](const void* p) { return p == nullptr || (((uintptr_t)p) & 15u) == 0; };
@@ -312,8 +303,9 @@ int launch_gather(int mode, GatherArgs& a, int* grid_out, cudaStream_t stream) {
 #undef CGNN_GATHER
   CGNN_CHECK_LAUNCH();
   return CGNN_OK;
-#endif
 }
+
+#endif  // CGNN_EMU
 
 int launch_build_agg(const cgnn_csr_t* csr, int32_t kind, int64_t num_graphs, int32_t max_nodes, int32_t* agg_in, int32_t* agg_out,
                      int32_t* row_graph, int skip_edge_cap, cudaStream_t stream) {

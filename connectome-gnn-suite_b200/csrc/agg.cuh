@@ -141,8 +141,7 @@ struct GatherArgs {
   const float* src;        // SAGE_FWD / GCN_FWD: t_in   GCN_BWD: z   SAGE_BWD: d_agg
   Act act;                 // SAGE_FWD: act on load   GCN_BWD: act_out (its backward)   SAGE_BWD: act_in (for the sums)
   const float* du; const float* demb;                                    // GCN_BWD upstream
-  const float* bn_scale; const float* bn_mean; const float* bn_rstd; const float* bn_s1; const float* bn_s2; const double* bn_sums64;
-  float inv_count; int bn_train, has_bn;
+  BnBwdDev bn;
   // SAGE_BWD
   const float* direct;     // d_u [rows, C]
   const float* t_raw;      // this layer's stored input (for the sums of the layer below)
@@ -152,10 +151,11 @@ struct GatherArgs {
   float* partials; int part_stride;   // GCN_BWD: dbias [C]; SAGE_BWD: prev sums [2C]
 };
 
+// Launchers.  A path that launches one kernel asks its launcher directly: -1 = not covered, nothing was launched (the
+// caller tries the next path), > 0 = an error.  A path of several kernels settles the coverage of all of them before the
+// first launch, through the *_supported predicate next to each later launcher; those launchers only return CGNN_OK or
+// an error.
 
-// agg.cu: one gather kernel; CGNN_OK when launched (grid in *grid_out: the caller reduces `partials` over it),
-// -1 when the shape is not covered.
-int launch_gather(int mode, GatherArgs& a, int* grid_out, cudaStream_t stream);
 // engine.cu: warp-specialised hidden-layer forward (64 -> 64 channels; also built for the simulator)
 int launch_gcn_fwd_ws(const float* t_in, const cgnn_act_t* act, const float* W, const float* bias, const cgnn_csr_t* csr,
                       int64_t num_graphs, int64_t rows, int32_t d_in, int32_t H, int32_t max_nodes, int32_t max_edges, float* z,
@@ -165,10 +165,21 @@ int launch_gcn_fwd_ws_pool(const float* t_in, const cgnn_act_t* act, const float
                            int64_t num_graphs, int64_t rows, int32_t d_in, int32_t H, int32_t max_nodes, int32_t max_edges,
                            const cgnn_act_t* act_out, float* emb, cudaStream_t stream);
 #ifndef CGNN_EMU
-// gemm_tc.cu: tensor-core contractions; same return convention.
+// agg.cu: one gather kernel (grid in *grid_out: the caller reduces `partials` over it), for C channels when
+// gather_supported(C, ...)
+bool gather_supported(int C, int max_nodes, int max_edges);
+int launch_gather(int mode, GatherArgs& a, int* grid_out, cudaStream_t stream);
+// gemm_tc.cu: tensor-core contractions.  The GraphSAGE forward and GCN backward ones run after a gather, when their
+// predicate holds for the same arguments (`shape`: where the launcher takes its launch shape from); the GraphSAGE
+// backward one runs first (-1 when not covered).
+struct GemmShape;
+bool sage_fwd_gemm_supported(const float* t_in, const float* agg, const float* z, int64_t rows, int32_t C, int32_t H,
+                             bool want_stats, size_t workspace_bytes, GemmShape* shape = nullptr);
 int launch_sage_fwd_gemm(const float* t_in, const cgnn_act_t* act, const float* agg, const float* W, const float* bias,
                          int64_t rows, int32_t C, int32_t H, float* z, double* partials, int* grid_out,
                          size_t workspace_bytes, cudaStream_t stream);
+bool gcn_bwd_gemm_supported(const float* dP, const float* t_in, const float* du_in, int64_t rows, int32_t d_in, int32_t H,
+                            int part_stride, size_t partial_bytes, GemmShape* shape = nullptr);
 int launch_gcn_bwd_gemm(const float* dP, const float* t_in, const cgnn_act_t* act_in, const float* W, int64_t rows,
                         int32_t d_in, int32_t H, float* du_in, const float* prev_mean, const float* prev_rstd, int want_prev,
                         float* partials, int part_stride, int o_pprev, int* grid_out, size_t partial_bytes,
@@ -209,7 +220,5 @@ int launch_gcn_bwd_wide(const float* du, const float* demb, const float* z, cons
 // agg.cu: blob builder; subjects with <= skip_edge_cap edges (and < 65536 rows) are skipped (built by the collate kernel)
 int launch_build_agg(const cgnn_csr_t* csr, int32_t kind, int64_t num_graphs, int32_t max_nodes, int32_t* agg_in, int32_t* agg_out,
                      int32_t* row_graph, int skip_edge_cap, cudaStream_t stream);
-// true when launch_gather covers C channels (checked before a tensor-core contraction commits to the gather that follows)
-bool gather_supported(int C, int max_nodes, int max_edges);
 
 }  // namespace cgnn

@@ -97,6 +97,28 @@ static inline Act make_act(const cgnn_act_t* a) {
   return r;
 }
 
+// ---- BatchNorm backward: dz = scale * (dy - s1 / count - xhat * s2 / count), xhat = (t - mean) * rstd -----------------
+// Device-side form of cgnn_bn_bwd_t (has = 0: no BatchNorm after this layer).
+struct BnBwdDev {
+  const float* scale; const float* mean; const float* rstd; const float* s1; const float* s2;
+  float inv_count; int train, has;
+  const double* sums64;     // [2, C] in double, read instead of s1 / s2 when given
+};
+
+static inline BnBwdDev make_bn_bwd(const cgnn_bn_bwd_t* bn) {
+  BnBwdDev r{};
+  if (!bn) return r;
+  r.scale = bn->scale; r.mean = bn->mean; r.rstd = bn->rstd; r.s1 = bn->s1; r.s2 = bn->s2; r.sums64 = bn->sums64;
+  r.inv_count = bn->count > 0 ? (float)(1.0 / bn->count) : 0.0f;
+  r.train = bn->train; r.has = 1;
+  return r;
+}
+
+// sum / count of channel c: from the double record when there is one
+__device__ __forceinline__ float bn_sum_over_count(const float* s, const double* s64, int c, float inv_count) {
+  return s64 ? (float)(s64[c] * (double)inv_count) : s[c] * inv_count;
+}
+
 // Dropout streams of CUDA-graph replays: the host-side seed is baked into a captured launch, so a graphed training step
 // keeps two salt words on the device (refreshed by cgnn_step_tick inside the graph) and every kernel folds them into
 // its stream key before anything else.  No salt (eager mode): the stream is a function of the host seed alone.

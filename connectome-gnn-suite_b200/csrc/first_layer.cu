@@ -23,7 +23,7 @@ struct FirstArgs {
   // forward
   float* z; float* agg_out; double* stats_partials;
   // backward
-  const float* du; const float* demb; const float* zin; Act act_out; rt::BnBwdDev bn; const float* agg_in;
+  const float* du; const float* demb; const float* zin; Act act_out; BnBwdDev bn; const float* agg_in;
   float* partials; int part_stride;     // per CTA: [dW H x K2][dbias H]
 };
 
@@ -358,12 +358,7 @@ int launch_first_bwd(int kind, const float* du, const float* demb, const float* 
   a.t_in = t_in; a.act_in = make_act(act_in);
   a.blob = csr->agg_in; a.meta = csr->graph_meta; a.B = num_graphs;
   a.K = d_in; a.H = H; a.max_nodes = max_nodes < 1 ? 1 : max_nodes; a.max_edges = max_edges;
-  a.du = du; a.demb = demb; a.zin = z; a.act_out = make_act(act_out); a.agg_in = agg;
-  a.bn.has = bn ? 1 : 0;
-  a.bn.scale = bn ? bn->scale : nullptr; a.bn.mean = bn ? bn->mean : nullptr; a.bn.rstd = bn ? bn->rstd : nullptr;
-  a.bn.s1 = bn ? bn->s1 : nullptr; a.bn.s2 = bn ? bn->s2 : nullptr; a.bn.sums64 = bn ? bn->sums64 : nullptr;
-  a.bn.train = bn ? bn->train : 0;
-  a.bn.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  a.du = du; a.demb = demb; a.zin = z; a.act_out = make_act(act_out); a.agg_in = agg; a.bn = make_bn_bwd(bn);
   const int K2 = kind == AGG_SAGE ? 2 * d_in : d_in;
   a.partials = partials; a.part_stride = H * K2 + H;
   int grid = first_grid(smem, num_graphs);

@@ -176,9 +176,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_fwd(GcnFwdArgs p) {
 
 // ------------------------------------------------------------------------------------------
 struct GcnBwdArgs {
-  const float* du; const float* demb; const float* z; Act act_out;
-  const float* bn_scale; const float* bn_mean; const float* bn_rstd; const float* bn_s1; const float* bn_s2; const double* bn_sums64;
-  float inv_count; int bn_train; int has_bn;
+  const float* du; const float* demb; const float* z; Act act_out; BnBwdDev bn;
   const float* t_in; Act act_in; const float* W;
   const int32_t* out_rowptr; const int32_t* out_col; const float* out_wn; const float* dinv;
   const int32_t* meta; long long B;
@@ -197,8 +195,8 @@ enum { CI_SCALE = 0, CI_SHIFT, CI_MEAN, CI_RSTD, CI_ROWS };                     
 __device__ __forceinline__ float gcn_dz(const GcnBwdArgs& p, const float* s_co, int H4, bool aff_out, float t, float up,
                                         uint32_t rh, int c) {
   const float dy = act_bwd(p.act_out, aff_out, t, s_co[CO_SCALE * H4 + c], s_co[CO_SHIFT * H4 + c], rh, c, up);
-  if (!p.has_bn) return dy;
-  if (!p.bn_train) return s_co[CO_BSC * H4 + c] * dy;
+  if (!p.bn.has) return dy;
+  if (!p.bn.train) return s_co[CO_BSC * H4 + c] * dy;
   const float xh = (t - s_co[CO_MEAN * H4 + c]) * s_co[CO_RSTD * H4 + c];
   return s_co[CO_BSC * H4 + c] * (dy - s_co[CO_S1N * H4 + c] - xh * s_co[CO_S2N * H4 + c]);
 }
@@ -229,12 +227,12 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
   }
   stage_affine(p.act_out, H, H4, s_co + CO_SCALE * H4, s_co + CO_SHIFT * H4);
   for (int c = tid; c < H4; c += kThreads) {
-    const bool ok = c < H && p.has_bn;
-    s_co[CO_BSC * H4 + c] = ok ? p.bn_scale[c] : (c < H ? 1.0f : 0.0f);
-    s_co[CO_MEAN * H4 + c] = ok ? p.bn_mean[c] : 0.0f;
-    s_co[CO_RSTD * H4 + c] = ok ? p.bn_rstd[c] : 0.0f;
-    s_co[CO_S1N * H4 + c] = (ok && p.bn_train) ? (p.bn_sums64 ? (float)(p.bn_sums64[c] * (double)p.inv_count) : p.bn_s1[c] * p.inv_count) : 0.0f;
-    s_co[CO_S2N * H4 + c] = (ok && p.bn_train) ? (p.bn_sums64 ? (float)(p.bn_sums64[H + c] * (double)p.inv_count) : p.bn_s2[c] * p.inv_count) : 0.0f;
+    const bool ok = c < H && p.bn.has;
+    s_co[CO_BSC * H4 + c] = ok ? p.bn.scale[c] : (c < H ? 1.0f : 0.0f);
+    s_co[CO_MEAN * H4 + c] = ok ? p.bn.mean[c] : 0.0f;
+    s_co[CO_RSTD * H4 + c] = ok ? p.bn.rstd[c] : 0.0f;
+    s_co[CO_S1N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s1, p.bn.sums64, c, p.bn.inv_count) : 0.0f;
+    s_co[CO_S2N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s2, p.bn.sums64 ? p.bn.sums64 + H : nullptr, c, p.bn.inv_count) : 0.0f;
   }
   stage_affine(p.act_in, K, K4, s_ci + CI_SCALE * K4, s_ci + CI_SHIFT * K4);
   for (int c = tid; c < K4; c += kThreads) {
@@ -581,7 +579,8 @@ int cgnn_gcn_layer_fwd_pool(const float* t_in, const cgnn_act_t* act, const floa
                             int32_t max_edges, const cgnn_act_t* act_out, float* emb, cgnn_stream_t stream_) {
   (void)ptr;
   if (num_graphs < 0 || rows < 0 || d_in <= 0 || H <= 0 || max_nodes < 0 || max_edges < 0) return CGNN_ERR_INVALID_ARG;
-  if (num_graphs == 0 || rows == 0) return CGNN_OK;
+  if (num_graphs == 0) return CGNN_OK;
+  if (rows == 0) return CGNN_ERR_UNSUPPORTED;   // subjects without a row: cgnn_pool_fwd writes their embeddings
   if (!t_in || !W || !csr || !csr->graph_meta || !csr->agg_in || !emb) return CGNN_ERR_INVALID_ARG;
   if (!tensor_cores_enabled()) return CGNN_ERR_UNSUPPORTED;
   const int rc = launch_gcn_fwd_ws_pool(t_in, act, W, bias, csr, num_graphs, rows, d_in, H, max_nodes, max_edges, act_out, emb,
@@ -633,50 +632,34 @@ int cgnn_gcn_layer_bwd(const float* du, const float* demb, const float* z, const
     if (rcw >= 0) return rcw;
   }
   // Tensor-core generation: gather kernel (dz on load, dP = A^^T dz, dbias) + tcgen05 contractions (du_in, dW).
-  if (tensor_cores_enabled() && scratch && csr->agg_out && csr->agg_kind == AGG_GCN && (H == 32 || H == 64 || H == 128) &&
-      d_in <= 128 && (d_in + 31) / 32 != 3 && aligned16(scratch) && aligned16(z) && (!du || aligned16(du)) &&
-      (!demb || aligned16(demb))) {
-    const size_t region_a = (size_t)2 * 160 * 128 * sizeof(float);   // dbias partials of <= 2 CTAs per SM
-    const int part_stride = H * d_in + 2 * d_in;
-    if (workspace_bytes > region_a + (size_t)part_stride * sizeof(float)) {
-      GatherArgs ga{};
-      ga.meta = csr->graph_meta; ga.B = num_graphs; ga.blob = csr->agg_out;
-      ga.C = H; ga.max_nodes = max_nodes; ga.max_edges = max_edges;
-      ga.src = z; ga.act = make_act(act_out); ga.du = du; ga.demb = demb;
-      ga.has_bn = bn ? 1 : 0;
-      ga.bn_scale = bn ? bn->scale : nullptr; ga.bn_mean = bn ? bn->mean : nullptr; ga.bn_rstd = bn ? bn->rstd : nullptr;
-      ga.bn_s1 = bn ? bn->s1 : nullptr; ga.bn_s2 = bn ? bn->s2 : nullptr; ga.bn_sums64 = bn ? bn->sums64 : nullptr;
-      ga.bn_train = bn ? bn->train : 0;
-      ga.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
-      ga.out = scratch; ga.partials = (float*)workspace; ga.part_stride = H;
-      int g1 = 0, g2 = 0;
-      int rc = launch_gather(GATHER_GCN_BWD, ga, &g1, stream);
-      if (rc > 0) return rc;
-      if (rc == CGNN_OK) {
-        float* parts_b = (float*)((char*)workspace + region_a);
-        rc = launch_gcn_bwd_gemm(scratch, t_in, act_in, W, rows, d_in, H, du_in, prev_mean, prev_rstd, prev_sums ? 1 : 0,
-                                 parts_b, part_stride, H * d_in, &g2, workspace_bytes - region_a, stream);
-        if (rc > 0) return rc;
-        if (rc == CGNN_OK) {
-          ReduceQueue rq(stream);
-          rq.add((const float*)workspace, g1, H, 1, H, H, dbias);
-          rq.add(parts_b, g2, part_stride, H, d_in, d_in, dW);
-          if (prev_sums) rq.add(parts_b + H * d_in, g2, part_stride, 2, d_in, d_in, prev_sums, 0, prev_sums64);
-          return rq.flush();
-        }
-      }
-    }
+  const size_t region_a = (size_t)2 * 160 * 128 * sizeof(float);   // dbias partials of <= 2 CTAs per SM
+  const int part_stride = H * d_in + 2 * d_in;
+  if (tensor_cores_enabled() && scratch && csr->agg_out && csr->agg_kind == AGG_GCN && aligned16(z) && (!du || aligned16(du)) &&
+      (!demb || aligned16(demb)) && workspace_bytes > region_a && gather_supported(H, max_nodes, max_edges) &&
+      gcn_bwd_gemm_supported(scratch, t_in, du_in, rows, d_in, H, part_stride, workspace_bytes - region_a)) {
+    GatherArgs ga{};
+    ga.meta = csr->graph_meta; ga.B = num_graphs; ga.blob = csr->agg_out;
+    ga.C = H; ga.max_nodes = max_nodes; ga.max_edges = max_edges;
+    ga.src = z; ga.act = make_act(act_out); ga.du = du; ga.demb = demb; ga.bn = make_bn_bwd(bn);
+    ga.out = scratch; ga.partials = (float*)workspace; ga.part_stride = H;
+    int g1 = 0, g2 = 0;
+    int rc = launch_gather(GATHER_GCN_BWD, ga, &g1, stream);
+    if (rc != CGNN_OK) return rc;
+    float* parts_b = (float*)((char*)workspace + region_a);
+    rc = launch_gcn_bwd_gemm(scratch, t_in, act_in, W, rows, d_in, H, du_in, prev_mean, prev_rstd, prev_sums ? 1 : 0,
+                             parts_b, part_stride, H * d_in, &g2, workspace_bytes - region_a, stream);
+    if (rc != CGNN_OK) return rc;
+    ReduceQueue rq(stream);
+    rq.add((const float*)workspace, g1, H, 1, H, H, dbias);
+    rq.add(parts_b, g2, part_stride, H, d_in, d_in, dW);
+    if (prev_sums) rq.add(parts_b + H * d_in, g2, part_stride, 2, d_in, d_in, prev_sums, 0, prev_sums64);
+    return rq.flush();
   }
 #endif
   if (!csr_out_ok_(csr)) return CGNN_ERR_NEED_CSR;   // the generic kernel walks the CSR arrays
   const DeviceInfo dev = device_info();
   GcnBwdArgs a;
-  a.du = du; a.demb = demb; a.z = z; a.act_out = make_act(act_out);
-  a.has_bn = bn ? 1 : 0;
-  a.bn_scale = bn ? bn->scale : nullptr; a.bn_mean = bn ? bn->mean : nullptr; a.bn_rstd = bn ? bn->rstd : nullptr;
-  a.bn_s1 = bn ? bn->s1 : nullptr; a.bn_s2 = bn ? bn->s2 : nullptr; a.bn_sums64 = bn ? bn->sums64 : nullptr;
-  a.bn_train = bn ? bn->train : 0;
-  a.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  a.du = du; a.demb = demb; a.z = z; a.act_out = make_act(act_out); a.bn = make_bn_bwd(bn);
   a.t_in = t_in; a.act_in = make_act(act_in); a.W = W;
   a.out_rowptr = csr->out_rowptr; a.out_col = csr->out_col; a.out_wn = csr->out_wn; a.dinv = csr->dinv;
   a.meta = csr->graph_meta; a.B = num_graphs;

@@ -14,6 +14,7 @@
 // X B products (contraction over channels) read K-major 128B-swizzled tiles, X^T Y products (contraction over the
 // rows of the tile) read MN-major SWIZZLE_128B_BASE32B tiles - the only MN-major layout for tf32; see tc05.cuh.
 // Every thread owns a fixed channel quad of the tile (rowtile.cuh), so the per-channel constants sit in registers.
+#include "agg.cuh"
 #include "rowtile.cuh"
 #include "tile.cuh"
 
@@ -269,39 +270,57 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
 }
 
 
+// Launch shape of one contraction: KB blocks of 32 contraction channels, WIDE operand rows (16-byte aligned, a multiple of
+// 32 channels), dynamic shared memory and grid.
+struct GemmShape {
+  int KB; bool wide; size_t smem; long long grid;
+  int o_stage;   // k_sage_fwd_gemm: the epilogue staging area
+};
+
+bool sage_fwd_gemm_supported(const float* t_in, const float* agg, const float* z, int64_t rows, int32_t C, int32_t H,
+                             bool want_stats, size_t workspace_bytes, GemmShape* s) {
+  GemmShape unused;
+  if (!s) s = &unused;
+  if (H != 32 && H != 64 && H != 128) return false;
+  if (C <= 0 || 2 * C > 128) return false;
+  s->wide = (C % 32 == 0) && ((((uintptr_t)t_in) | ((uintptr_t)agg)) & 15u) == 0;
+  s->KB = (2 * C + 31) / 32;
+  if (s->KB == 3 || (!s->wide && s->KB > 2)) return false;
+  if ((((uintptr_t)z) & 15u) != 0) return false;
+  const DeviceInfo dev = device_info();
+  const int KP = 32 * s->KB;
+  const size_t a_bytes = (size_t)2 * s->KB * kRows * 128, b_bytes = (size_t)2 * s->KB * H * 128;
+  const size_t c_bytes = (size_t)2 * KP * 4;
+  size_t stage_bytes = (size_t)kRows * H * 4;
+  size_t total = a_bytes + b_bytes + c_bytes;
+  s->o_stage = (int)((total + 15) & ~(size_t)15);     // never aliases the operand: the epilogue of tile t-1 runs
+  total = s->o_stage + stage_bytes;                     // while the MMAs of tile t read it
+  s->smem = total + 1024;
+  if (s->smem > (size_t)dev.smem_optin) return false;
+  const long long ntiles = (rows + kRows - 1) / kRows;
+  s->grid = dev.sm_count;
+  if (s->grid > ntiles) s->grid = ntiles;
+  if (want_stats) {
+    const size_t rec = (size_t)(1 + 2 * H) * sizeof(double);
+    if ((size_t)s->grid * rec > workspace_bytes) s->grid = (long long)(workspace_bytes / rec);
+  }
+  return s->grid >= 1;
+}
+
 int launch_sage_fwd_gemm(const float* t_in, const cgnn_act_t* act, const float* agg, const float* W, const float* bias,
                          int64_t rows, int32_t C, int32_t H, float* z, double* partials, int* grid_out,
                          size_t workspace_bytes, cudaStream_t stream) {
-  if (H != 32 && H != 64 && H != 128) return -1;
-  if (C <= 0 || 2 * C > 128) return -1;
-  const bool wide = (C % 32 == 0) && ((((uintptr_t)t_in) | ((uintptr_t)agg)) & 15u) == 0;
-  const int KB = (2 * C + 31) / 32, HB = H / 32;
-  if (KB == 3 || (!wide && KB > 2)) return -1;
-  if ((((uintptr_t)z) & 15u) != 0) return -1;
-  const DeviceInfo dev = device_info();
+  GemmShape s;
+  if (!sage_fwd_gemm_supported(t_in, agg, z, rows, C, H, partials != nullptr, workspace_bytes, &s)) return CGNN_ERR_INVALID_ARG;
+  const int KB = s.KB, HB = H / 32;
+  const bool wide = s.wide; const size_t smem = s.smem; const long long grid = s.grid;
   SageFwdGemmArgs a;
   a.t_in = t_in; a.act = make_act(act); a.agg = agg; a.W = W; a.bias = bias;
   a.rows = rows; a.C = C; a.H = H;
   a.z = z; a.partials = partials;
   a.tmem_cols = 32;
   while (a.tmem_cols < (uint32_t)(2 * H)) a.tmem_cols <<= 1;   // two accumulator buffers
-  const int KP = 32 * KB;
-  const size_t a_bytes = (size_t)2 * KB * kRows * 128, b_bytes = (size_t)2 * KB * H * 128;
-  const size_t c_bytes = (size_t)2 * KP * 4;
-  size_t stage_bytes = (size_t)kRows * H * 4;
-  size_t total = a_bytes + b_bytes + c_bytes;
-  a.o_stage = (int)((total + 15) & ~(size_t)15);      // never aliases the operand: the epilogue of tile t-1 runs
-  total = a.o_stage + stage_bytes;                      // while the MMAs of tile t read it
-  const size_t smem = total + 1024;
-  if (smem > (size_t)dev.smem_optin) return -1;
-  const long long ntiles = (rows + kRows - 1) / kRows;
-  long long grid = dev.sm_count;
-  if (grid > ntiles) grid = ntiles;
-  if (partials) {
-    const size_t rec = (size_t)(1 + 2 * H) * sizeof(double);
-    if ((size_t)grid * rec > workspace_bytes) grid = (long long)(workspace_bytes / rec);
-  }
-  if (grid < 1) return -1;
+  a.o_stage = s.o_stage;
   *grid_out = (int)grid;
 #define CGNN_SF(KB_, HB_, W_, NT_)                                                                    \
   {                                                                                                   \
@@ -529,41 +548,51 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
   if (warp == 0) tc::tmem_dealloc(taddr, p.tmem_cols);
 }
 
-// Returns CGNN_OK when launched (grid in *grid_out; the caller reduces the partial records), -1 when the shape is
-// not covered (the caller falls back to the generic kernel).
+bool gcn_bwd_gemm_supported(const float* dP, const float* t_in, const float* du_in, int64_t rows, int32_t d_in, int32_t H,
+                            int part_stride, size_t partial_bytes, GemmShape* s) {
+  GemmShape unused;
+  if (!s) s = &unused;
+  if (H != 32 && H != 64 && H != 128) return false;
+  if (d_in <= 0 || d_in > 128) return false;
+  const int HB = H / 32, KB = (d_in + 31) / 32;
+  if (KB == 3) return false;
+  if ((((uintptr_t)dP) & 15u) != 0) return false;
+  s->KB = KB;
+  s->wide = (d_in % 32 == 0) && ((((uintptr_t)t_in) & 15u) == 0) && (!du_in || (((uintptr_t)du_in) & 15u) == 0);
+  if (!s->wide && KB > 2) return false;
+  if (du_in && 32 * KB > 2 * H) return false;   // the du_in staging must stay inside the K-major dP operand (see the two commits)
+  const DeviceInfo dev = device_info();
+  const int KP = 32 * KB;
+  size_t total = (size_t)4 * HB * kRows * 128 + (size_t)2 * KB * kRows * 128 + (size_t)2 * HB * KP * 128 + (size_t)2 * KP * 4;
+  const size_t a_view = (size_t)3 * HB * kRows * 128 + (size_t)4 * kRows * 128;   // the M = 128 view of the MN-major dP lo tile ends here
+  if (total < a_view) total = a_view;
+  if (total < (size_t)kRows * KP * 4) total = (size_t)kRows * KP * 4;
+  s->smem = total + 1024;
+  if (s->smem > (size_t)dev.smem_optin) return false;
+  const long long ntiles = (rows + kRows - 1) / kRows;
+  s->grid = dev.sm_count;
+  if (s->grid > ntiles) s->grid = ntiles;
+  const size_t rec = (size_t)part_stride * sizeof(float);
+  if ((size_t)s->grid * rec > partial_bytes) s->grid = (long long)(partial_bytes / rec);
+  return s->grid >= 1;
+}
+
+// Launches k_gcn_bwd_gemm (grid in *grid_out; the caller reduces the partial records).
 int launch_gcn_bwd_gemm(const float* dP, const float* t_in, const cgnn_act_t* act_in, const float* W, int64_t rows,
                         int32_t d_in, int32_t H, float* du_in, const float* prev_mean, const float* prev_rstd, int want_prev,
                         float* partials, int part_stride, int o_pprev, int* grid_out, size_t partial_bytes,
                         cudaStream_t stream) {
-  if (H != 32 && H != 64 && H != 128) return -1;
-  if (d_in <= 0 || d_in > 128) return -1;
-  const int HB = H / 32, KB = (d_in + 31) / 32;
-  if (KB == 3) return -1;
-  if ((((uintptr_t)dP) & 15u) != 0) return -1;
-  const bool wide = (d_in % 32 == 0) && ((((uintptr_t)t_in) & 15u) == 0) && (!du_in || (((uintptr_t)du_in) & 15u) == 0);
-  if (!wide && KB > 2) return -1;
-  if (du_in && 32 * KB > 2 * H) return -1;   // the du_in staging must stay inside the K-major dP operand (see the two commits)
-  const DeviceInfo dev = device_info();
+  GemmShape s;
+  if (!gcn_bwd_gemm_supported(dP, t_in, du_in, rows, d_in, H, part_stride, partial_bytes, &s)) return CGNN_ERR_INVALID_ARG;
+  const int KB = s.KB, HB = H / 32;
+  const bool wide = s.wide; const size_t smem = s.smem; const long long grid = s.grid;
   GcnBwdGemmArgs a;
   a.dP = dP; a.t_in = t_in; a.act_in = make_act(act_in); a.W = W;
   a.rows = rows; a.H = H; a.Kin = d_in;
   a.du_in = du_in; a.prev_mean = prev_mean; a.prev_rstd = prev_rstd; a.want_prev = want_prev;
   a.partials = partials; a.part_stride = part_stride; a.o_pprev = o_pprev;
-  const int KP = 32 * KB;
   a.tmem_cols = 32;
-  while (a.tmem_cols < (uint32_t)(2 * KP)) a.tmem_cols <<= 1;
-  size_t total = (size_t)4 * HB * kRows * 128 + (size_t)2 * KB * kRows * 128 + (size_t)2 * HB * KP * 128 + (size_t)2 * KP * 4;
-  const size_t a_view = (size_t)3 * HB * kRows * 128 + (size_t)4 * kRows * 128;   // the M = 128 view of the MN-major dP lo tile ends here
-  if (total < a_view) total = a_view;
-  if (total < (size_t)kRows * KP * 4) total = (size_t)kRows * KP * 4;
-  const size_t smem = total + 1024;
-  if (smem > (size_t)dev.smem_optin) return -1;
-  const long long ntiles = (rows + kRows - 1) / kRows;
-  long long grid = dev.sm_count;
-  if (grid > ntiles) grid = ntiles;
-  const size_t rec = (size_t)part_stride * sizeof(float);
-  if ((size_t)grid * rec > partial_bytes) grid = (long long)(partial_bytes / rec);
-  if (grid < 1) return -1;
+  while (a.tmem_cols < (uint32_t)(2 * 32 * KB)) a.tmem_cols <<= 1;
   *grid_out = (int)grid;
 #define CGNN_GB(HB_, KB_, W_)                                                                         \
   {                                                                                                   \
@@ -588,7 +617,7 @@ int launch_gcn_bwd_gemm(const float* dP, const float* t_in, const cgnn_act_t* ac
 // ================================================================================================================
 struct SageBwdGemmArgs {
   const float* du; const float* demb; const int32_t* row_graph; const int32_t* meta;   // upstream: per row, or pooled per subject
-  const float* z; Act act_out; rt::BnBwdDev bn;
+  const float* z; Act act_out; BnBwdDev bn;
   const float* t_in; const float* agg; Act act_in; const float* W;
   long long rows; int H, C;
   float* direct; float* nbr;          // d_u, d_agg [rows, C] (NULL: the layer input needs no gradient)
@@ -858,12 +887,7 @@ int launch_sage_bwd_gemm(const float* du, const float* demb, const int32_t* row_
   const DeviceInfo dev = device_info();
   SageBwdGemmArgs a;
   a.du = du; a.demb = demb; a.row_graph = row_graph; a.meta = meta;
-  a.z = z; a.act_out = make_act(act_out);
-  a.bn.has = bn ? 1 : 0;
-  a.bn.scale = bn ? bn->scale : nullptr; a.bn.mean = bn ? bn->mean : nullptr; a.bn.rstd = bn ? bn->rstd : nullptr;
-  a.bn.s1 = bn ? bn->s1 : nullptr; a.bn.s2 = bn ? bn->s2 : nullptr; a.bn.sums64 = bn ? bn->sums64 : nullptr;
-  a.bn.train = bn ? bn->train : 0;
-  a.bn.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  a.z = z; a.act_out = make_act(act_out); a.bn = make_bn_bwd(bn);
   a.t_in = t_in; a.agg = agg; a.act_in = make_act(act_in); a.W = W;
   a.rows = rows; a.H = H; a.C = C;
   a.direct = direct; a.nbr = nbr;

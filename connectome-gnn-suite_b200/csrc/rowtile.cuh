@@ -126,15 +126,6 @@ __device__ __forceinline__ float4 act_bwd4(const Act& a, const ChanQuad& cq, flo
 struct BnQuad {
   float bsc[4], mean[4], rstd[4], s1n[4], s2n[4];
 };
-struct BnBwdDev {
-  const float* scale; const float* mean; const float* rstd; const float* s1; const float* s2;
-  float inv_count; int train, has;
-  const double* sums64;     // [2, C] in double, read instead of s1 / s2 when given
-};
-// sum / count of channel c: from the double record when there is one
-__device__ __forceinline__ float bn_sum_over_count(const float* s, const double* s64, int c, float inv_count) {
-  return s64 ? (float)(s64[c] * (double)inv_count) : s[c] * inv_count;
-}
 __device__ __forceinline__ void bn_quad_init(BnQuad& b, const BnBwdDev& bn, int c0, int C) {
 #pragma unroll
   for (int j = 0; j < 4; ++j) {

@@ -178,9 +178,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_fwd(SageFwdArgs p) {
 
 // ------------------------------------------------------------------------------------------
 struct SageBwdArgs {
-  const float* du; const float* demb; const float* z; Act act_out;
-  const float* bn_scale; const float* bn_mean; const float* bn_rstd; const float* bn_s1; const float* bn_s2; const double* bn_sums64;
-  float inv_count; int bn_train; int has_bn;
+  const float* du; const float* demb; const float* z; Act act_out; BnBwdDev bn;
   const float* t_in; Act act_in; const float* W;
   const int32_t* in_rowptr; const int32_t* in_col; const float* in_w; const float* wsum;
   const int32_t* meta; long long B;
@@ -197,8 +195,8 @@ __device__ __forceinline__ float sage_dq(const SageBwdArgs& p, const float* s_co
                                          uint32_t rh, int c) {
   const float dy = act_bwd(p.act_out, aff_out, t, s_co[SO_SCALE * H4 + c], s_co[SO_SHIFT * H4 + c], rh, c, up);
   float dz = dy;
-  if (p.has_bn) {
-    if (p.bn_train) {
+  if (p.bn.has) {
+    if (p.bn.train) {
       const float xh = (t - s_co[SO_MEAN * H4 + c]) * s_co[SO_RSTD * H4 + c];
       dz = s_co[SO_BSC * H4 + c] * (dy - s_co[SO_S1N * H4 + c] - xh * s_co[SO_S2N * H4 + c]);
     } else {
@@ -233,12 +231,12 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
   }
   stage_affine(p.act_out, H, H4, s_co + SO_SCALE * H4, s_co + SO_SHIFT * H4);
   for (int c = tid; c < H4; c += kThreads) {
-    const bool ok = c < H && p.has_bn;
-    s_co[SO_BSC * H4 + c] = ok ? p.bn_scale[c] : (c < H ? 1.0f : 0.0f);
-    s_co[SO_MEAN * H4 + c] = ok ? p.bn_mean[c] : 0.0f;
-    s_co[SO_RSTD * H4 + c] = ok ? p.bn_rstd[c] : 0.0f;
-    s_co[SO_S1N * H4 + c] = (ok && p.bn_train) ? (p.bn_sums64 ? (float)(p.bn_sums64[c] * (double)p.inv_count) : p.bn_s1[c] * p.inv_count) : 0.0f;
-    s_co[SO_S2N * H4 + c] = (ok && p.bn_train) ? (p.bn_sums64 ? (float)(p.bn_sums64[H + c] * (double)p.inv_count) : p.bn_s2[c] * p.inv_count) : 0.0f;
+    const bool ok = c < H && p.bn.has;
+    s_co[SO_BSC * H4 + c] = ok ? p.bn.scale[c] : (c < H ? 1.0f : 0.0f);
+    s_co[SO_MEAN * H4 + c] = ok ? p.bn.mean[c] : 0.0f;
+    s_co[SO_RSTD * H4 + c] = ok ? p.bn.rstd[c] : 0.0f;
+    s_co[SO_S1N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s1, p.bn.sums64, c, p.bn.inv_count) : 0.0f;
+    s_co[SO_S2N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s2, p.bn.sums64 ? p.bn.sums64 + H : nullptr, c, p.bn.inv_count) : 0.0f;
   }
   stage_affine(p.act_in, K, K4, s_ci, s_ci + K4);
   __syncthreads();
@@ -556,21 +554,20 @@ int cgnn_sage_layer_fwd(const float* t_in, const cgnn_act_t* act, const float* W
     if (rcw > 0) return rcw;
   }
   // Tensor-core generation: gather kernel (weighted mean of the neighbours) + tcgen05 contraction.
-  if (tensor_cores_enabled() && agg && csr->agg_in && csr->agg_kind == AGG_SAGE && (H == 32 || H == 64 || H == 128) &&
-      2 * d_in <= 128 && (2 * d_in + 31) / 32 != 3 && (d_in <= 32 || d_in % 32 == 0) && aligned16(agg) && aligned16(z)) {
+  if (tensor_cores_enabled() && agg && csr->agg_in && csr->agg_kind == AGG_SAGE && aligned16(agg) &&
+      gather_supported(d_in, max_nodes, max_edges) &&
+      sage_fwd_gemm_supported(t_in, agg, z, rows, d_in, H, bn_stats != nullptr, workspace_bytes)) {
     GatherArgs ga{};
     ga.meta = csr->graph_meta; ga.B = num_graphs; ga.blob = csr->agg_in;
     ga.C = d_in; ga.max_nodes = max_nodes; ga.max_edges = max_edges;
     ga.src = t_in; ga.act = make_act(act); ga.out = agg;
     int g1 = 0, g2 = 0;
     int rc = launch_gather(GATHER_SAGE_FWD, ga, &g1, stream);
-    if (rc > 0) return rc;
-    if (rc == CGNN_OK) {
-      rc = launch_sage_fwd_gemm(t_in, act, agg, W, bias, rows, d_in, H, z, bn_stats ? (double*)workspace : nullptr, &g2,
-                                workspace_bytes, stream);
-      if (rc > 0) return rc;
-      if (rc == CGNN_OK) return bn_stats ? launch_stats_merge((const double*)workspace, g2, H, bn_stats, stream) : CGNN_OK;
-    }
+    if (rc != CGNN_OK) return rc;
+    rc = launch_sage_fwd_gemm(t_in, act, agg, W, bias, rows, d_in, H, z, bn_stats ? (double*)workspace : nullptr, &g2,
+                              workspace_bytes, stream);
+    if (rc != CGNN_OK) return rc;
+    return bn_stats ? launch_stats_merge((const double*)workspace, g2, H, bn_stats, stream) : CGNN_OK;
   }
 #endif
   if (!arrays_fwd) return CGNN_ERR_NEED_CSR;       // the generic kernel walks the CSR arrays
@@ -672,10 +669,9 @@ int cgnn_sage_layer_bwd(const float* du, const float* demb, const float* z, cons
     if (rcw >= 0) return rcw;
   }
   // Tensor-core generation: tcgen05 contractions (dz on load, [d_u || d_agg], dW, dbias) + transposed gather kernel.
+  // The gather runs second: its coverage is settled before the contractions launch.
   if (tensor_cores_enabled() && agg && csr->agg_out && csr->row_graph && csr->agg_kind == AGG_SAGE &&
-      (H == 32 || H == 64 || H == 128) && 2 * d_in <= 128 && (2 * d_in + 31) / 32 != 3 && (d_in <= 32 || d_in % 32 == 0) &&
-      aligned16(z) && (!du || aligned16(du)) && (!demb || aligned16(demb)) && (!du_in || (scratch && aligned16(scratch))) &&
-      (!du_in || gather_supported(d_in, max_nodes, max_edges))) {
+      (!du_in || (aligned16(scratch) && gather_supported(d_in, max_nodes, max_edges)))) {
     const int part_stride = H * 2 * d_in + H;
     const size_t region_a = (size_t)160 * part_stride * sizeof(float);   // partial records of <= 160 CTAs
     if (workspace_bytes > region_a + (size_t)2 * 160 * 2 * d_in * sizeof(float)) {
@@ -698,7 +694,7 @@ int cgnn_sage_layer_bwd(const float* du, const float* demb, const float* z, cons
         ga.out = du_in;
         ga.partials = (float*)((char*)workspace + region_a); ga.part_stride = 2 * d_in;
         rc = launch_gather(GATHER_SAGE_BWD, ga, &g2, stream);
-        if (rc != CGNN_OK) return rc > 0 ? rc : CGNN_ERR_TILE_TOO_LARGE;
+        if (rc != CGNN_OK) return rc;
         if (prev_sums) rq.add(ga.partials, g2, 2 * d_in, 2, d_in, d_in, prev_sums, 0, prev_sums64);     // all three after the gather: one launch
         return rq.flush();
       }
@@ -708,12 +704,7 @@ int cgnn_sage_layer_bwd(const float* du, const float* demb, const float* z, cons
   if (!arrays_bwd) return CGNN_ERR_NEED_CSR;       // the generic kernels walk the CSR arrays
   const DeviceInfo dev = device_info();
   SageBwdArgs a;
-  a.du = du; a.demb = demb; a.z = z; a.act_out = make_act(act_out);
-  a.has_bn = bn ? 1 : 0;
-  a.bn_scale = bn ? bn->scale : nullptr; a.bn_mean = bn ? bn->mean : nullptr; a.bn_rstd = bn ? bn->rstd : nullptr;
-  a.bn_s1 = bn ? bn->s1 : nullptr; a.bn_s2 = bn ? bn->s2 : nullptr; a.bn_sums64 = bn ? bn->sums64 : nullptr;
-  a.bn_train = bn ? bn->train : 0;
-  a.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  a.du = du; a.demb = demb; a.z = z; a.act_out = make_act(act_out); a.bn = make_bn_bwd(bn);
   a.t_in = t_in; a.act_in = make_act(act_in); a.W = W;
   a.in_rowptr = csr->in_rowptr; a.in_col = csr->in_col; a.in_w = csr->in_w; a.wsum = csr->wsum;
   a.meta = csr->graph_meta; a.B = num_graphs;

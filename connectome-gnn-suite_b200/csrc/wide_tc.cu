@@ -408,7 +408,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
 // ---- dz = relu'(z) * BatchNorm-backward(dropout-backward(upstream)) materialised, plus its column sums (GraphSAGE) ------
 struct WideDzArgs {
   const float* z; const float* du; const float* demb; const int32_t* row_graph; const int32_t* meta;
-  Act act_out; rt::BnBwdDev bn; long long rows; float* dz; float* partials;   // per CTA [256]
+  Act act_out; BnBwdDev bn; long long rows; float* dz; float* partials;   // per CTA [256]
 };
 
 __global__ void __launch_bounds__(kThreads, 2) k_wide_dz(WideDzArgs p) {
@@ -574,12 +574,7 @@ int launch_gcn_bwd_wide(const float* du, const float* demb, const float* z, cons
   GatherArgs ga{};
   ga.meta = csr->graph_meta; ga.B = num_graphs; ga.blob = csr->agg_out;
   ga.C = WN; ga.max_nodes = max_nodes; ga.max_edges = max_edges;
-  ga.src = z; ga.act = make_act(act_out); ga.du = du; ga.demb = demb;
-  ga.has_bn = bn ? 1 : 0;
-  ga.bn_scale = bn ? bn->scale : nullptr; ga.bn_mean = bn ? bn->mean : nullptr; ga.bn_rstd = bn ? bn->rstd : nullptr;
-  ga.bn_s1 = bn ? bn->s1 : nullptr; ga.bn_s2 = bn ? bn->s2 : nullptr; ga.bn_sums64 = bn ? bn->sums64 : nullptr;
-  ga.bn_train = bn ? bn->train : 0;
-  ga.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  ga.src = z; ga.act = make_act(act_out); ga.du = du; ga.demb = demb; ga.bn = make_bn_bwd(bn);
   ga.out = scratch; ga.partials = (float*)workspace; ga.part_stride = WN;
   int g1 = 0, g2 = 0, g3 = 0;
   int rc = launch_gather(GATHER_GCN_BWD, ga, &g1, stream);
@@ -653,12 +648,7 @@ int launch_sage_bwd_wide(const float* du, const float* demb, const float* z, con
   // (1) dz and dbias
   WideDzArgs a{};
   a.z = z; a.du = du; a.demb = demb; a.row_graph = csr->row_graph; a.meta = csr->graph_meta;
-  a.act_out = make_act(act_out);
-  a.bn.has = bn ? 1 : 0;
-  a.bn.scale = bn ? bn->scale : nullptr; a.bn.mean = bn ? bn->mean : nullptr; a.bn.rstd = bn ? bn->rstd : nullptr;
-  a.bn.s1 = bn ? bn->s1 : nullptr; a.bn.s2 = bn ? bn->s2 : nullptr; a.bn.sums64 = bn ? bn->sums64 : nullptr;
-  a.bn.train = bn ? bn->train : 0;
-  a.bn.inv_count = (bn && bn->count > 0) ? (float)(1.0 / bn->count) : 0.0f;
+  a.act_out = make_act(act_out); a.bn = make_bn_bwd(bn);
   a.rows = rows; a.dz = dz; a.partials = (float*)workspace;
   long long gdz = 2LL * dev.sm_count;
   if (gdz > (rows + 15) / 16) gdz = (rows + 15) / 16;
@@ -700,7 +690,7 @@ int launch_sage_bwd_wide(const float* du, const float* demb, const float* z, con
   ga.partials = (float*)workspace; ga.part_stride = 2 * WN;
   int g4 = 0;
   rc = launch_gather(GATHER_SAGE_BWD, ga, &g4, stream);
-  if (rc != CGNN_OK) return rc > 0 ? rc : CGNN_ERR_TILE_TOO_LARGE;
+  if (rc != CGNN_OK) return rc;
   if ((size_t)g4 * 2 * WN * sizeof(float) > region_a) return CGNN_ERR_WORKSPACE;
   if (prev_sums) return launch_reduce_partials(ga.partials, g4, 2 * WN, 2, WN, WN, prev_sums, stream, 0, prev_sums64);
   return CGNN_OK;

@@ -352,14 +352,14 @@ def run_fwd_pool(eng, sizes, seed=0):
 
 
 # ---- the dispatch table ---------------------------------------------------------------------------------------------
-# (id, runner, kwargs, runs on the simulator, kernels a B200 must show for it)
+# (id, runner, kwargs, runs on the simulator, kernels a B200 must show for it, kernels it must not show)
 R84 = ("rand", (84, 84, 84, 84), 64, 1)
 SMALL16 = ("rand", (20,) * 16, 64, 2)
 CASES, EMU_CASES = [], []
 
 
-def case(cid, fn, kw, emu, expect=()):
-    CASES.append(pytest.param(fn, kw, set(expect), id=cid))
+def case(cid, fn, kw, emu, expect=(), forbid=()):
+    CASES.append(pytest.param(fn, kw, set(expect), set(forbid), id=cid))
     if emu:
         EMU_CASES.append(pytest.param(fn, kw, id=cid))
 
@@ -414,6 +414,9 @@ case("sage-fwd-wide256", run_layer_fwd, dict(kind="sage", d_in=256, H=256, graph
 for H in (20, 96):
     case(f"sage-fwd-generic-H{H}", run_layer_fwd, dict(kind="sage", d_in=64, H=H, graph=("rand", (84, 30, 1), 64, 8)), True,
          ["k_sage_fwd"])
+# the contraction's operands exceed shared memory: no gather may run first only to be thrown away
+case("sage-fwd-generic-d64-H128", run_layer_fwd, dict(kind="sage", d_in=64, H=128, graph=("rand", (84, 30, 1), 64, 8)), True,
+     ["k_sage_fwd"], forbid=["k_gather<0>", "k_sage_fwd_gemm"])
 case("sage-fwd-ingest360-first", run_layer_fwd, dict(kind="sage", d_in=1, H=64, graph=("ingest", 2, 360, "dense", 0.9),
                                                       hidden=False), True, ["k_gather<0>", "k_sage_fwd_gemm"])
 case("sage-fwd-ingest360-hidden", run_layer_fwd, dict(kind="sage", d_in=64, H=64, graph=("ingest", 2, 360, "dense", 0.9)), True,
@@ -451,6 +454,9 @@ for kind in ("gcn", "sage"):
                                                              first=True), True, ["k_gcn_bwd"] if kind == "gcn" else [gemm])
     case(f"{kind}-bwd-ingest360-hidden", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=("ingest", 2, 360, "dense", 0.9),
                                                               pooled=True), True, generic)
+# du_in of 128 channels does not fit the contraction's dP operand at H = 32: no gather may run first only to be thrown away
+case("gcn-bwd-generic-d128-H32", run_layer_bwd, dict(kind="gcn", d_in=128, H=32, graph=("rand", (84, 30, 1), 128, 14)), True,
+     ["k_gcn_bwd"], forbid=["k_gather<1>", "k_gcn_bwd_gemm"])
 # -- pool, BatchNorm backward sums
 case("pool-sums-C64", run_pool_and_sums, dict(C=64, graph=R84), True, ["k_pool_fwd_quad", "k_bn_bwd_sums_quad"])
 case("pool-sums-C20-wrap-salt", run_pool_and_sums, dict(C=20, graph=("rand", (360,), 20, 15), row_base=ROW_BASE_WRAP,
@@ -534,12 +540,13 @@ def _run_profiled(fn, kw):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("fn,kw,expect", CASES)
-def test_contract_on_b200(request, fn, kw, expect):
+@pytest.mark.parametrize("fn,kw,expect,forbid", CASES)
+def test_contract_on_b200(request, fn, kw, expect, forbid):
     r, names = _run_profiled(fn, kw)
     _SEEN[request.node.callspec.id] = (names, r)
     missing = expect - names
     assert not missing, f"intended kernels {sorted(missing)} did not run; ran: {sorted(names)}"
+    assert not forbid & names, f"kernels {sorted(forbid & names)} must not run; ran: {sorted(names)}"
 
 
 @pytest.mark.gpu
@@ -558,7 +565,7 @@ def test_dispatch_table():
     run in this session (deselected) are run here."""
     for p in CASES:
         if p.id not in _SEEN:
-            fn, kw, _ = p.values
+            fn, kw, _, _ = p.values
             r, names = _run_profiled(fn, kw)
             _SEEN[p.id] = (names, r)
     print("\ncase | worst error (x 2^-23 x mag) | kernels")
