@@ -200,7 +200,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
       if (!valid || !live_quad) continue;
       const long long grow = nb + row;
       if (MODE == GATHER_SAGE_FWD) {
-        const float inv = rt::rcp_fast(aux + 1e-8f);   // weighted mean (models.py:149); ~1 ulp off the exact quotient
+        const float inv = fast_rcp(aux + 1e-8f);   // weighted mean (models.py:149); ~1 ulp off the exact quotient
         acc.x *= inv; acc.y *= inv; acc.z *= inv; acc.w *= inv;
       }
       if (MODE == GATHER_SAGE_BWD) {

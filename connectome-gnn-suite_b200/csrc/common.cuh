@@ -118,6 +118,25 @@ static inline BnBwdDev make_bn_bwd(const cgnn_bn_bwd_t* bn) {
 __device__ __forceinline__ float bn_sum_over_count(const float* s, const double* s64, int c, float inv_count) {
   return s64 ? (float)(s64[c] * (double)inv_count) : s[c] * inv_count;
 }
+// the per-channel coefficients of the BatchNorm backward, channel c of C (c >= C: padding)
+struct BnCoef {
+  float mean, rstd, bsc, s1n, s2n;   // in the order bn_bwd_dz reads them
+};
+__device__ __forceinline__ BnCoef bn_bwd_coef(const BnBwdDev& bn, int c, int C) {
+  const bool ok = bn.has && c < C;
+  BnCoef k;
+  k.bsc = ok ? bn.scale[c] : (c < C ? 1.0f : 0.0f);
+  k.mean = ok ? bn.mean[c] : 0.0f;
+  k.rstd = ok ? bn.rstd[c] : 0.0f;
+  k.s1n = (ok && bn.train) ? bn_sum_over_count(bn.s1, bn.sums64, c, bn.inv_count) : 0.0f;
+  k.s2n = (ok && bn.train) ? bn_sum_over_count(bn.s2, bn.sums64 ? bn.sums64 + C : nullptr, c, bn.inv_count) : 0.0f;
+  return k;
+}
+// dz of one element in train mode (eval mode: dz = bsc * dy)
+__device__ __forceinline__ float bn_bwd_dz(const BnCoef& k, float t, float dy) {
+  const float xh = (t - k.mean) * k.rstd;
+  return k.bsc * (dy - k.s1n - xh * k.s2n);
+}
 
 // Dropout streams of CUDA-graph replays: the host-side seed is baked into a captured launch, so a graphed training step
 // keeps two salt words on the device (refreshed by cgnn_step_tick inside the graph) and every kernel folds them into
@@ -135,7 +154,6 @@ __device__ __forceinline__ uint32_t fmix32(uint32_t h) {
 }
 // Dropout stream: one mix per row (cheap, no avalanche of its own), one full-avalanche hash per channel QUAD, from
 // which the four 16-bit fields of the quad are cut - the second pair from a multiply / xor-shift of the first word.
-// (The row-tile kernels evaluate the same function a quad at a time, rowtile.cuh::drop_keep4.)
 __device__ __forceinline__ uint32_t drop_row_hash(const Act& a, long long grow) {
   uint32_t lo = (uint32_t)grow, hi = (uint32_t)((unsigned long long)grow >> 32);
   return (lo * 0x9E3779B1u) ^ a.k0 ^ fmix32(hi + a.k1);
@@ -144,11 +162,19 @@ __device__ __forceinline__ uint32_t drop_second_word(uint32_t y) {
   uint32_t w = y * 0x9E3779B1u + 0x7F4A7C15u;
   return w ^ (w >> 15);
 }
+// the stream's key of channel quad `quad` (channels 4 quad .. 4 quad + 3), the same for every row
+__device__ __forceinline__ uint32_t drop_quad_key(const Act& a, int quad) { return (uint32_t)quad * 0x632BE5ABu + a.k1; }
+// whether the low (half 0) or high (half 1) 16-bit field of a stream word keeps its channel
+__device__ __forceinline__ bool drop_field_kept(const Act& a, uint32_t w, int half) { return (half ? (w >> 16) : (w & 0xffffu)) >= a.thresh; }
+// keep bits of a channel quad at a row: bit j = channel 4 quad + j kept
+__device__ __forceinline__ uint32_t drop_keep4(const Act& a, uint32_t row_hash, uint32_t quad_key) {
+  const uint32_t w0 = fmix32(row_hash + quad_key), w1 = drop_second_word(w0);
+  return (drop_field_kept(a, w0, 0) ? 1u : 0u) | (drop_field_kept(a, w0, 1) ? 2u : 0u) | (drop_field_kept(a, w1, 0) ? 4u : 0u) |
+         (drop_field_kept(a, w1, 1) ? 8u : 0u);
+}
 __device__ __forceinline__ bool drop_keep(const Act& a, uint32_t row_hash, int c) {
-  const uint32_t y = fmix32(row_hash + (uint32_t)(c >> 2) * 0x632BE5ABu + a.k1);
-  const uint32_t w = (c & 2) ? drop_second_word(y) : y;
-  uint32_t bits = (c & 1) ? (w >> 16) : (w & 0xffffu);
-  return bits >= a.thresh;
+  const uint32_t y = fmix32(row_hash + drop_quad_key(a, c >> 2));
+  return drop_field_kept(a, (c & 2) ? drop_second_word(y) : y, c & 1);
 }
 
 // u = dropout(relu?(sc * t + sh)).  `affine` is warp-uniform (a.scale != nullptr).

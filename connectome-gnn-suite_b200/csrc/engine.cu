@@ -19,7 +19,7 @@
 //                               then z_i = sum_e w^_e P_src(e) + dinv_i^2 P_i + b: half a warp per row, float4
 //                               lanes, records two at a time; write z (coalesced), BatchNorm statistics
 //
-// Only t_in, the records and z cross HBM.  The same sources run on the test-only simulator (ws.cuh).
+// Only t_in, the records and z cross HBM.  The same sources run on the test-only simulator (tc05.cuh).
 #include "engine.cuh"
 
 namespace cgnn {
@@ -41,7 +41,7 @@ struct Args {
 };
 
 template <bool POOL>
-__global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ ws::TensorMap tmap, Args p) {
+__global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ tc::TensorMap tmap, Args p) {
   act_salt(p.act);   // device-side dropout salt (CUDA-graph replays)
 #ifdef CGNN_EMU
   CGNN_SMEM_DECL;
@@ -51,7 +51,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
 #endif
   __shared__ Barriers bars;
   __shared__ uint32_t tmem_base_s;
-  unsigned char* base = ws::smem_align1024(smem_raw);
+  unsigned char* base = tc::smem_align1024(smem_raw);
   unsigned char* w_hi = base;                           // [2 K blocks][64 rows][128 B]
   unsigned char* w_lo = base + 2 * kC * 128;
   unsigned char* s_stage = base + p.o_stage;
@@ -64,33 +64,29 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
   // ---- one-time setup ------------------------------------------------------------------------------------------
-  if (warp == kWarpAlloc) ws::tmem_alloc(&tmem_base_s, kTmemCols);
+  if (warp == kWarpAlloc) tc::tmem_alloc(&tmem_base_s, kTmemCols);
   if (tid == 0) {
-    for (int i = 0; i < kNS; ++i) { ws::mbar_init(&bars.stage_full[i], 1); ws::mbar_init(&bars.stage_free[i], 4 * 32); }
-    for (int i = 0; i < 2; ++i) { ws::mbar_init(&bars.a_full[i], 4 * 32); ws::mbar_init(&bars.a_free[i], 1); }
-    for (int i = 0; i < kMaxTiles; ++i) { ws::mbar_init(&bars.d_full[i], 1); ws::mbar_init(&bars.d_free[i], kGathWarps); }
-    for (int i = 0; i < 2; ++i) { ws::mbar_init(&bars.blob_full[i], 1); ws::mbar_init(&bars.blob_free[i], kGathWarps); }
-    ws::fence_mbar_init();
+    for (int i = 0; i < kNS; ++i) { tc::mbar_init(&bars.stage_full[i], 1); tc::mbar_init(&bars.stage_free[i], 4 * 32); }
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.a_full[i], 4 * 32); tc::mbar_init(&bars.a_free[i], 1); }
+    for (int i = 0; i < kMaxTiles; ++i) { tc::mbar_init(&bars.d_full[i], 1); tc::mbar_init(&bars.d_free[i], kGathWarps); }
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.blob_full[i], 1); tc::mbar_init(&bars.blob_free[i], kGathWarps); }
+    tc::fence_mbar_init();
   }
-  if (warp == kWarpTile && lane == 0) ws::prefetch_tensor_map(&tmap);
+  if (warp == kWarpTile && lane == 0) tc::prefetch_tensor_map(&tmap);
   // W [64 out][64 in] -> K-major operand rows n = output channel, hi / lo parts
   for (int idx = tid; idx < kC * (kC / 4); idx += kNT) {
     const int n = idx / (kC / 4), k = (idx - n * (kC / 4)) * 4;
-    const float4 v = *reinterpret_cast<const float4*>(p.W + n * kC + k);
-    const float4 h = make_float4(ws::tf32_hi(v.x), ws::tf32_hi(v.y), ws::tf32_hi(v.z), ws::tf32_hi(v.w));
-    const uint32_t off = ws::kmajor_offset(n, k, kC);
-    *reinterpret_cast<float4*>(w_hi + off) = h;
-    *reinterpret_cast<float4*>(w_lo + off) = make_float4(v.x - h.x, v.y - h.y, v.z - h.z, v.w - h.w);
+    tc::store_split4(w_hi, w_lo, n, k, kC, *reinterpret_cast<const float4*>(p.W + n * kC + k));
   }
   for (int c = tid; c < kC; c += kNT) {
     s_scale[c] = p.act.scale ? p.act.scale[c] : 1.0f;
     s_shift[c] = p.act.scale ? p.act.shift[c] : 0.0f;
     s_bias[c] = p.bias ? p.bias[c] : 0.0f;
   }
-  ws::fence_proxy_async();        // the W operands are read by the tensor core (async proxy)
-  ws::fence_before_sync();
+  tc::fence_proxy_async();        // the W operands are read by the tensor core (async proxy)
+  tc::fence_before_sync();
   __syncthreads();
-  ws::fence_after_sync();
+  tc::fence_after_sync();
   const uint32_t tmem = tmem_base_s;
 
   if (warp == kWarpTile) {
@@ -101,9 +97,9 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
         const Unit un = unit_geom(p.src(), u);
         for (int t = 0; t < un.tiles; ++t, ++tcount)
           for (int h = 0; h < 2; ++h) {
-            ws::mbar_wait_relaxed(&bars.stage_free[h], (tcount & 1u) ^ 1u);
-            ws::mbar_arrive_expect_tx(&bars.stage_full[h], kStageBytes);
-            ws::tma_load_box(s_stage + h * kStageBytes, &tmap, 32 * h, un.row0 + (long long)t * kTR, &bars.stage_full[h]);
+            tc::mbar_wait(&bars.stage_free[h], (tcount & 1u) ^ 1u);
+            tc::mbar_arrive_expect_tx(&bars.stage_full[h], kStageBytes);
+            tc::tma_load_box(s_stage + h * kStageBytes, &tmap, 32 * h, un.row0 + (long long)t * kTR, &bars.stage_full[h]);
           }
       }
     }
@@ -114,36 +110,36 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
       for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
         const Unit un = unit_geom(p.src(), u);
         const uint32_t b = ucount % (uint32_t)p.nblob, use = ucount / (uint32_t)p.nblob;
-        ws::mbar_wait_relaxed(&bars.blob_free[b], (use & 1u) ^ 1u);
-        ws::mbar_arrive_expect_tx(&bars.blob_full[b], (uint32_t)un.blob_bytes);
-        ws::bulk_load(s_blob + (size_t)b * p.blob_cap_bytes, p.blob + un.blob_word0, (uint32_t)un.blob_bytes, &bars.blob_full[b]);
+        tc::mbar_wait(&bars.blob_free[b], (use & 1u) ^ 1u);
+        tc::mbar_arrive_expect_tx(&bars.blob_full[b], (uint32_t)un.blob_bytes);
+        tc::bulk_load(s_blob + (size_t)b * p.blob_cap_bytes, p.blob + un.blob_word0, (uint32_t)un.blob_bytes, &bars.blob_full[b]);
       }
     }
   } else if (warp == kWarpMma) {
     // ================================ MMA issuer ===================================================================
     if (lane == 0) {
-      const uint32_t idesc = ws::idesc_tf32(kTR, kC);
-      const uint64_t b_hi = ws::smem_desc_sw128(ws::smem_u32(w_hi)), b_lo = ws::smem_desc_sw128(ws::smem_u32(w_lo));
+      const uint32_t idesc = tc::idesc_tf32(kTR, kC);
+      const uint64_t b_hi = tc::smem_desc_sw128(tc::smem_u32(w_hi)), b_lo = tc::smem_desc_sw128(tc::smem_u32(w_lo));
       uint32_t tcount = 0, uses[kMaxTiles] = {0, 0, 0};
       for (long long u = blockIdx.x; u < p.units; u += gridDim.x) {
         const Unit un = unit_geom(p.src(), u);
         for (int t = 0; t < un.tiles; ++t, ++tcount) {
-          ws::mbar_wait_relaxed(&bars.d_free[t], (uses[t] & 1u) ^ 1u);     // the gather warps have drained this slot's previous tile
+          tc::mbar_wait(&bars.d_free[t], (uses[t] & 1u) ^ 1u);     // the gather warps have drained this slot's previous tile
           ++uses[t];
           const uint32_t d = tmem + kColD + (uint32_t)(kC * t);
 #pragma unroll
           for (int h = 0; h < 2; ++h) {
-            ws::mbar_wait_relaxed(&bars.a_full[h], tcount & 1u);
-            ws::fence_after_sync();
+            tc::mbar_wait(&bars.a_full[h], tcount & 1u);
+            tc::fence_after_sync();
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks) {
               const uint64_t bo = (uint64_t)((h * kC * 128 + ks * 32) >> 4);
               const uint32_t ac = (uint32_t)(32 * h + 8 * ks);
-              ws::mma_tf32x3_ts(d, tmem + kColAHi + ac, tmem + kColALo + ac, b_hi + bo, b_lo + bo, idesc, (h | ks) ? 1u : 0u);
+              tc::mma_tf32x3_ts(d, tmem + kColAHi + ac, tmem + kColALo + ac, b_hi + bo, b_lo + bo, idesc, (h | ks) ? 1u : 0u);
             }
-            ws::mma_commit(&bars.a_free[h]);       // this half of the A columns may be rewritten once these MMAs are done
+            tc::mma_commit(&bars.a_free[h]);       // this half of the A columns may be rewritten once these MMAs are done
           }
-          ws::mma_commit(&bars.d_full[t]);
+          tc::mma_commit(&bars.d_full[t]);
         }
       }
     }
@@ -158,11 +154,11 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
     for (long long u = blockIdx.x; u < p.units; u += gridDim.x) {
       const Unit un = unit_geom(p.src(), u);
       for (int t = 0; t < un.tiles; ++t, ++tcount) {
-        ws::mbar_wait_relaxed(&bars.stage_full[h], tcount & 1u);
+        tc::mbar_wait(&bars.stage_full[h], tcount & 1u);
         float4 v[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const float4*>(slot + ws::box_chunk_offset(row, j));
-        ws::mbar_arrive(&bars.stage_free[h]);      // the values are in registers: the slot may be refilled
+        for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const float4*>(slot + tc::box_chunk_offset(row, j));
+        tc::mbar_arrive(&bars.stage_free[h]);      // the values are in registers: the slot may be refilled
         const long long grow = un.row0 + (long long)t * kTR + row;
         const uint32_t rh = p.act.drop ? drop_row_hash(p.act, p.act.row_base + grow) : 0u;
 #pragma unroll
@@ -178,30 +174,31 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
             for (int e = 0; e < 4; ++e) y[e] = fmaxf(y[e], 0.0f);
           }
           if (p.act.drop) {
-            const uint32_t keep = keep4(p.act, rh, c0 >> 2);
+            const uint32_t keep = drop_keep4(p.act, rh, drop_quad_key(p.act, c0 >> 2));
 #pragma unroll
             for (int e = 0; e < 4; ++e) y[e] = ((keep >> e) & 1u) ? y[e] * p.act.keep_scale : 0.0f;
           }
           v[j] = make_float4(y[0], y[1], y[2], y[3]);
         }
-        ws::mbar_wait_relaxed(&bars.a_free[h], (tcount & 1u) ^ 1u);    // the MMAs that read these columns for the previous tile are done
-        ws::fence_after_sync();
+        tc::mbar_wait(&bars.a_free[h], (tcount & 1u) ^ 1u);    // the MMAs that read these columns for the previous tile are done
+        tc::fence_after_sync();
 #pragma unroll
         for (int part = 0; part < 2; ++part) {
           float hi[16], lo[16];
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
-            const float4 x = v[4 * part + j];
-            hi[4 * j + 0] = ws::tf32_hi(x.x); hi[4 * j + 1] = ws::tf32_hi(x.y); hi[4 * j + 2] = ws::tf32_hi(x.z); hi[4 * j + 3] = ws::tf32_hi(x.w);
-            lo[4 * j + 0] = x.x - hi[4 * j + 0]; lo[4 * j + 1] = x.y - hi[4 * j + 1]; lo[4 * j + 2] = x.z - hi[4 * j + 2]; lo[4 * j + 3] = x.w - hi[4 * j + 3];
+            float4 h, l;
+            tc::split4(v[4 * part + j], h, l);
+            hi[4 * j + 0] = h.x; hi[4 * j + 1] = h.y; hi[4 * j + 2] = h.z; hi[4 * j + 3] = h.w;
+            lo[4 * j + 0] = l.x; lo[4 * j + 1] = l.y; lo[4 * j + 2] = l.z; lo[4 * j + 3] = l.w;
           }
           const uint32_t col = (uint32_t)(32 * h + 16 * part);
-          ws::tmem_st<16>(lane_addr + kColAHi + col, hi);
-          ws::tmem_st<16>(lane_addr + kColALo + col, lo);
+          tc::tmem_st<16>(lane_addr + kColAHi + col, hi);
+          tc::tmem_st<16>(lane_addr + kColALo + col, lo);
         }
-        ws::tmem_st_wait();
-        ws::fence_before_sync();
-        ws::mbar_arrive(&bars.a_full[h]);
+        tc::tmem_st_wait();
+        tc::fence_before_sync();
+        tc::mbar_arrive(&bars.a_full[h]);
       }
     }
   } else if (warp >= kGathWarp0) {
@@ -250,7 +247,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
       }
     };
     if (gw == 0 && (long long)blockIdx.x < p.units) build_table(blockIdx.x, s_tab);
-    ws::named_sync(1, kGathThreads);
+    tc::named_sync(1, kGathThreads);
 
     for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
       const int* tab = s_tab + (ucount & 1u) * kTabInts;
@@ -258,12 +255,12 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
       const long long row0 = (long long)(uint32_t)tab[4] | ((long long)tab[5] << 32);
       // ---- drain: the unit's projected tiles, tensor memory -> P (rows of a subject start at a multiple of 8) ----
       for (int t = 0; t < tiles; ++t) {
-        ws::mbar_wait(&bars.d_full[t], uses[t] & 1u);
+        tc::mbar_wait(&bars.d_full[t], uses[t] & 1u);
         ++uses[t];
-        ws::fence_after_sync();
+        tc::fence_after_sync();
         float v[16];
-        ws::tmem_ld<16>(tmem + ((uint32_t)(32 * q) << 16) + kColD + (uint32_t)(kC * t + 16 * cg), v);
-        ws::tmem_ld_wait();
+        tc::tmem_ld<16>(tmem + ((uint32_t)(32 * q) << 16) + kColD + (uint32_t)(kC * t + 16 * cg), v);
+        tc::tmem_ld_wait();
         const int drow = t * kTR + 32 * q + lane;
         if (drow < rows) {
           int j = 0;
@@ -273,15 +270,15 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
           for (int k = 0; k < 4; ++k)
             *reinterpret_cast<float4*>(s_p + p_chunk_offset(prow, i, 4 * cg + k)) = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
         }
-        ws::fence_before_sync();
+        tc::fence_before_sync();
         __syncwarp();
-        if (lane == 0) ws::mbar_arrive(&bars.d_free[t]);
+        if (lane == 0) tc::mbar_arrive(&bars.d_free[t]);
       }
       const uint32_t b = ucount % (uint32_t)p.nblob;
-      ws::mbar_wait(&bars.blob_full[b], (ucount / (uint32_t)p.nblob) & 1u);
+      tc::mbar_wait(&bars.blob_full[b], (ucount / (uint32_t)p.nblob) & 1u);
       // the next unit's table goes into the other buffer now; it becomes visible at the barrier that ends this unit
       if (gw == 0 && u + gridDim.x < p.units) build_table(u + gridDim.x, s_tab + ((ucount + 1) & 1u) * kTabInts);
-      ws::named_sync(1, kGathThreads);            // P is complete
+      tc::named_sync(1, kGathThreads);            // P is complete
 
       // ---- gather: half a warp per row, pairs of rows in lock step -------------------------------------------------
       const int32_t* blob = reinterpret_cast<const int32_t*>(s_blob + (size_t)b * p.blob_cap_bytes);
@@ -353,9 +350,9 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
       }
       }
       __syncwarp();
-      if (lane == 0) ws::mbar_arrive(&bars.blob_free[b]);     // this warp has read its last record of the unit
+      if (lane == 0) tc::mbar_arrive(&bars.blob_free[b]);     // this warp has read its last record of the unit
       if (POOL) {
-        ws::named_sync(1, kGathThreads);          // every warp's partial sums are in place
+        tc::named_sync(1, kGathThreads);          // every warp's partial sums are in place
         const long long g0 = (long long)tab[6];
         for (int j = gw; j < nsub; j += kGathWarps) {
           // mean over the subject's rows (models.py:57-59)
@@ -366,7 +363,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
           }
         }
       }
-      ws::named_sync(1, kGathThreads);            // every warp is done with P: the next drain may overwrite it
+      tc::named_sync(1, kGathThreads);            // every warp is done with P: the next drain may overwrite it
     }
 
     // ---- BatchNorm statistics of this CTA: {count, mean[64], M2[64]} as doubles --------------------------------------
@@ -383,7 +380,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
           rec[gt * 9 + 5 + j] = (float)fmax((double)s2v[j] - (double)s1v[j] * m1, 0.0);
         }
       }
-      ws::named_sync(1, kGathThreads);
+      tc::named_sync(1, kGathThreads);
       double* out = p.partials + (size_t)blockIdx.x * (1 + 2 * kC);
       for (int c = gt; c < kC; c += kGathThreads) {
         const int qd = c >> 2, j = c & 3;
@@ -404,16 +401,16 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ w
     }
   }
 
-  ws::fence_before_sync();
+  tc::fence_before_sync();
   __syncthreads();
-  if (warp == kWarpAlloc) ws::tmem_dealloc(tmem, kTmemCols);
+  if (warp == kWarpAlloc) tc::tmem_dealloc(tmem, kTmemCols);
 }
 
 }  // namespace eng
 
 #ifndef CGNN_EMU
 // ---- host: tensor-map encoder through the runtime's driver entry point (no -lcuda) ---------------------------------
-namespace ws {
+namespace tc {
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -442,7 +439,7 @@ int make_tensor_map(TensorMap* m, const float* base, long long rows, int cols, i
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? CGNN_OK : CGNN_ERR_CUDA;
 }
-}  // namespace ws
+}  // namespace tc
 #endif
 
 // Returns CGNN_OK when launched (grid in *grid_out: the caller merges `partials`), -1 when the shape is not covered.
@@ -511,8 +508,8 @@ static int launch_ws(const float* t_in, const cgnn_act_t* act, const float* W, c
   }
   if (grid < 1) return -1;
   *grid_out = (int)grid;
-  ws::TensorMap tmap;
-  if (ws::make_tensor_map(&tmap, t_in, rows, kC, kTR) != CGNN_OK) return -1;
+  tc::TensorMap tmap;
+  if (tc::make_tensor_map(&tmap, t_in, rows, kC, kTR) != CGNN_OK) return -1;
   if (pool) {
     auto kfn = k_gcn_fwd_ws<true>;
     cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -2,7 +2,7 @@
 // network in eval mode): role layout, tensor-memory column plan, unit geometry, the P-tile swizzle.
 #pragma once
 #include "agg.cuh"
-#include "ws.cuh"
+#include "tc05.cuh"
 
 namespace cgnn {
 namespace eng {
@@ -58,13 +58,6 @@ __device__ __forceinline__ Unit unit_geom(const UnitSrc& p, long long u) {
   if (bytes > p.blob_cap_bytes) bytes = p.blob_cap_bytes;
   r.blob_bytes = (int)bytes;
   return r;
-}
-
-// keep bits of channel quad `quad` at a row (same stream as common.cuh::drop_keep)
-__device__ __forceinline__ uint32_t keep4(const Act& a, uint32_t row_hash, int quad) {
-  const uint32_t w0 = fmix32(row_hash + (uint32_t)quad * 0x632BE5ABu + a.k1), w1 = drop_second_word(w0);
-  return ((w0 & 0xffffu) >= a.thresh ? 1u : 0u) | ((w0 >> 16) >= a.thresh ? 2u : 0u) | ((w1 & 0xffffu) >= a.thresh ? 4u : 0u) |
-         ((w1 >> 16) >= a.thresh ? 8u : 0u);
 }
 
 // byte offset of 16-byte chunk c (0..15) of row `prow` of the P tile; `key` = the row's index inside its subject

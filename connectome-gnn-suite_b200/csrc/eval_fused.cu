@@ -67,11 +67,7 @@ __global__ void __launch_bounds__(256) k_eval_prep(PrepArgs p) {
     unsigned char* lo = hi + 2 * kC * 128;
     for (int idx = tid; idx < kC * (kC / 4); idx += blockDim.x) {
       const int n = idx / (kC / 4), k = (idx - n * (kC / 4)) * 4;
-      const float4 v = *reinterpret_cast<const float4*>(W + n * kC + k);
-      const float4 h = make_float4(ws::tf32_hi(v.x), ws::tf32_hi(v.y), ws::tf32_hi(v.z), ws::tf32_hi(v.w));
-      const uint32_t off = ws::kmajor_offset(n, k, kC);
-      *reinterpret_cast<float4*>(hi + off) = h;
-      *reinterpret_cast<float4*>(lo + off) = make_float4(v.x - h.x, v.y - h.y, v.z - h.z, v.w - h.w);
+      tc::store_split4(hi, lo, n, k, kC, *reinterpret_cast<const float4*>(W + n * kC + k));
     }
     return;
   }
@@ -96,7 +92,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
 #endif
   __shared__ EvalBarriers bars;
   __shared__ uint32_t tmem_base_s;
-  unsigned char* base = ws::smem_align1024(smem_raw);
+  unsigned char* base = tc::smem_align1024(smem_raw);
   unsigned char* w_hi = base;
   unsigned char* w_lo = base + 2 * kC * 128;
   unsigned char* s_ring = base + p.o_ring;          // [2 channel halves][128 rows][128 B], TMA-box swizzle
@@ -113,14 +109,14 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int L = p.L, NH = p.L - 1;
 
-  if (warp == kWarpAlloc) ws::tmem_alloc(&tmem_base_s, kTmemCols);
+  if (warp == kWarpAlloc) tc::tmem_alloc(&tmem_base_s, kTmemCols);
   if (tid == 0) {
-    ws::mbar_init(&bars.w_full, 1); ws::mbar_init(&bars.w_free, 1);
-    for (int i = 0; i < 2; ++i) { ws::mbar_init(&bars.ring_full[i], kGathWarps); ws::mbar_init(&bars.ring_free[i], 4 * 32); }
-    for (int i = 0; i < 2; ++i) { ws::mbar_init(&bars.a_full[i], 4 * 32); ws::mbar_init(&bars.a_free[i], 1); }
-    for (int i = 0; i < kMaxTiles; ++i) { ws::mbar_init(&bars.d_full[i], 1); ws::mbar_init(&bars.d_free[i], kGathWarps); }
-    for (int i = 0; i < 2; ++i) { ws::mbar_init(&bars.blob_full[i], 1); ws::mbar_init(&bars.blob_free[i], kGathWarps); }
-    ws::fence_mbar_init();
+    tc::mbar_init(&bars.w_full, 1); tc::mbar_init(&bars.w_free, 1);
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.ring_full[i], kGathWarps); tc::mbar_init(&bars.ring_free[i], 4 * 32); }
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.a_full[i], 4 * 32); tc::mbar_init(&bars.a_free[i], 1); }
+    for (int i = 0; i < kMaxTiles; ++i) { tc::mbar_init(&bars.d_full[i], 1); tc::mbar_init(&bars.d_free[i], kGathWarps); }
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.blob_full[i], 1); tc::mbar_init(&bars.blob_free[i], kGathWarps); }
+    tc::fence_mbar_init();
   }
   for (int c = tid; c < kC; c += kNT) s_b1[c] = p.b1 ? p.b1[c] : 0.0f;
   for (int i = tid; i < kC * kFeat; i += kNT) { const int k = i >> 6, c = i & 63; s_w1[i] = k < p.F ? p.W1[c * p.F + k] : 0.0f; }
@@ -134,24 +130,24 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
     for (int i = tid; i < K * M; i += kNT) wc[i] = p.Wc[i];
     for (int i = tid; i < K; i += kNT) bc[i] = p.bc[i];
   }
-  ws::fence_before_sync();
+  tc::fence_before_sync();
   __syncthreads();
-  ws::fence_after_sync();
+  tc::fence_after_sync();
   const uint32_t tmem = tmem_base_s;
 
   if (warp == kWarpTile) {
     // ================================ W loader =====================================================================
     if (lane == 0 && NH >= 1) {
       if (NH == 1) {                       // one hidden layer: its weights stay for the whole kernel
-        ws::mbar_arrive_expect_tx(&bars.w_full, kWImgBytes);
-        ws::bulk_load(w_hi, p.wimg, kWImgBytes, &bars.w_full);
+        tc::mbar_arrive_expect_tx(&bars.w_full, kWImgBytes);
+        tc::bulk_load(w_hi, p.wimg, kWImgBytes, &bars.w_full);
       } else {
         uint32_t wq = 0;
         for (long long u = blockIdx.x; u < p.units; u += gridDim.x)
           for (int hl = 0; hl < NH; ++hl, ++wq) {
-            ws::mbar_wait_relaxed(&bars.w_free, (wq & 1u) ^ 1u);    // the previous layer's MMAs no longer read the buffer
-            ws::mbar_arrive_expect_tx(&bars.w_full, kWImgBytes);
-            ws::bulk_load(w_hi, p.wimg + (size_t)hl * kWImgBytes, kWImgBytes, &bars.w_full);
+            tc::mbar_wait(&bars.w_free, (wq & 1u) ^ 1u);    // the previous layer's MMAs no longer read the buffer
+            tc::mbar_arrive_expect_tx(&bars.w_full, kWImgBytes);
+            tc::bulk_load(w_hi, p.wimg + (size_t)hl * kWImgBytes, kWImgBytes, &bars.w_full);
           }
       }
     }
@@ -162,40 +158,40 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
       for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
         const Unit un = unit_geom(p.src(), u);
         const uint32_t b = ucount % (uint32_t)p.nblob, use = ucount / (uint32_t)p.nblob;
-        ws::mbar_wait_relaxed(&bars.blob_free[b], (use & 1u) ^ 1u);
-        ws::mbar_arrive_expect_tx(&bars.blob_full[b], (uint32_t)un.blob_bytes);
-        ws::bulk_load(s_blob + (size_t)b * p.blob_cap_bytes, p.blob + un.blob_word0, (uint32_t)un.blob_bytes, &bars.blob_full[b]);
+        tc::mbar_wait(&bars.blob_free[b], (use & 1u) ^ 1u);
+        tc::mbar_arrive_expect_tx(&bars.blob_full[b], (uint32_t)un.blob_bytes);
+        tc::bulk_load(s_blob + (size_t)b * p.blob_cap_bytes, p.blob + un.blob_word0, (uint32_t)un.blob_bytes, &bars.blob_full[b]);
       }
     }
   } else if (warp == kWarpMma) {
     // ================================ MMA issuer ===================================================================
     if (lane == 0 && NH >= 1) {
-      const uint32_t idesc = ws::idesc_tf32(kTR, kC);
-      const uint64_t b_hi = ws::smem_desc_sw128(ws::smem_u32(w_hi)), b_lo = ws::smem_desc_sw128(ws::smem_u32(w_lo));
+      const uint32_t idesc = tc::idesc_tf32(kTR, kC);
+      const uint64_t b_hi = tc::smem_desc_sw128(tc::smem_u32(w_hi)), b_lo = tc::smem_desc_sw128(tc::smem_u32(w_lo));
       uint32_t tq = 0, wq = 0, uses[kMaxTiles] = {0, 0, 0};
       for (long long u = blockIdx.x; u < p.units; u += gridDim.x) {
         const Unit un = unit_geom(p.src(), u);
         for (int hl = 0; hl < NH; ++hl) {
-          if (NH > 1 || wq == 0) { ws::mbar_wait_relaxed(&bars.w_full, wq & 1u); ++wq; }
+          if (NH > 1 || wq == 0) { tc::mbar_wait(&bars.w_full, wq & 1u); ++wq; }
           for (int t = 0; t < un.tiles; ++t, ++tq) {
-            ws::mbar_wait_relaxed(&bars.d_free[t], (uses[t] & 1u) ^ 1u);
+            tc::mbar_wait(&bars.d_free[t], (uses[t] & 1u) ^ 1u);
             ++uses[t];
             const uint32_t d = tmem + kColD + (uint32_t)(kC * t);
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-              ws::mbar_wait_relaxed(&bars.a_full[h], tq & 1u);
-              ws::fence_after_sync();
+              tc::mbar_wait(&bars.a_full[h], tq & 1u);
+              tc::fence_after_sync();
 #pragma unroll
               for (int ks = 0; ks < 4; ++ks) {
                 const uint64_t bo = (uint64_t)((h * kC * 128 + ks * 32) >> 4);
                 const uint32_t ac = (uint32_t)(32 * h + 8 * ks);
-                ws::mma_tf32x3_ts(d, tmem + kColAHi + ac, tmem + kColALo + ac, b_hi + bo, b_lo + bo, idesc, (h | ks) ? 1u : 0u);
+                tc::mma_tf32x3_ts(d, tmem + kColAHi + ac, tmem + kColALo + ac, b_hi + bo, b_lo + bo, idesc, (h | ks) ? 1u : 0u);
               }
-              ws::mma_commit(&bars.a_free[h]);
+              tc::mma_commit(&bars.a_free[h]);
             }
-            ws::mma_commit(&bars.d_full[t]);
+            tc::mma_commit(&bars.d_full[t]);
           }
-          if (NH > 1) ws::mma_commit(&bars.w_free);     // fires when this layer's last MMA has read the weights
+          if (NH > 1) tc::mma_commit(&bars.w_free);     // fires when this layer's last MMA has read the weights
         }
       }
     }
@@ -210,29 +206,30 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
       const Unit un = unit_geom(p.src(), u);
       for (int hl = 0; hl < NH; ++hl)
         for (int t = 0; t < un.tiles; ++t, ++tq) {
-          ws::mbar_wait_relaxed(&bars.ring_full[h], tq & 1u);
+          tc::mbar_wait(&bars.ring_full[h], tq & 1u);
           float4 v[8];
 #pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const float4*>(slot + ws::box_chunk_offset(row, j));
-          ws::mbar_arrive(&bars.ring_free[h]);
-          ws::mbar_wait_relaxed(&bars.a_free[h], (tq & 1u) ^ 1u);
-          ws::fence_after_sync();
+          for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const float4*>(slot + tc::box_chunk_offset(row, j));
+          tc::mbar_arrive(&bars.ring_free[h]);
+          tc::mbar_wait(&bars.a_free[h], (tq & 1u) ^ 1u);
+          tc::fence_after_sync();
 #pragma unroll
           for (int part = 0; part < 2; ++part) {
             float hi[16], lo[16];
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
-              const float4 x = v[4 * part + j];
-              hi[4 * j + 0] = ws::tf32_hi(x.x); hi[4 * j + 1] = ws::tf32_hi(x.y); hi[4 * j + 2] = ws::tf32_hi(x.z); hi[4 * j + 3] = ws::tf32_hi(x.w);
-              lo[4 * j + 0] = x.x - hi[4 * j + 0]; lo[4 * j + 1] = x.y - hi[4 * j + 1]; lo[4 * j + 2] = x.z - hi[4 * j + 2]; lo[4 * j + 3] = x.w - hi[4 * j + 3];
+              float4 h, l;
+              tc::split4(v[4 * part + j], h, l);
+              hi[4 * j + 0] = h.x; hi[4 * j + 1] = h.y; hi[4 * j + 2] = h.z; hi[4 * j + 3] = h.w;
+              lo[4 * j + 0] = l.x; lo[4 * j + 1] = l.y; lo[4 * j + 2] = l.z; lo[4 * j + 3] = l.w;
             }
             const uint32_t col = (uint32_t)(32 * h + 16 * part);
-            ws::tmem_st<16>(lane_addr + kColAHi + col, hi);
-            ws::tmem_st<16>(lane_addr + kColALo + col, lo);
+            tc::tmem_st<16>(lane_addr + kColAHi + col, hi);
+            tc::tmem_st<16>(lane_addr + kColALo + col, lo);
           }
-          ws::tmem_st_wait();
-          ws::fence_before_sync();
-          ws::mbar_arrive(&bars.a_full[h]);
+          tc::tmem_st_wait();
+          tc::fence_before_sync();
+          tc::mbar_arrive(&bars.a_full[h]);
         }
     }
   } else if (warp >= kGathWarp0) {
@@ -270,7 +267,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
       }
     };
     if (gw == 0 && (long long)blockIdx.x < p.units) build_table(blockIdx.x, s_tab);
-    ws::named_sync(1, kGathThreads);
+    tc::named_sync(1, kGathThreads);
 
     for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
       const int* tab = s_tab + (ucount & 1u) * kTabInts;
@@ -283,9 +280,9 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
         s_x[idx] = k < p.F ? p.x[(row0 + r) * p.F + k] : 0.0f;
       }
       const uint32_t b = ucount % (uint32_t)p.nblob;
-      ws::mbar_wait(&bars.blob_full[b], (ucount / (uint32_t)p.nblob) & 1u);
+      tc::mbar_wait(&bars.blob_full[b], (ucount / (uint32_t)p.nblob) & 1u);
       if (gw == 0 && u + gridDim.x < p.units) build_table(u + gridDim.x, s_tab + ((ucount + 1) & 1u) * kTabInts);
-      ws::named_sync(1, kGathThreads);
+      tc::named_sync(1, kGathThreads);
       const int32_t* blob = reinterpret_cast<const int32_t*>(s_blob + (size_t)b * p.blob_cap_bytes);
 
       for (int l = 0; l < L; ++l) {          // l = 0: the narrow first layer; l >= 1: hidden layer over the P tile
@@ -293,12 +290,12 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
         if (l >= 1) {
           // ---- drain this layer's projected tiles, tensor memory -> P ------------------------------------------------
           for (int t = 0; t < tiles; ++t) {
-            ws::mbar_wait(&bars.d_full[t], uses[t] & 1u);
+            tc::mbar_wait(&bars.d_full[t], uses[t] & 1u);
             ++uses[t];
-            ws::fence_after_sync();
+            tc::fence_after_sync();
             float v[16];
-            ws::tmem_ld<16>(tmem + ((uint32_t)(32 * q) << 16) + kColD + (uint32_t)(kC * t + 16 * cg), v);
-            ws::tmem_ld_wait();
+            tc::tmem_ld<16>(tmem + ((uint32_t)(32 * q) << 16) + kColD + (uint32_t)(kC * t + 16 * cg), v);
+            tc::tmem_ld_wait();
             const int drow = t * kTR + 32 * q + lane;
             if (drow < rows) {
               int j = 0;
@@ -308,9 +305,9 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
               for (int k = 0; k < 4; ++k)
                 *reinterpret_cast<float4*>(s_p + p_chunk_offset(prow, i, 4 * cg + k)) = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
             }
-            ws::fence_before_sync();
+            tc::fence_before_sync();
             __syncwarp();
-            if (lane == 0) ws::mbar_arrive(&bars.d_free[t]);
+            if (lane == 0) tc::mbar_arrive(&bars.d_free[t]);
           }
         } else {
           // ---- first layer: P = x W1^T with plain FMAs (F <= 8 input channels), written like a drained tile ------------
@@ -335,7 +332,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
             }
           }
         }
-        ws::named_sync(1, kGathThreads);            // P is complete
+        tc::named_sync(1, kGathThreads);            // P is complete
         const float4 bq = l == 0 ? b1q : *reinterpret_cast<const float4*>(s_hb + (l - 1) * kC + 4 * cl);
         const float4 scq = *reinterpret_cast<const float4*>(s_aff + (2 * l) * kC + 4 * cl);
         const float4 shq = *reinterpret_cast<const float4*>(s_aff + (2 * l + 1) * kC + 4 * cl);
@@ -344,12 +341,12 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
           while (cur < t) {
             if (cur >= 0) {
               __syncwarp();
-              if (lane == 0) { ws::mbar_arrive(&bars.ring_full[0]); ws::mbar_arrive(&bars.ring_full[1]); }
+              if (lane == 0) { tc::mbar_arrive(&bars.ring_full[0]); tc::mbar_arrive(&bars.ring_full[1]); }
             }
             ++cur;
             const uint32_t par = ((rq + (uint32_t)cur) & 1u) ^ 1u;     // the converters have read the slot's previous tile
-            ws::mbar_wait(&bars.ring_free[0], par);
-            ws::mbar_wait(&bars.ring_free[1], par);
+            tc::mbar_wait(&bars.ring_free[0], par);
+            tc::mbar_wait(&bars.ring_free[1], par);
           }
         };
         for (int j = 0; j < nsub; ++j) {
@@ -407,7 +404,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
               const int t_mine = ur >> 7;
               const int t0 = __shfl_sync(kFull, t_mine, 0), t1 = __shfl_sync(kFull, t_mine, 16);
               const int hh = cl >> 3, jc = cl & 7, rr = ur & 127;
-              unsigned char* dst = s_ring + hh * kStageBytes + ws::box_chunk_offset(rr, jc);
+              unsigned char* dst = s_ring + hh * kStageBytes + tc::box_chunk_offset(rr, jc);
               advance_to(t0);
               if (valid && t_mine == t0) *reinterpret_cast<float4*>(dst) = uo;
               if (t1 != t0) {
@@ -426,15 +423,15 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
           advance_to(tiles - 1);
           if (cur >= 0) {
             __syncwarp();
-            if (lane == 0) { ws::mbar_arrive(&bars.ring_full[0]); ws::mbar_arrive(&bars.ring_full[1]); }
+            if (lane == 0) { tc::mbar_arrive(&bars.ring_full[0]); tc::mbar_arrive(&bars.ring_full[1]); }
           }
           rq += (uint32_t)tiles;
-          ws::named_sync(1, kGathThreads);          // every warp is done with P (and x): the next drain may overwrite it
+          tc::named_sync(1, kGathThreads);          // every warp is done with P (and x): the next drain may overwrite it
         }
       }
       __syncwarp();
-      if (lane == 0) ws::mbar_arrive(&bars.blob_free[b]);
-      ws::named_sync(1, kGathThreads);              // the readout partials are complete; P, x and the blob are free
+      if (lane == 0) tc::mbar_arrive(&bars.blob_free[b]);
+      tc::named_sync(1, kGathThreads);              // the readout partials are complete; P, x and the blob are free
 
       // ---- mean-pool readout and MLP head: one warp per subject ------------------------------------------------------
       {
@@ -468,13 +465,13 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
           __syncwarp();
         }
       }
-      ws::named_sync(1, kGathThreads);              // s_pool is rewritten by the next unit
+      tc::named_sync(1, kGathThreads);              // s_pool is rewritten by the next unit
     }
   }
 
-  ws::fence_before_sync();
+  tc::fence_before_sync();
   __syncthreads();
-  if (warp == kWarpAlloc) ws::tmem_dealloc(tmem, kTmemCols);
+  if (warp == kWarpAlloc) tc::tmem_dealloc(tmem, kTmemCols);
 }
 
 }  // namespace evf

@@ -150,7 +150,7 @@ __global__ void __launch_bounds__(NT, 2) k_first_fwd(FirstArgs p) {
       *reinterpret_cast<float4*>(p.z + (nb + r) * H + 4 * q) = make_float4(o[0], o[1], o[2], o[3]);
       if (want_stats) {        // BatchNorm batch statistics: training only
         cnt += 1;
-        const float inv = rt::rcp_fast((float)cnt);
+        const float inv = fast_rcp((float)cnt);
 #pragma unroll
         for (int j = 0; j < 4; ++j) wf[j].push(o[j], inv);
       }

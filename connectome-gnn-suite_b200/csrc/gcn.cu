@@ -187,19 +187,8 @@ struct GcnBwdArgs {
   int o_w, o_co, o_ci, o_dz, o_dp, o_u, o_raw, o_red, o_csr;
 };
 
-// Per-channel constant rows staged in shared memory.
-enum { CO_SCALE = 0, CO_SHIFT, CO_BSC, CO_MEAN, CO_RSTD, CO_S1N, CO_S2N, CO_ROWS };  // x H4
-enum { CI_SCALE = 0, CI_SHIFT, CI_MEAN, CI_RSTD, CI_ROWS };                          // x K4
-
-// dz of one element: dropout/ReLU backward of the upstream gradient, then BatchNorm backward.
-__device__ __forceinline__ float gcn_dz(const GcnBwdArgs& p, const float* s_co, int H4, bool aff_out, float t, float up,
-                                        uint32_t rh, int c) {
-  const float dy = act_bwd(p.act_out, aff_out, t, s_co[CO_SCALE * H4 + c], s_co[CO_SHIFT * H4 + c], rh, c, up);
-  if (!p.bn.has) return dy;
-  if (!p.bn.train) return s_co[CO_BSC * H4 + c] * dy;
-  const float xh = (t - s_co[CO_MEAN * H4 + c]) * s_co[CO_RSTD * H4 + c];
-  return s_co[CO_BSC * H4 + c] * (dy - s_co[CO_S1N * H4 + c] - xh * s_co[CO_S2N * H4 + c]);
-}
+// Per-channel constant rows of the layer input staged in shared memory.
+enum { CI_SCALE = 0, CI_SHIFT, CI_MEAN, CI_RSTD, CI_ROWS };   // x K4
 
 template <int HC, int MAXT>
 __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
@@ -207,7 +196,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
   CGNN_SMEM_DECL;
   float* sm = reinterpret_cast<float*>(cgnn_smem);
   float* s_w = sm + p.o_w;      // [H4][K4] natural layout, zero padded
-  float* s_co = sm + p.o_co;    // [CO_ROWS][H4]
+  float* s_co = sm + p.o_co;    // [DZ_ROWS][H4]
   float* s_ci = sm + p.o_ci;    // [CI_ROWS][K4]
   float* s_dz = sm + p.o_dz;    // [max_nodes][H4]
   float* s_dp = sm + p.o_dp;    // [kChunkRows][ldp]
@@ -225,15 +214,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
     const int h = idx / K4, k = idx - h * K4;
     s_w[idx] = (h < H && k < K) ? p.W[h * K + k] : 0.0f;
   }
-  stage_affine(p.act_out, H, H4, s_co + CO_SCALE * H4, s_co + CO_SHIFT * H4);
-  for (int c = tid; c < H4; c += kThreads) {
-    const bool ok = c < H && p.bn.has;
-    s_co[CO_BSC * H4 + c] = ok ? p.bn.scale[c] : (c < H ? 1.0f : 0.0f);
-    s_co[CO_MEAN * H4 + c] = ok ? p.bn.mean[c] : 0.0f;
-    s_co[CO_RSTD * H4 + c] = ok ? p.bn.rstd[c] : 0.0f;
-    s_co[CO_S1N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s1, p.bn.sums64, c, p.bn.inv_count) : 0.0f;
-    s_co[CO_S2N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s2, p.bn.sums64 ? p.bn.sums64 + H : nullptr, c, p.bn.inv_count) : 0.0f;
-  }
+  stage_dz_consts(p.act_out, p.bn, H, H4, s_co);
   stage_affine(p.act_in, K, K4, s_ci + CI_SCALE * K4, s_ci + CI_SHIFT * K4);
   for (int c = tid; c < K4; c += kThreads) {
     const bool ok = c < K && p.want_prev;
@@ -312,10 +293,10 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
             }
             const uint32_t rh = p.act_out.drop ? drop_row_hash(p.act_out, p.act_out.row_base + nb + i) : 0u;
             float4 o;
-            o.x = gcn_dz(p, s_co, H4, aff_out, zv[u].x, uv[u].x, rh, c);
-            o.y = gcn_dz(p, s_co, H4, aff_out, zv[u].y, uv[u].y, rh, c + 1);
-            o.z = gcn_dz(p, s_co, H4, aff_out, zv[u].z, uv[u].z, rh, c + 2);
-            o.w = gcn_dz(p, s_co, H4, aff_out, zv[u].w, uv[u].w, rh, c + 3);
+            o.x = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, zv[u].x, uv[u].x, rh, c);
+            o.y = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, zv[u].y, uv[u].y, rh, c + 1);
+            o.z = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, zv[u].z, uv[u].z, rh, c + 2);
+            o.w = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, zv[u].w, uv[u].w, rh, c + 3);
             *reinterpret_cast<float4*>(s_dz + i * H4 + c) = o;
           }
         }
@@ -328,7 +309,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
           const float t = p.z[(nb + i) * H + c];
           const float up = p.du ? p.du[(nb + i) * H + c] : p.demb[g * H + c] * inv_n;
           const uint32_t rh = p.act_out.drop ? drop_row_hash(p.act_out, p.act_out.row_base + nb + i) : 0u;
-          dz = gcn_dz(p, s_co, H4, aff_out, t, up, rh, c);
+          dz = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, t, up, rh, c);
         }
         s_dz[idx] = dz;
       }
@@ -673,7 +654,7 @@ int cgnn_gcn_layer_bwd(const float* du, const float* demb, const float* z, const
   if (a.H4 > 128 || ntiles_w > 4 * kThreads) return CGNN_ERR_TILE_TOO_LARGE;
   int off = 0;
   a.o_w = off; off += a.H4 * a.K4;
-  a.o_co = off; off += CO_ROWS * a.H4;
+  a.o_co = off; off += DZ_ROWS * a.H4;
   a.o_ci = off; off += CI_ROWS * a.K4;
   a.o_dz = off; off += a.max_nodes * a.H4;
   a.o_dp = off; off += kChunkRows * a.ldp;

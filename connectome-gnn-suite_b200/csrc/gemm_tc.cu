@@ -36,7 +36,7 @@ __device__ __forceinline__ void stage_weight_kmajor(const float* __restrict__ W,
     if (n < n_valid) v = rt::ld_quad<false>(W, n, ldw, 4 * q);
     v = rt::mask_quad(v, 4 * q, k_valid);
     float4 h, l;
-    rt::split4(v, h, l);
+    tc::split4(v, h, l);
     const uint32_t off = rt::kmajor_quad_offset(n, q, rows);
     rt::sts4(hi + off, h);
     rt::sts4(lo + off, l);
@@ -56,7 +56,7 @@ __device__ __forceinline__ void stage_weight_transposed(const float* __restrict_
       if (k + 3 < k_valid) v.w = W[(size_t)(k + 3) * ldw + n];
     }
     float4 h, l;
-    rt::split4(v, h, l);
+    tc::split4(v, h, l);
     const uint32_t off = rt::kmajor_quad_offset(n, q, rows);
     rt::sts4(hi + off, h);
     rt::sts4(lo + off, l);
@@ -100,7 +100,7 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
   const bool affine = p.act.scale != nullptr;
 
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, p.tmem_cols);
-  if (tid == 0) tc::mbar_init(&mbar, 1);
+  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::fence_mbar_init(); }
   stage_weight_kmajor(p.W, K, H, K, H, KP, b_hi, b_lo, NT);
   if (!WIDE) {
     for (int c = tid; c < KP; c += NT) { s_scale[c] = (c < C && p.act.scale) ? p.act.scale[c] : (c < C ? 1.0f : 0.0f); s_shift[c] = (c < C && p.act.scale) ? p.act.shift[c] : 0.0f; }
@@ -177,7 +177,7 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
         *reinterpret_cast<float4*>(p.z + (r0 + r) * H + 4 * qh) = v;
         if (want_stats) {      // BatchNorm batch statistics: training only
           cnt += 1;
-          const float inv = rt::rcp_fast((float)cnt);
+          const float inv = fast_rcp((float)cnt);
           wf[0].push(v.x, inv); wf[1].push(v.y, inv); wf[2].push(v.z, inv); wf[3].push(v.w, inv);
         }
       }
@@ -199,10 +199,10 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
       float4 h, l;
       if constexpr (WIDE) {
         const float4 u = live ? rt::act_fwd4(p.act, cq, pu[i], rk, (uint32_t)row) : make_float4(0.f, 0.f, 0.f, 0.f);
-        rt::split4(u, h, l);
+        tc::split4(u, h, l);
         rt::sts4(a_hi + koff_u + i * MC::RS * rt::kRowBytes, h);
         rt::sts4(a_lo + koff_u + i * MC::RS * rt::kRowBytes, l);
-        rt::split4(pa[i], h, l);
+        tc::split4(pa[i], h, l);
         rt::sts4(a_hi + koff_a + i * MC::RS * rt::kRowBytes, h);
         rt::sts4(a_lo + koff_a + i * MC::RS * rt::kRowBytes, l);
       } else if (4 * qc < K) {
@@ -213,7 +213,7 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
           const int kk = 4 * qc + j;
           if (live && kk < C) e[j] = act_fwd(p.act, affine, e[j], s_scale[kk], s_shift[kk], rhash, kk);
         }
-        rt::split4(make_float4(e[0], e[1], e[2], e[3]), h, l);
+        tc::split4(make_float4(e[0], e[1], e[2], e[3]), h, l);
         rt::sts4(a_hi + koff_u + i * MC::RS * rt::kRowBytes, h);
         rt::sts4(a_lo + koff_u + i * MC::RS * rt::kRowBytes, l);
       }
@@ -380,7 +380,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
   const bool aff_in = p.act_in.scale != nullptr;
 
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, p.tmem_cols);
-  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::mbar_init(&mbar_dw, 1); }
+  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::mbar_init(&mbar_dw, 1); tc::fence_mbar_init(); }
   stage_weight_transposed(p.W, Kin, Kin, H, KP, H, b1_hi, b1_lo);   // operand row n = input channel, k = h: W[h][n]
   stage_affine(p.act_in, Kin, KP, s_ci, s_ci + KP);
   if (!WIDE) {   // padded channels of the u operand stay zero
@@ -439,7 +439,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
 #pragma unroll
     for (int i = 0; i < M1::NQ; ++i) {
       float4 h, l;
-      rt::split4(dpn[i], h, l);
+      tc::split4(dpn[i], h, l);
       if (p.du_in) {
         rt::sts4(a1k_hi + koff1 + i * M1::RS * rt::kRowBytes, h);
         rt::sts4(a1k_lo + koff1 + i * M1::RS * rt::kRowBytes, l);
@@ -455,7 +455,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
         float4 u = make_float4(0.f, 0.f, 0.f, 0.f);
         if (row < p.rows) u = rt::mask_quad(rt::act_fwd4(p.act_in, cq, tin[i], rk, (uint32_t)row), c2, Kin);
         float4 h, l;
-        rt::split4(u, h, l);
+        tc::split4(u, h, l);
         rt::sts4(a2_hi + moff2 + i * M2::RS * rt::kRowBytes, h);
         rt::sts4(a2_lo + moff2 + i * M2::RS * rt::kRowBytes, l);
       }
@@ -520,7 +520,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
     constexpr int CW = KP / 4;
     const int q = warp & 3, cg = warp >> 2;
     float v[CW];
-    tc::tmem_ld_cols<CW>(taddr + ((uint32_t)(32 * q) << 16) + (uint32_t)(KP + cg * CW), v);
+    tc::tmem_ld<CW>(taddr + ((uint32_t)(32 * q) << 16) + (uint32_t)(KP + cg * CW), v);
+    tc::tmem_ld_wait();
     const int h = 32 * q + lane;
     if (h < H) {
 #pragma unroll
@@ -658,7 +659,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
   const bool need_du = p.direct != nullptr;
 
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, p.tmem_cols);
-  if (tid == 0) tc::mbar_init(&mbar, 1);
+  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::fence_mbar_init(); }
   // operand row j = column j of W [H][2C], contraction index = h
   stage_weight_transposed(p.W, K2, K2, H, MP, H, wk_hi, wk_lo);
   stage_affine(p.act_in, C, 32 * CB, s_ci, s_ci + 32 * CB);
@@ -745,7 +746,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
   auto store_du = [&](long long r0, uint32_t b) {
     const int lq = warp & 3, cg = warp >> 2;
     float v[16];
-    tc::tmem_ld_cols<16>(t_du + b * (uint32_t)TR + ((uint32_t)(32 * lq) << 16) + (uint32_t)(16 * cg), v);
+    tc::tmem_ld<16>(t_du + b * (uint32_t)TR + ((uint32_t)(32 * lq) << 16) + (uint32_t)(16 * cg), v);
+    tc::tmem_ld_wait();
     const int j = 32 * lq + lane;
     if (j < K2) {
       float* dst = (j < C ? p.direct + j : p.nbr + (j - C)) + (r0 + 16 * cg) * C;
@@ -779,7 +781,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
         colsum[0] += dz.x; colsum[1] += dz.y; colsum[2] += dz.z; colsum[3] += dz.w;
       }
       float4 h, l;
-      rt::split4(dz, h, l);
+      tc::split4(dz, h, l);
       if (need_du) {
         rt::sts4(dzk_hi + koff_z + i * MHq::RS * rt::kRowBytes, h);
         rt::sts4(dzk_lo + koff_z + i * MHq::RS * rt::kRowBytes, l);
@@ -795,10 +797,10 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
       float4 h, l;
       if constexpr (WIDE) {
         const float4 u = live ? rt::act_fwd4(p.act_in, cq_in, tq[i], rk_in, (uint32_t)row) : make_float4(0.f, 0.f, 0.f, 0.f);
-        rt::split4(u, h, l);
+        tc::split4(u, h, l);
         rt::sts4(ua_hi + moff_u + i * MCq::RS * rt::kRowBytes, h);
         rt::sts4(ua_lo + moff_u + i * MCq::RS * rt::kRowBytes, l);
-        rt::split4(aq[i], h, l);
+        tc::split4(aq[i], h, l);
         rt::sts4(ua_hi + moff_a + i * MCq::RS * rt::kRowBytes, h);
         rt::sts4(ua_lo + moff_a + i * MCq::RS * rt::kRowBytes, l);
       } else if (4 * qc < K2) {
@@ -809,7 +811,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
           const int kk = 4 * qc + j;
           if (live && kk < C) e[j] = act_fwd(p.act_in, aff_in, e[j], s_ci[kk], s_ci[32 * CB + kk], rhash, kk);
         }
-        rt::split4(make_float4(e[0], e[1], e[2], e[3]), h, l);
+        tc::split4(make_float4(e[0], e[1], e[2], e[3]), h, l);
         rt::sts4(ua_hi + moff_u + i * MCq::RS * rt::kRowBytes, h);
         rt::sts4(ua_lo + moff_u + i * MCq::RS * rt::kRowBytes, l);
       }
@@ -845,7 +847,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
     constexpr int CW = H / 4;
     const int lq = warp & 3, cg = warp >> 2;
     float v[CW];
-    tc::tmem_ld_cols<CW>(t_dw + ((uint32_t)(32 * lq) << 16) + (uint32_t)(cg * CW), v);
+    tc::tmem_ld<CW>(t_dw + ((uint32_t)(32 * lq) << 16) + (uint32_t)(cg * CW), v);
+    tc::tmem_ld_wait();
     const int j = 32 * lq + lane;
     if (j < K2) {
 #pragma unroll

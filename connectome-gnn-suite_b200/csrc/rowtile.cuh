@@ -11,12 +11,6 @@
 namespace cgnn {
 namespace rt {
 
-__device__ __forceinline__ float rcp_fast(float x) {
-  float r;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-  return r;
-}
-
 // thread <-> (quad column q, first row r) for a tile of TR rows x 4*Q channels; Q in {8, 16, 32}
 template <int Q, int TR, int NT = kThreads>
 struct QuadMap {
@@ -36,16 +30,12 @@ __device__ __forceinline__ uint32_t mnmajor_quad_offset(int row, int q, int rows
 // advancing a thread's row by RS (a multiple of 8) moves either offset by RS * 128 bytes
 constexpr uint32_t kRowBytes = 128;
 
-__device__ __forceinline__ void split4(float4 v, float4& h, float4& l) {
-  h = make_float4(tc::tf32_hi(v.x), tc::tf32_hi(v.y), tc::tf32_hi(v.z), tc::tf32_hi(v.w));
-  l = make_float4(v.x - h.x, v.y - h.y, v.z - h.z, v.w - h.w);
-}
 __device__ __forceinline__ void sts4(unsigned char* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 
 // ---- per-thread constants of one channel quad of an Act ---------------------------------------------------------
 struct ChanQuad {
   float sc[4], sh[4];
-  uint32_t ck;         // dropout: (c >> 2) * 0x632BE5AB + k1 of this quad
+  uint32_t ck;         // dropout: drop_quad_key of this quad
 };
 __device__ __forceinline__ void chan_quad_init(ChanQuad& cq, const Act& a, int c0, int C) {
 #pragma unroll
@@ -54,7 +44,7 @@ __device__ __forceinline__ void chan_quad_init(ChanQuad& cq, const Act& a, int c
     cq.sc[j] = ok ? a.scale[c0 + j] : 1.0f;
     cq.sh[j] = ok ? a.shift[c0 + j] : 0.0f;
   }
-  cq.ck = (uint32_t)(c0 >> 2) * 0x632BE5ABu + a.k1;
+  cq.ck = drop_quad_key(a, c0 >> 2);
 }
 // Dropout row key: the per-row hash of common.cuh::drop_row_hash for global row ids (row_base + row) computed from
 // 32-bit pieces - the high word's hash is formed once per kernel (and once more for rows behind a 2^32 boundary).
@@ -75,13 +65,6 @@ __device__ __forceinline__ uint32_t row_hash_at(const Act& a, const RowKey& k, u
   const uint32_t hh = lo >= k.lo0 ? k.hh0 : k.hh1;
   return (lo * 0x9E3779B1u) ^ a.k0 ^ hh;
 }
-// keep masks of the quad's 4 channels at row `row` of the batch (bit j = channel c0 + j kept); same stream as drop_keep()
-__device__ __forceinline__ uint32_t drop_keep4(const Act& a, const ChanQuad& cq, const RowKey& rk, uint32_t row) {
-  const uint32_t rh = row_hash_at(a, rk, row);
-  const uint32_t w0 = fmix32(rh + cq.ck), w1 = drop_second_word(w0);
-  return ((w0 & 0xffffu) >= a.thresh ? 1u : 0u) | ((w0 >> 16) >= a.thresh ? 2u : 0u) |
-         ((w1 & 0xffffu) >= a.thresh ? 4u : 0u) | ((w1 >> 16) >= a.thresh ? 8u : 0u);
-}
 // u = dropout(relu?(sc t + sh)) on the quad
 __device__ __forceinline__ float4 act_fwd4(const Act& a, const ChanQuad& cq, float4 t, const RowKey& rk, uint32_t row) {
   float y[4] = {t.x, t.y, t.z, t.w};
@@ -94,7 +77,7 @@ __device__ __forceinline__ float4 act_fwd4(const Act& a, const ChanQuad& cq, flo
     for (int j = 0; j < 4; ++j) y[j] = fmaxf(y[j], 0.0f);
   }
   if (a.drop) {
-    const uint32_t keep = drop_keep4(a, cq, rk, row);
+    const uint32_t keep = drop_keep4(a, row_hash_at(a, rk, row), cq.ck);
 #pragma unroll
     for (int j = 0; j < 4; ++j) y[j] = ((keep >> j) & 1u) ? y[j] * a.keep_scale : 0.0f;
   }
@@ -113,7 +96,7 @@ __device__ __forceinline__ float4 act_bwd4(const Act& a, const ChanQuad& cq, flo
     }
   }
   if (a.drop) {
-    pass &= drop_keep4(a, cq, rk, row);
+    pass &= drop_keep4(a, row_hash_at(a, rk, row), cq.ck);
 #pragma unroll
     for (int j = 0; j < 4; ++j) d[j] *= a.keep_scale;
   }
@@ -122,34 +105,20 @@ __device__ __forceinline__ float4 act_bwd4(const Act& a, const ChanQuad& cq, flo
   return make_float4(d[0], d[1], d[2], d[3]);
 }
 
-// BatchNorm-backward coefficients of one channel quad:  dz = bsc * (dy - s1n - xhat * s2n), xhat = (t - mean) * rstd
+// BatchNorm-backward coefficients of one channel quad
 struct BnQuad {
-  float bsc[4], mean[4], rstd[4], s1n[4], s2n[4];
+  BnCoef k[4];
 };
 __device__ __forceinline__ void bn_quad_init(BnQuad& b, const BnBwdDev& bn, int c0, int C) {
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const bool ok = bn.has && c0 + j < C;
-    b.bsc[j] = ok ? bn.scale[c0 + j] : 1.0f;
-    b.mean[j] = ok ? bn.mean[c0 + j] : 0.0f;
-    b.rstd[j] = ok ? bn.rstd[c0 + j] : 0.0f;
-    b.s1n[j] = (ok && bn.train) ? bn_sum_over_count(bn.s1, bn.sums64, c0 + j, bn.inv_count) : 0.0f;
-    b.s2n[j] = (ok && bn.train) ? bn_sum_over_count(bn.s2, bn.sums64 ? bn.sums64 + C : nullptr, c0 + j, bn.inv_count) : 0.0f;
-  }
+  for (int j = 0; j < 4; ++j) b.k[j] = bn_bwd_coef(bn, c0 + j, C);
 }
 __device__ __forceinline__ float4 bn_bwd4(const BnBwdDev& bn, const BnQuad& b, float4 t, float4 dy) {
   if (!bn.has) return dy;
   const float tv[4] = {t.x, t.y, t.z, t.w};
   float d[4] = {dy.x, dy.y, dy.z, dy.w};
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    if (bn.train) {
-      const float xh = (tv[j] - b.mean[j]) * b.rstd[j];
-      d[j] = b.bsc[j] * (d[j] - b.s1n[j] - xh * b.s2n[j]);
-    } else {
-      d[j] = b.bsc[j] * d[j];
-    }
-  }
+  for (int j = 0; j < 4; ++j) d[j] = bn.train ? bn_bwd_dz(b.k[j], tv[j], d[j]) : b.k[j].bsc * d[j];
   return make_float4(d[0], d[1], d[2], d[3]);
 }
 
@@ -192,7 +161,8 @@ __device__ __forceinline__ void drain_rows_to_staging(uint32_t taddr, float4* st
   constexpr int CW = NC / (NT / 128);   // columns per warp: 4 lane quarters x NT / 128 column groups
   const int lq = warp & 3, cg = warp >> 2, row = 32 * lq + lane;
   float v[CW];
-  tc::tmem_ld_cols<CW>(taddr + ((uint32_t)(32 * lq) << 16) + (uint32_t)(cg * CW), v);
+  tc::tmem_ld<CW>(taddr + ((uint32_t)(32 * lq) << 16) + (uint32_t)(cg * CW), v);
+  tc::tmem_ld_wait();
 #pragma unroll
   for (int j = 0; j < CW / 4; ++j)
     stage[stage_index(row, cg * (CW / 4) + j, NC / 4)] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);

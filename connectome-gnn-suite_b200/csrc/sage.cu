@@ -36,17 +36,14 @@ __device__ __forceinline__ void sage_cat_rows(const float* s_u, int K4, float* s
   }
 }
 
-// Whole-subject input tile: async raw copy into s_u (row stride K), CSR alongside; then the previous layer's
-// BatchNorm/dropout in place (row stride becomes K4 only when K == K4, otherwise a strided rewrite back to front).
-__device__ __forceinline__ void sage_transform_tile(float* s_u, int n, int K, int K4, const Act& act, const float* s_scale,
-                                                    const float* s_shift, long long nb) {
+// Whole-subject input tile of K % 4 == 0 channels, copied raw into s_u: the previous layer's BatchNorm/dropout in place.
+__device__ __forceinline__ void sage_transform_tile(float* s_u, int n, int K, const Act& act, const float* s_scale, const float* s_shift,
+                                                    long long nb) {
   const bool affine = act.scale != nullptr;
-  if (K == K4) {
-    for (int idx = threadIdx.x; idx < n * K4; idx += blockDim.x) {
-      const int r = idx / K4, c = idx - r * K4;
-      const uint32_t rh = act.drop ? drop_row_hash(act, act.row_base + nb + r) : 0u;
-      s_u[idx] = act_fwd(act, affine, s_u[idx], s_scale[c], s_shift[c], rh, c);
-    }
+  for (int idx = threadIdx.x; idx < n * K; idx += blockDim.x) {
+    const int r = idx / K, c = idx - r * K;
+    const uint32_t rh = act.drop ? drop_row_hash(act, act.row_base + nb + r) : 0u;
+    s_u[idx] = act_fwd(act, affine, s_u[idx], s_scale[c], s_shift[c], rh, c);
   }
 }
 
@@ -119,7 +116,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_fwd(SageFwdArgs p) {
     cp_async_wait<0>();
     __syncthreads();
     if (K == K4) {
-      sage_transform_tile(s_u, n, K, K4, p.act, s_scale, s_shift, nb);
+      sage_transform_tile(s_u, n, K, p.act, s_scale, s_shift, nb);
       __syncthreads();
     }
     const float* wsum_g = p.wsum + nb;
@@ -188,21 +185,10 @@ struct SageBwdArgs {
   int o_w, o_co, o_ci, o_u, o_cat, o_dq, o_red, o_csr;
 };
 
-enum { SO_SCALE = 0, SO_SHIFT, SO_BSC, SO_MEAN, SO_RSTD, SO_S1N, SO_S2N, SO_ROWS };
-
 // dq of one element: dropout backward, BatchNorm backward, ReLU mask of the layer's own output.
 __device__ __forceinline__ float sage_dq(const SageBwdArgs& p, const float* s_co, int H4, bool aff_out, float t, float up,
                                          uint32_t rh, int c) {
-  const float dy = act_bwd(p.act_out, aff_out, t, s_co[SO_SCALE * H4 + c], s_co[SO_SHIFT * H4 + c], rh, c, up);
-  float dz = dy;
-  if (p.bn.has) {
-    if (p.bn.train) {
-      const float xh = (t - s_co[SO_MEAN * H4 + c]) * s_co[SO_RSTD * H4 + c];
-      dz = s_co[SO_BSC * H4 + c] * (dy - s_co[SO_S1N * H4 + c] - xh * s_co[SO_S2N * H4 + c]);
-    } else {
-      dz = s_co[SO_BSC * H4 + c] * dy;
-    }
-  }
+  const float dz = staged_dz(p.act_out, p.bn, s_co, H4, aff_out, t, up, rh, c);
   return t > 0.0f ? dz : 0.0f;
 }
 
@@ -212,7 +198,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
   CGNN_SMEM_DECL;
   float* sm = reinterpret_cast<float*>(cgnn_smem);
   float* s_w = sm + p.o_w;      // [H4][2*K4] natural layout
-  float* s_co = sm + p.o_co;    // [SO_ROWS][H4]
+  float* s_co = sm + p.o_co;    // [DZ_ROWS][H4]
   float* s_ci = sm + p.o_ci;    // [2][K4] scale, shift of act_in
   float* s_u = sm + p.o_u;      // [max_nodes][K4]
   float* s_cat = sm + p.o_cat;  // [kChunkRows][ldc]
@@ -229,15 +215,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
     const int half = kk >= K4, k = kk - half * K4;
     s_w[idx] = (h < H && k < K) ? p.W[h * 2 * K + half * K + k] : 0.0f;
   }
-  stage_affine(p.act_out, H, H4, s_co + SO_SCALE * H4, s_co + SO_SHIFT * H4);
-  for (int c = tid; c < H4; c += kThreads) {
-    const bool ok = c < H && p.bn.has;
-    s_co[SO_BSC * H4 + c] = ok ? p.bn.scale[c] : (c < H ? 1.0f : 0.0f);
-    s_co[SO_MEAN * H4 + c] = ok ? p.bn.mean[c] : 0.0f;
-    s_co[SO_RSTD * H4 + c] = ok ? p.bn.rstd[c] : 0.0f;
-    s_co[SO_S1N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s1, p.bn.sums64, c, p.bn.inv_count) : 0.0f;
-    s_co[SO_S2N * H4 + c] = (ok && p.bn.train) ? bn_sum_over_count(p.bn.s2, p.bn.sums64 ? p.bn.sums64 + H : nullptr, c, p.bn.inv_count) : 0.0f;
-  }
+  stage_dz_consts(p.act_out, p.bn, H, H4, s_co);
   stage_affine(p.act_in, K, K4, s_ci, s_ci + K4);
   __syncthreads();
 
@@ -281,7 +259,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
     cp_async_wait<0>();
     __syncthreads();
     if (K == K4) {
-      sage_transform_tile(s_u, n, K, K4, p.act_in, s_ci, s_ci + K4, nb);
+      sage_transform_tile(s_u, n, K, p.act_in, s_ci, s_ci + K4, nb);
       __syncthreads();
     }
     const float* wsum_g = p.wsum + nb;
@@ -719,7 +697,7 @@ int cgnn_sage_layer_bwd(const float* du, const float* demb, const float* z, cons
   if (a.H4 > 128 || a.K4 > 128 || ntiles_w > 4 * kThreads) return CGNN_ERR_TILE_TOO_LARGE;
   int off = 0;
   a.o_w = off; off += a.H4 * 2 * a.K4;
-  a.o_co = off; off += SO_ROWS * a.H4;
+  a.o_co = off; off += DZ_ROWS * a.H4;
   a.o_ci = off; off += 2 * a.K4;
   a.o_u = off; off += a.max_nodes * a.K4;
   a.o_cat = off; off += kChunkRows * a.ldc;

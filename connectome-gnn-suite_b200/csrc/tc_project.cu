@@ -27,7 +27,7 @@ __global__ void __launch_bounds__(128) k_project_tf32x3(const float* __restrict_
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long long r0 = (long long)blockIdx.x * kTcRows;
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, tmem_cols);
-  if (tid == 0) tc::mbar_init(&mbar, 1);
+  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::fence_mbar_init(); }
 
   const int q = K >> 2;
   for (int idx = tid; idx < kTcRows * q; idx += blockDim.x) {
@@ -54,7 +54,8 @@ __global__ void __launch_bounds__(128) k_project_tf32x3(const float* __restrict_
   const long long row = r0 + 32 * warp + lane;
   for (int c0 = 0; c0 < N; c0 += 32) {
     float v[32];
-    tc::tmem_ld32(taddr + ((uint32_t)(32 * warp) << 16) + (uint32_t)c0, v);
+    tc::tmem_ld<32>(taddr + ((uint32_t)(32 * warp) << 16) + (uint32_t)c0, v);
+    tc::tmem_ld_wait();
     if (row < rows) {
 #pragma unroll
       for (int j = 0; j < 32; j += 4)
@@ -83,7 +84,7 @@ __global__ void __launch_bounds__(128) k_project_tf32x3_ts(const float* __restri
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long long r0 = (long long)blockIdx.x * kTcRows;
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, tmem_cols);
-  if (tid == 0) tc::mbar_init(&mbar, 1);
+  if (tid == 0) { tc::mbar_init(&mbar, 1); tc::fence_mbar_init(); }
   const int q = K >> 2;
   for (int idx = tid; idx < N * q; idx += blockDim.x) {
     const int n = idx / q, k = (idx - n * q) << 2;
@@ -106,8 +107,8 @@ __global__ void __launch_bounds__(128) k_project_tf32x3_ts(const float* __restri
     float h[8], l[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) { h[j] = tc::tf32_hi(v[j]); l[j] = v[j] - h[j]; }
-    tc::tmem_st8(lane_base + (uint32_t)(N + k), h);
-    tc::tmem_st8(lane_base + (uint32_t)(N + K + k), l);
+    tc::tmem_st<8>(lane_base + (uint32_t)(N + k), h);
+    tc::tmem_st<8>(lane_base + (uint32_t)(N + K + k), l);
   }
   tc::tmem_st_wait();
   tc::fence_before_sync();
@@ -120,9 +121,7 @@ __global__ void __launch_bounds__(128) k_project_tf32x3_ts(const float* __restri
     for (int k = 0; k < K; k += 8) {
       const uint32_t kb = (uint32_t)(k >> 5), ko = (uint32_t)((k & 31) * 4);
       const uint64_t dh = tc::smem_desc_sw128(bh + kb * (uint32_t)N * 128u + ko), dl = tc::smem_desc_sw128(bl + kb * (uint32_t)N * 128u + ko);
-      tc::mma_tf32_ts(taddr, taddr + (uint32_t)(N + K + k), dh, idesc, acc);   // lo * hi
-      tc::mma_tf32_ts(taddr, taddr + (uint32_t)(N + k), dl, idesc, 1u);        // hi * lo
-      tc::mma_tf32_ts(taddr, taddr + (uint32_t)(N + k), dh, idesc, 1u);        // hi * hi
+      tc::mma_tf32x3_ts(taddr, taddr + (uint32_t)(N + k), taddr + (uint32_t)(N + K + k), dh, dl, idesc, acc);
       acc = 1;
     }
     tc::mma_commit(&mbar);
@@ -131,7 +130,8 @@ __global__ void __launch_bounds__(128) k_project_tf32x3_ts(const float* __restri
   tc::fence_after_sync();
   for (int c0 = 0; c0 < N; c0 += 32) {
     float v[32];
-    tc::tmem_ld32(lane_base + (uint32_t)c0, v);
+    tc::tmem_ld<32>(lane_base + (uint32_t)c0, v);
+    tc::tmem_ld_wait();
     if (row < rows) {
 #pragma unroll
       for (int j = 0; j < 32; j += 4)

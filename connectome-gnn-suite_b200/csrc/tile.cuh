@@ -1,6 +1,5 @@
-// tile.cuh - building blocks shared by the GCN / GraphSAGE layer kernels: staging rows of an
-// activation tensor into shared memory with the previous layer's BatchNorm+ReLU+dropout applied,
-// per-channel constant staging, Welford statistics epilogue.
+// tile.cuh - building blocks shared by the GCN / GraphSAGE layer kernels: per-channel constant staging, the output
+// gradient of the backward kernels, Welford statistics epilogue, CSR rows in shared memory.
 #pragma once
 #include "common.cuh"
 
@@ -17,44 +16,27 @@ __device__ __forceinline__ void stage_affine(const Act& a, int C, int C4, float*
   }
 }
 
-// Stage `R` rows x C4 channels into dst[r*ld + c]: rows [0, rows) come from t[(grow0 + r)*C + c]
-// (global row ids, row stride C) with act applied; rows >= `rows` and channels >= C are zero.
-// If raw != nullptr the untransformed values are stored there too (same layout).
-// VEC: C % 4 == 0 and 16-byte aligned rows -> float4 loads.
-template <bool VEC>
-__device__ __forceinline__ void stage_rows(const float* __restrict__ t, long long grow0, int rows, int R, int C,
-                                           int C4, int ld, const Act& a, const float* s_scale,
-                                           const float* s_shift, float* dst, float* raw) {
-  const bool affine = a.scale != nullptr;
-  if (VEC) {
-    const int q4 = C4 >> 2;
-    for (int idx = threadIdx.x; idx < R * q4; idx += blockDim.x) {
-      const int r = idx / q4, c = (idx - r * q4) << 2;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f), rv = v;
-      if (r < rows) {
-        rv = *reinterpret_cast<const float4*>(t + (grow0 + r) * C + c);
-        const uint32_t rh = a.drop ? drop_row_hash(a, a.row_base + grow0 + r) : 0u;
-        v.x = act_fwd(a, affine, rv.x, s_scale[c], s_shift[c], rh, c);
-        v.y = act_fwd(a, affine, rv.y, s_scale[c + 1], s_shift[c + 1], rh, c + 1);
-        v.z = act_fwd(a, affine, rv.z, s_scale[c + 2], s_shift[c + 2], rh, c + 2);
-        v.w = act_fwd(a, affine, rv.w, s_scale[c + 3], s_shift[c + 3], rh, c + 3);
-      }
-      *reinterpret_cast<float4*>(dst + r * ld + c) = v;
-      if (raw) *reinterpret_cast<float4*>(raw + r * ld + c) = rv;
-    }
-  } else {
-    for (int idx = threadIdx.x; idx < R * C4; idx += blockDim.x) {
-      const int r = idx / C4, c = idx - r * C4;
-      float v = 0.0f, rv = 0.0f;
-      if (r < rows && c < C) {
-        rv = t[(grow0 + r) * C + c];
-        const uint32_t rh = a.drop ? drop_row_hash(a, a.row_base + grow0 + r) : 0u;
-        v = act_fwd(a, affine, rv, s_scale[c], s_shift[c], rh, c);
-      }
-      dst[r * ld + c] = v;
-      if (raw) raw[r * ld + c] = rv;
-    }
+// Per-channel constants of the output gradient dz of a GCN / GraphSAGE backward, [DZ_ROWS][H4] in shared memory: the
+// output activation's affine map and the BatchNorm-backward coefficients.  CTAs of kThreads; caller syncs.
+enum { DZ_SCALE = 0, DZ_SHIFT, DZ_BSC, DZ_MEAN, DZ_RSTD, DZ_S1N, DZ_S2N, DZ_ROWS };
+__device__ __forceinline__ void stage_dz_consts(const Act& act_out, const BnBwdDev& bn, int H, int H4, float* s) {
+  stage_affine(act_out, H, H4, s + DZ_SCALE * H4, s + DZ_SHIFT * H4);
+  for (int c = threadIdx.x; c < H4; c += kThreads) {
+    const BnCoef k = bn_bwd_coef(bn, c, H);
+    s[DZ_BSC * H4 + c] = k.bsc;
+    s[DZ_MEAN * H4 + c] = k.mean;
+    s[DZ_RSTD * H4 + c] = k.rstd;
+    s[DZ_S1N * H4 + c] = k.s1n;
+    s[DZ_S2N * H4 + c] = k.s2n;
   }
+}
+// dz of one element: dropout/ReLU backward of the upstream gradient, then BatchNorm backward
+__device__ __forceinline__ float staged_dz(const Act& act_out, const BnBwdDev& bn, const float* s, int H4, bool aff_out, float t,
+                                           float up, uint32_t rh, int c) {
+  const float dy = act_bwd(act_out, aff_out, t, s[DZ_SCALE * H4 + c], s[DZ_SHIFT * H4 + c], rh, c, up);
+  if (!bn.has) return dy;
+  if (!bn.train) return s[DZ_BSC * H4 + c] * dy;
+  return bn_bwd_dz(BnCoef{s[DZ_MEAN * H4 + c], s[DZ_RSTD * H4 + c], s[DZ_BSC * H4 + c], s[DZ_S1N * H4 + c], s[DZ_S2N * H4 + c]}, t, dy);
 }
 
 // Per-warp running Welford state for HC channels per lane (channel = lane + 32*j).

@@ -61,7 +61,7 @@ __global__ void __launch_bounds__(256) k_wide_prep_w(const float* __restrict__ W
       v = *reinterpret_cast<const float4*>(W + (size_t)n * ldw + 4 * q);
     }
     float4 h, l;
-    rt::split4(v, h, l);
+    tc::split4(v, h, l);
     const size_t off = (size_t)(q >> 3) * (2 * W_B_HALF) + rt::kmajor_quad_offset(n, q & 7, WN);
     *reinterpret_cast<float4*>(img + off) = h;
     *reinterpret_cast<float4*>(img + off + W_B_HALF) = l;
@@ -85,7 +85,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
   if (warp == 0) tc::tmem_alloc(&tmem_base_s, 512);
-  if (tid == 0) { tc::mbar_init(&mbar[0], 1); tc::mbar_init(&mbar[1], 1); }
+  if (tid == 0) { tc::mbar_init(&mbar[0], 1); tc::mbar_init(&mbar[1], 1); tc::fence_mbar_init(); }
   tc::fence_before_sync();
   __syncthreads();
   tc::fence_after_sync();
@@ -143,7 +143,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
     constexpr int J = decltype(JC)::value;
     const int lq = warp & 3, cg = warp >> 2, row = 32 * lq + lane;
     float v[16];
-    tc::tmem_ld_cols<16>(taddr + ((uint32_t)(32 * lq) << 16) + pend_buf * (uint32_t)WN + (uint32_t)(J * W_SLAB + cg * 16), v);
+    tc::tmem_ld<16>(taddr + ((uint32_t)(32 * lq) << 16) + pend_buf * (uint32_t)WN + (uint32_t)(J * W_SLAB + cg * 16), v);
+    tc::tmem_ld_wait();
 #pragma unroll
     for (int j = 0; j < 4; ++j)
       staging[rt::stage_index(row, 4 * cg + j, W_SLAB / 4)] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
@@ -159,7 +160,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
         *reinterpret_cast<float4*>(p.out + (pend_r0 + r) * WN + J * W_SLAB + 4 * qs) = x;
         if (want_stats) {
           cnt[J] += 1;
-          const float inv = rt::rcp_fast((float)cnt[J]);
+          const float inv = fast_rcp((float)cnt[J]);
           wf[J][0].push(x.x, inv); wf[J][1].push(x.y, inv); wf[J][2].push(x.z, inv); wf[J][3].push(x.w, inv);
         }
       }
@@ -186,7 +187,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
 #pragma unroll
     for (int i = 0; i < 2; ++i) {
       float4 h, l;
-      rt::split4(pa[i], h, l);
+      tc::split4(pa[i], h, l);
       rt::sts4(a_hi + koff + i * 64 * rt::kRowBytes, h);
       rt::sts4(a_lo + koff + i * 64 * rt::kRowBytes, l);
     }
@@ -275,6 +276,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
   if (tid == 0) {
 #pragma unroll
     for (int s = 0; s < X_STAGES; ++s) tc::mbar_init(&mbar[s], 1);
+    tc::fence_mbar_init();
   }
   tc::fence_before_sync();
   __syncthreads();
@@ -325,7 +327,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
     for (int i = 0; i < 2; ++i) {
       const long long row = c * XR + r + 8 * i;
       float4 h, l;
-      rt::split4(dp[i], h, l);
+      tc::split4(dp[i], h, l);
       rt::sts4(a_hi + moff + i * 8 * rt::kRowBytes, h);
       rt::sts4(a_hi + X_HALF + moff + i * 8 * rt::kRowBytes, l);
       float4 u = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -341,7 +343,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
           }
         }
       }
-      rt::split4(u, h, l);
+      tc::split4(u, h, l);
       rt::sts4(a_hi + 2 * X_HALF + moff + i * 8 * rt::kRowBytes, h);
       rt::sts4(a_hi + 3 * X_HALF + moff + i * 8 * rt::kRowBytes, l);
     }
@@ -376,7 +378,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
         float v[32];
         const int c0 = cg * 64 + sub * 32;
         if (issued > 0u) {
-          tc::tmem_ld32(taddr + ((uint32_t)(32 * lq) << 16) + (uint32_t)(half * WN + c0), v);
+          tc::tmem_ld<32>(taddr + ((uint32_t)(32 * lq) << 16) + (uint32_t)(half * WN + c0), v);
+          tc::tmem_ld_wait();
         } else {
 #pragma unroll
           for (int j = 0; j < 32; ++j) v[j] = 0.0f;
