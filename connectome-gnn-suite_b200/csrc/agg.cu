@@ -117,11 +117,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
   rt::BnQuad bq;
   if (MODE == GATHER_GCN_BWD) rt::bn_quad_init(bq, p.bn, c0, C);
   float pmean[4] = {0.f, 0.f, 0.f, 0.f}, prstd[4] = {0.f, 0.f, 0.f, 0.f};
-  if (MODE == GATHER_SAGE_BWD && p.want_prev) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-      if (c0 + j < C) { pmean[j] = p.prev_mean[c0 + j]; prstd[j] = p.prev_rstd[c0 + j]; }
-  }
+  if (MODE == GATHER_SAGE_BWD && p.want_prev) rt::bn_stats_quad(pmean, prstd, p.prev_mean, p.prev_rstd, c0, C, true);
   float s1[4] = {0.f, 0.f, 0.f, 0.f}, s2[4] = {0.f, 0.f, 0.f, 0.f};   // GCN_BWD: s1 = dbias; SAGE_BWD: sums of the layer below
 
   const int4* meta = reinterpret_cast<const int4*>(p.meta);
@@ -141,12 +137,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
       cp_async_commit();
     }
     // ---- load phase: this thread's channel quad of rows rl, rl + RP, ... transformed on the way in --------------
-    const float inv_n = 1.0f / ((float)n + 1e-8f);
     float4 pooled = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (MODE == GATHER_GCN_BWD && !p.du && live_quad) {
-      pooled = rt::ld_quad<VEC>(p.demb, g, C, c0);
-      pooled = make_float4(pooled.x * inv_n, pooled.y * inv_n, pooled.z * inv_n, pooled.w * inv_n);
-    }
+    if (MODE == GATHER_GCN_BWD && !p.du && live_quad) pooled = rt::pooled_quad<VEC>(p.demb, g, C, c0, n);
     // UL rows per thread are loaded before any is processed: one exposed memory latency per batch of UL
     constexpr int UL = MODE == GATHER_GCN_BWD ? 2 : 6;
     for (int r = rl; r < n; r += UL * RP) {
@@ -168,7 +160,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
           float4 o = a[u];
           if (MODE == GATHER_SAGE_FWD || MODE == GATHER_GCN_FWD) o = rt::act_fwd4(p.act, cq, a[u], rk, (uint32_t)(nb + rr));
           if (MODE == GATHER_GCN_BWD) {
-            o = rt::bn_bwd4(p.bn, bq, a[u], rt::act_bwd4(p.act, cq, a[u], b[MODE == GATHER_GCN_BWD ? u : 0], rk, (uint32_t)(nb + rr)));
+            o = rt::dz4<false>(p.act, cq, p.bn, bq, a[u], b[MODE == GATHER_GCN_BWD ? u : 0], rk, (uint32_t)(nb + rr));
             if (!VEC) o = rt::mask_quad(o, c0, C);
             s1[0] += o.x; s1[1] += o.y; s1[2] += o.z; s1[3] += o.w;
           }
@@ -211,13 +203,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
           const float4 dyp = rt::act_bwd4(p.act, cq, raw, acc, rk, (uint32_t)grow);
           const float rv[4] = {raw.x, raw.y, raw.z, raw.w}, dv[4] = {dyp.x, dyp.y, dyp.z, dyp.w};
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (c0 + j < C) {
-              const float xh = (rv[j] - pmean[j]) * prstd[j];
-              s1[j] += dv[j];
-              s2[j] = fmaf(dv[j], xh, s2[j]);
-            }
-          }
+          for (int j = 0; j < 4; ++j)
+            if (c0 + j < C) bn_sums_add(s1[j], s2[j], dv[j], rv[j], pmean[j], prstd[j]);
         }
       }
       rt::st_quad<VEC>(p.out, grow, C, c0, acc);
@@ -235,11 +222,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_gather(GatherArgs p) {
     const int nrec = MODE == GATHER_GCN_BWD ? 1 : 2;
     for (int idx = tid; idx < nrec * C; idx += kThreads) {
       const int which = idx / C, c = idx - which * C;
-      float s = 0.0f;
-      if (c / (4 * LPR) == slab) {
-        const int q = (c % (4 * LPR)) >> 2, j = c & 3;
-        for (int t = q; t < kThreads; t += LPR) s += red[8 * t + 4 * which + j];
-      }
+      const float s = c / (4 * LPR) == slab ? quad_sum(red, 8, 4 * which, kThreads, LPR, (c % (4 * LPR)) >> 2, c & 3) : 0.0f;
       p.partials[(size_t)blockIdx.x * p.part_stride + idx] = s;
     }
   }

@@ -137,6 +137,15 @@ __device__ __forceinline__ float bn_bwd_dz(const BnCoef& k, float t, float dy) {
   const float xh = (t - k.mean) * k.rstd;
   return k.bsc * (dy - k.s1n - xh * k.s2n);
 }
+// one element's share of the BatchNorm-backward sums of the layer below: s1 += dy, s2 += dy * xhat
+__device__ __forceinline__ void bn_sums_add(float& s1, float& s2, float dy, float t, float mean, float rstd) {
+  const float xh = (t - mean) * rstd;
+  s1 += dy;
+  s2 = fmaf(dy, xh, s2);
+}
+
+// d loss / d row of a mean-pooled subject of n rows = d loss / d embedding * pool_bwd_scale(n)
+__device__ __forceinline__ float pool_bwd_scale(int n) { return 1.0f / ((float)n + 1e-8f); }
 
 // Dropout streams of CUDA-graph replays: the host-side seed is baked into a captured launch, so a graphed training step
 // keeps two salt words on the device (refreshed by cgnn_step_tick inside the graph) and every kernel folds them into
@@ -317,6 +326,36 @@ struct Welford {
   }
 };
 
+// Welford state of one thread's channel quad; deposit() leaves the record {count, mean[4], M2[4]} at rec[0..8]
+struct QuadWelford {
+  int cnt;
+  Welford w[4];
+  __device__ __forceinline__ void init() {
+    cnt = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) w[j].init();
+  }
+  __device__ __forceinline__ void push(float4 v) {
+    cnt += 1;
+    const float inv = fast_rcp((float)cnt);
+    w[0].push(v.x, inv); w[1].push(v.y, inv); w[2].push(v.z, inv); w[3].push(v.w, inv);
+  }
+  __device__ __forceinline__ void deposit(float* rec) const {
+    rec[0] = (float)cnt;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { rec[1 + j] = w[j].mean; rec[5 + j] = w[j].m2; }
+  }
+};
+
+// Chan's merge of the Welford record {nb, mb, qb} into {n, mean, m2}; empty records are skipped
+__device__ __forceinline__ void welford_merge(double& n, double& mean, double& m2, double nb, double mb, double qb) {
+  if (nb <= 0.0) return;
+  const double nt = n + nb, delta = mb - mean;
+  mean += delta * (nb / nt);
+  m2 += qb + delta * delta * (n * nb / nt);
+  n = nt;
+}
+
 // Shared by the layer kernels: merge per-warp Welford records held in shared memory into the
 // CTA's record and write it (as doubles) to `out` = {count, mean[C], M2[C]} of this CTA.
 //   s_cnt[kWarps], s_mean[kWarps][ldc], s_m2[kWarps][ldc]
@@ -324,15 +363,23 @@ __device__ __forceinline__ void cta_write_stats(const float* s_cnt, const float*
                                                 int ldc, int C, double* out) {
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     double n = 0.0, mean = 0.0, m2 = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
-      double nb = (double)s_cnt[w];
-      if (nb <= 0.0) continue;
-      double mb = (double)s_mean[w * ldc + c], qb = (double)s_m2[w * ldc + c];
-      double nt = n + nb, delta = mb - mean;
-      mean += delta * (nb / nt);
-      m2 += qb + delta * delta * (n * nb / nt);
-      n = nt;
-    }
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w)
+      welford_merge(n, mean, m2, (double)s_cnt[w], (double)s_mean[w * ldc + c], (double)s_m2[w * ldc + c]);
+    out[1 + c] = mean;
+    out[1 + C + c] = m2;
+    if (c == 0) out[0] = n;
+  }
+}
+
+// The same record from per-thread quad records (QuadWelford::deposit): thread th < nt owns channel quad th % Q of each
+// pass of 4 Q channels and left pass P's record at rec[9 (P nt + th)].  Channel c is merged over th = q, q + Q, ...
+// in that order; thread t of the nt threads writes channels t, t + nt, ...
+__device__ __forceinline__ void cta_write_quad_stats(const float* rec, int nt, int Q, int C, int t, double* out) {
+  for (int c = t; c < C; c += nt) {
+    const float* r = rec + (size_t)(c / (4 * Q)) * nt * 9;
+    const int q = (c >> 2) % Q, j = c & 3;
+    double n = 0.0, mean = 0.0, m2 = 0.0;
+    for (int th = q; th < nt; th += Q) welford_merge(n, mean, m2, (double)r[th * 9], (double)r[th * 9 + 1 + j], (double)r[th * 9 + 5 + j]);
     out[1 + c] = mean;
     out[1 + C + c] = m2;
     if (c == 0) out[0] = n;

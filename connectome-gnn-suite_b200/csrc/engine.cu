@@ -381,23 +381,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_fwd_ws(const __grid_constant__ t
         }
       }
       tc::named_sync(1, kGathThreads);
-      double* out = p.partials + (size_t)blockIdx.x * (1 + 2 * kC);
-      for (int c = gt; c < kC; c += kGathThreads) {
-        const int qd = c >> 2, j = c & 3;
-        double n = 0.0, mean = 0.0, m2 = 0.0;
-        for (int th = qd; th < kGathThreads; th += 16) {     // the threads whose channel quad is qd
-          const double nb_ = (double)rec[th * 9];
-          if (nb_ <= 0.0) continue;
-          const double mb = (double)rec[th * 9 + 1 + j], qb = (double)rec[th * 9 + 5 + j];
-          const double nt = n + nb_, delta = mb - mean;
-          mean += delta * (nb_ / nt);
-          m2 += qb + delta * delta * (n * nb_ / nt);
-          n = nt;
-        }
-        out[1 + c] = mean;
-        out[1 + kC + c] = m2;
-        if (c == 0) out[0] = n;
-      }
+      cta_write_quad_stats(rec, kGathThreads, 16, kC, gt, p.partials + (size_t)blockIdx.x * (1 + 2 * kC));
     }
   }
 

@@ -112,11 +112,9 @@ __global__ void __launch_bounds__(NT, 2) k_first_fwd(FirstArgs p) {
   float b4[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) b4[j] = p.bias ? p.bias[4 * q + j] : 0.0f;
-  int cnt = 0;
   const bool want_stats = p.stats_partials != nullptr;
-  Welford wf[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) wf[j].init();
+  QuadWelford wf;
+  wf.init();
 
   const int4* meta = reinterpret_cast<const int4*>(p.meta);
   int4 m_next = make_int4(0, 0, 0, 0);
@@ -148,39 +146,16 @@ __global__ void __launch_bounds__(NT, 2) k_first_fwd(FirstArgs p) {
         for (int j = 0; j < 4; ++j) o[j] = fmaxf(o[j], 0.0f);
       }
       *reinterpret_cast<float4*>(p.z + (nb + r) * H + 4 * q) = make_float4(o[0], o[1], o[2], o[3]);
-      if (want_stats) {        // BatchNorm batch statistics: training only
-        cnt += 1;
-        const float inv = fast_rcp((float)cnt);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) wf[j].push(o[j], inv);
-      }
+      if (want_stats) wf.push(make_float4(o[0], o[1], o[2], o[3]));   // BatchNorm batch statistics: training only
     }
     __syncthreads();   // tiles and blob are rewritten by the next subject
   }
 
   if (p.stats_partials) {
     float* rec = reinterpret_cast<float*>(cgnn_smem);   // [NT][9]
-    rec[tid * 9] = (float)cnt;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { rec[tid * 9 + 1 + j] = wf[j].mean; rec[tid * 9 + 5 + j] = wf[j].m2; }
+    wf.deposit(rec + tid * 9);
     __syncthreads();
-    double* out = p.stats_partials + (size_t)blockIdx.x * (1 + 2 * H);
-    for (int c = tid; c < H; c += NT) {
-      const int qq = c >> 2, j = c & 3;
-      double n = 0.0, mean = 0.0, m2 = 0.0;
-      for (int th = qq; th < NT; th += QH) {
-        const double nb_ = (double)rec[th * 9];
-        if (nb_ <= 0.0) continue;
-        const double mb = (double)rec[th * 9 + 1 + j], qb = (double)rec[th * 9 + 5 + j];
-        const double nt = n + nb_, delta = mb - mean;
-        mean += delta * (nb_ / nt);
-        m2 += qb + delta * delta * (n * nb_ / nt);
-        n = nt;
-      }
-      out[1 + c] = mean;
-      out[1 + H + c] = m2;
-      if (c == 0) out[0] = n;
-    }
+    cta_write_quad_stats(rec, NT, QH, H, tid, p.stats_partials + (size_t)blockIdx.x * (1 + 2 * H));
   }
 }
 
@@ -216,11 +191,7 @@ __global__ void __launch_bounds__(NT, 2) k_first_bwd(FirstArgs p) {
     stage_subject<SAGE, true, NT>(p, m, g, s_x, s_a, s_blob);
     const long long nb = m.x;
     float4 pooled = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (!p.du) {
-      const float inv_n = 1.0f / ((float)m.y + 1e-8f);
-      pooled = rt::ld_quad<true>(p.demb, g, H, 4 * q);
-      pooled = make_float4(pooled.x * inv_n, pooled.y * inv_n, pooled.z * inv_n, pooled.w * inv_n);
-    }
+    if (!p.du) pooled = rt::pooled_quad<true>(p.demb, g, H, 4 * q, m.y);
     constexpr int UB = 4;     // rows in flight per thread
     for (int r = rsub; r < m.y; r += UB * RS) {
       float4 zv[UB], uv[UB];
@@ -236,13 +207,7 @@ __global__ void __launch_bounds__(NT, 2) k_first_bwd(FirstArgs p) {
       for (int u = 0; u < UB; ++u) {
         const int rr = r + u * RS;
         if (rr >= m.y) continue;
-        float4 dz = rt::bn_bwd4(p.bn, bq, zv[u], rt::act_bwd4(p.act_out, cq, zv[u], uv[u], rk, (uint32_t)(nb + rr)));
-        if (SAGE) {
-          if (!(zv[u].x > 0.0f)) dz.x = 0.0f;
-          if (!(zv[u].y > 0.0f)) dz.y = 0.0f;
-          if (!(zv[u].z > 0.0f)) dz.z = 0.0f;
-          if (!(zv[u].w > 0.0f)) dz.w = 0.0f;
-        }
+        const float4 dz = rt::dz4<SAGE>(p.act_out, cq, p.bn, bq, zv[u], uv[u], rk, (uint32_t)(nb + rr));
         const float d4[4] = {dz.x, dz.y, dz.z, dz.w};
 #pragma unroll
         for (int j = 0; j < 4; ++j) db[j] += d4[j];

@@ -263,7 +263,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
     const long long nb = cur.x;
     const int n = cur.y, eb = cur.z, m = cur.w;
     const bool csr_here = p.csr_smem && m <= p.max_edges;
-    const float inv_n = 1.0f / ((float)n + 1e-8f);
+    const float inv_n = pool_bwd_scale(n);
     if (csr_here) stage_csr_async(s_csr, p.max_nodes, p.max_edges, p.out_rowptr, p.out_col, p.out_wn, p.dinv, nb, n, eb, m);
     cp_async_commit();
 
@@ -406,9 +406,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
                 if (p.want_prev) {
                   const float t0 = raw[r * K + ch];
                   const float dyp = act_bwd(p.act_in, aff_in, t0, s_ci[CI_SCALE * K4 + ch], s_ci[CI_SHIFT * K4 + ch], rh, ch, acc[i][q]);
-                  const float xh = (t0 - s_ci[CI_MEAN * K4 + ch]) * s_ci[CI_RSTD * K4 + ch];
-                  ps1[q] += dyp;
-                  ps2[q] = fmaf(dyp, xh, ps2[q]);
+                  bn_sums_add(ps1[q], ps2[q], dyp, t0, s_ci[CI_MEAN * K4 + ch], s_ci[CI_RSTD * K4 + ch]);
                 }
               }
             }
@@ -442,11 +440,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
     if (ch < H4) s_red[warp * H4 + ch] = acc_db[j];
   }
   __syncthreads();
-  for (int c = tid; c < H4; c += kThreads) {
-    float s = 0.0f;
-    for (int w = 0; w < kWarps; ++w) s += s_red[w * H4 + c];
-    part[p.o_pdb + c] = s;
-  }
+  for (int c = tid; c < H4; c += kThreads) part[p.o_pdb + c] = warp_rows_sum(s_red, H4, c);
   __syncthreads();
   if (p.want_prev) {
 #pragma unroll
@@ -454,10 +448,7 @@ __global__ void __launch_bounds__(kThreads) k_gcn_bwd(GcnBwdArgs p) {
     __syncthreads();
     for (int c = tid; c < 2 * K4; c += kThreads) {
       const int which = c / K4, ch = c - which * K4;
-      const int tx = ch >> 2, q = ch & 3;
-      float s = 0.0f;
-      for (int mth = tx; mth < ntu; mth += tk) s += s_red[mth * 8 + which * 4 + q];
-      part[p.o_pprev + c] = s;
+      part[p.o_pprev + c] = quad_sum(s_red, 8, which * 4, ntu, tk, ch >> 2, ch & 3);
     }
   }
 }

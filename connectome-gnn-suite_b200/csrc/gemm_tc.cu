@@ -154,11 +154,9 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
     }
   };
 
-  int cnt = 0;
   const bool want_stats = p.partials != nullptr;
-  Welford wf[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) wf[j].init();
+  QuadWelford wf;
+  wf.init();
 
   // accumulators of the tile starting at row r0 (TMEM buffer b) -> bias + ReLU -> z, BatchNorm statistics
   auto epilogue = [&](long long r0, uint32_t b) {
@@ -175,11 +173,7 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
         v.z = fmaxf(v.z + bias4[2], 0.0f);
         v.w = fmaxf(v.w + bias4[3], 0.0f);
         *reinterpret_cast<float4*>(p.z + (r0 + r) * H + 4 * qh) = v;
-        if (want_stats) {      // BatchNorm batch statistics: training only
-          cnt += 1;
-          const float inv = fast_rcp((float)cnt);
-          wf[0].push(v.x, inv); wf[1].push(v.y, inv); wf[2].push(v.z, inv); wf[3].push(v.w, inv);
-        }
+        if (want_stats) wf.push(v);   // BatchNorm batch statistics: training only
       }
     }
   };
@@ -242,27 +236,9 @@ __global__ void __launch_bounds__(NT, 1) k_sage_fwd_gemm(SageFwdGemmArgs p) {
 
   if (p.partials) {
     float* rec = reinterpret_cast<float*>(base);   // [NT][9] over the operand tile (every MMA has completed)
-    rec[tid * 9] = (float)cnt;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { rec[tid * 9 + 1 + j] = wf[j].mean; rec[tid * 9 + 5 + j] = wf[j].m2; }
+    wf.deposit(rec + tid * 9);
     __syncthreads();
-    double* out = p.partials + (size_t)blockIdx.x * (1 + 2 * H);
-    for (int c = tid; c < H; c += NT) {
-      const int q = c >> 2, j = c & 3;
-      double n = 0.0, mean = 0.0, m2 = 0.0;
-      for (int th = q; th < NT; th += QH) {
-        const double nb = (double)rec[th * 9];
-        if (nb <= 0.0) continue;
-        const double mb = (double)rec[th * 9 + 1 + j], qb = (double)rec[th * 9 + 5 + j];
-        const double nt = n + nb, delta = mb - mean;
-        mean += delta * (nb / nt);
-        m2 += qb + delta * delta * (n * nb / nt);
-        n = nt;
-      }
-      out[1 + c] = mean;
-      out[1 + H + c] = m2;
-      if (c == 0) out[0] = n;
-    }
+    cta_write_quad_stats(rec, NT, QH, H, tid, p.partials + (size_t)blockIdx.x * (1 + 2 * H));
   }
   tc::fence_before_sync();
   __syncthreads();
@@ -395,12 +371,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
   rt::chan_quad_init(cq, p.act_in, c2, Kin);
   const rt::RowKey rk = rt::row_key(p.act_in);
   float pmean[4], prstd[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const bool ok = p.want_prev && c2 + j < Kin;
-    pmean[j] = ok ? p.prev_mean[c2 + j] : 0.0f;
-    prstd[j] = ok ? p.prev_rstd[c2 + j] : 0.0f;
-  }
+  rt::bn_stats_quad(pmean, prstd, p.prev_mean, p.prev_rstd, c2, Kin, p.want_prev);
   tc::fence_proxy_async();
   tc::fence_before_sync();
   __syncthreads();
@@ -538,10 +509,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_gcn_bwd_gemm(GcnBwdGemmArgs p) 
     __syncthreads();
     for (int c = tid; c < 2 * Kin; c += kThreads) {
       const int which = c / Kin, ch = c - which * Kin;
-      const int q = ch >> 2, j = ch & 3;
-      float s = 0.0f;
-      for (int th = q; th < kThreads; th += Q2) s += red[th * 8 + which * 4 + j];
-      part[p.o_pprev + c] = s;
+      part[p.o_pprev + c] = quad_sum(red, 8, which * 4, kThreads, Q2, ch >> 2, ch & 3);
     }
   }
   tc::fence_before_sync();
@@ -708,12 +676,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
       if (t < ntiles && row < p.rows) {
         zv = rt::ld_quad<true>(p.z, row, H, 4 * qh);
         if (p.du) uv = rt::ld_quad<true>(p.du, row, H, 4 * qh);
-        else {
-          const int g = rg[i];
-          const float inv_n = 1.0f / ((float)meta[g].y + 1e-8f);
-          const float4 e = rt::ld_quad<true>(p.demb, g, H, 4 * qh);
-          uv = make_float4(e.x * inv_n, e.y * inv_n, e.z * inv_n, e.w * inv_n);
-        }
+        else uv = rt::pooled_quad<true>(p.demb, rg[i], H, 4 * qh, meta[rg[i]].y);
       }
       zq[i] = zv; uq[i] = uv;
     }
@@ -772,12 +735,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
       const long long row = r0 + rh + i * MHq::RS;
       float4 dz = make_float4(0.f, 0.f, 0.f, 0.f);
       if (row < p.rows) {
-        const float4 dy = rt::act_bwd4(p.act_out, cq_out, zq[i], uq[i], rk_out, (uint32_t)row);
-        dz = rt::bn_bwd4(p.bn, bq, zq[i], dy);
-        if (!(zq[i].x > 0.0f)) dz.x = 0.0f;
-        if (!(zq[i].y > 0.0f)) dz.y = 0.0f;
-        if (!(zq[i].z > 0.0f)) dz.z = 0.0f;
-        if (!(zq[i].w > 0.0f)) dz.w = 0.0f;
+        dz = rt::dz4<true>(p.act_out, cq_out, p.bn, bq, zq[i], uq[i], rk_out, (uint32_t)row);
         colsum[0] += dz.x; colsum[1] += dz.y; colsum[2] += dz.z; colsum[3] += dz.w;
       }
       float4 h, l;
@@ -860,12 +818,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_sage_bwd_gemm(SageBwdGemmArgs p
     __syncthreads();
     *reinterpret_cast<float4*>(red + 4 * tid) = make_float4(colsum[0], colsum[1], colsum[2], colsum[3]);
     __syncthreads();
-    for (int c = tid; c < H; c += kThreads) {
-      const int q = c >> 2, j = c & 3;
-      float s = 0.0f;
-      for (int th = q; th < kThreads; th += QH) s += red[4 * th + j];
-      part[p.o_pdb + c] = s;
-    }
+    for (int c = tid; c < H; c += kThreads) part[p.o_pdb + c] = quad_sum(red, 4, 0, kThreads, QH, c >> 2, c & 3);
   }
   tc::fence_before_sync();
   __syncthreads();

@@ -53,11 +53,7 @@ __global__ void __launch_bounds__(kThreads) k_pool_fwd(PoolArgs p) {
     }
     __syncthreads();
     const float denom = (float)n + 1e-8f;
-    for (int c = tid; c < C; c += kThreads) {
-      float s = 0.0f;
-      for (int w = 0; w < kWarps; ++w) s += s_red[w * C4 + c];
-      p.emb[g * C + c] = s / denom;
-    }
+    for (int c = tid; c < C; c += kThreads) p.emb[g * C + c] = warp_rows_sum(s_red, C4, c) / denom;
     __syncthreads();
   }
 }
@@ -96,12 +92,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_pool_fwd_quad(PoolArgs p) {
     }
     s_red[tid] = acc;
     __syncthreads();
-    if (tid < C) {
-      const int qq = tid >> 2, j = tid & 3;
-      float s = 0.0f;
-      for (int t = qq; t < kThreads; t += Q) s += reinterpret_cast<const float*>(&s_red[t])[j];
-      p.emb[g * C + tid] = s / ((float)n + 1e-8f);
-    }
+    if (tid < C) p.emb[g * C + tid] = quad_sum(reinterpret_cast<const float*>(s_red), 4, 0, kThreads, Q, tid >> 2, tid & 3) / ((float)n + 1e-8f);
     __syncthreads();
   }
 }

@@ -76,7 +76,7 @@ __global__ void __launch_bounds__(kThreads) k_bn_bwd_sums(BnSumsArgs p) {
   for (long long g = blockIdx.x; g < p.B; g += gridDim.x) {
     const long long nb = p.ptr[g];
     const int n = (int)(p.ptr[g + 1] - nb);
-    const float inv_n = 1.0f / ((float)n + 1e-8f);
+    const float inv_n = pool_bwd_scale(n);
     for (int i = warp; i < n; i += kWarps) {
       const long long grow = nb + i;
       const uint32_t rh = p.act.drop ? drop_row_hash(p.act, p.act.row_base + grow) : 0u;
@@ -87,9 +87,7 @@ __global__ void __launch_bounds__(kThreads) k_bn_bwd_sums(BnSumsArgs p) {
           const float t = p.z[grow * C + ch];
           const float up = p.du ? p.du[grow * C + ch] : p.demb[g * C + ch] * inv_n;
           const float dy = act_bwd(p.act, affine, t, s_c[ch], s_c[C4 + ch], rh, ch, up);
-          const float xh = (t - s_c[2 * C4 + ch]) * s_c[3 * C4 + ch];
-          s1[j] += dy;
-          s2[j] = fmaf(dy, xh, s2[j]);
+          bn_sums_add(s1[j], s2[j], dy, t, s_c[2 * C4 + ch], s_c[3 * C4 + ch]);
         }
       }
     }
@@ -101,11 +99,7 @@ __global__ void __launch_bounds__(kThreads) k_bn_bwd_sums(BnSumsArgs p) {
   }
   __syncthreads();
   float* part = p.partials + (size_t)blockIdx.x * 2 * C4;
-  for (int c = tid; c < 2 * C4; c += kThreads) {
-    float s = 0.0f;
-    for (int w = 0; w < kWarps; ++w) s += s_red[w * 2 * C4 + c];
-    part[c] = s;
-  }
+  for (int c = tid; c < 2 * C4; c += kThreads) part[c] = warp_rows_sum(s_red, 2 * C4, c);
 }
 
 #ifndef CGNN_EMU
@@ -121,8 +115,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_bn_bwd_sums_quad(BnSumsArgs p) 
   rt::chan_quad_init(cq, p.act, 4 * q, C);
   const rt::RowKey rk = rt::row_key(p.act);
   float mean[4], rstd[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) { mean[j] = p.mean[4 * q + j]; rstd[j] = p.rstd[4 * q + j]; }
+  rt::bn_stats_quad(mean, rstd, p.mean, p.rstd, 4 * q, 4 * Q, true);
   float s1[4] = {0.f, 0.f, 0.f, 0.f}, s2[4] = {0.f, 0.f, 0.f, 0.f};
   long long nb_next = 0, ne_next = 0;
   if ((long long)blockIdx.x < p.B) { nb_next = p.ptr[blockIdx.x]; ne_next = p.ptr[blockIdx.x + 1]; }
@@ -131,11 +124,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_bn_bwd_sums_quad(BnSumsArgs p) 
     const int n = (int)(ne_next - nb);
     if (g + gridDim.x < p.B) { nb_next = p.ptr[g + gridDim.x]; ne_next = p.ptr[g + gridDim.x + 1]; }
     float4 pooled = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (!p.du) {
-      const float inv_n = 1.0f / ((float)n + 1e-8f);
-      pooled = rt::ld_quad<true>(p.demb, g, C, 4 * q);
-      pooled = make_float4(pooled.x * inv_n, pooled.y * inv_n, pooled.z * inv_n, pooled.w * inv_n);
-    }
+    if (!p.du) pooled = rt::pooled_quad<true>(p.demb, g, C, 4 * q, n);
     for (int i = r; i < n; i += 4 * RS) {
       float4 zv[4], uv[4];
 #pragma unroll
@@ -152,11 +141,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_bn_bwd_sums_quad(BnSumsArgs p) 
           const float4 dy = rt::act_bwd4(p.act, cq, zv[u], uv[u], rk, (uint32_t)(nb + i + u * RS));
           const float tv[4] = {zv[u].x, zv[u].y, zv[u].z, zv[u].w}, dv[4] = {dy.x, dy.y, dy.z, dy.w};
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float xh = (tv[j] - mean[j]) * rstd[j];
-            s1[j] += dv[j];
-            s2[j] = fmaf(dv[j], xh, s2[j]);
-          }
+          for (int j = 0; j < 4; ++j) bn_sums_add(s1[j], s2[j], dv[j], tv[j], mean[j], rstd[j]);
         }
     }
   }
@@ -166,10 +151,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_bn_bwd_sums_quad(BnSumsArgs p) 
   float* part = p.partials + (size_t)blockIdx.x * 2 * p.C4;
   for (int idx = tid; idx < 2 * C; idx += kThreads) {
     const int which = idx / C, c = idx - which * C;
-    const int qq = c >> 2, j = c & 3;
-    float s = 0.0f;
-    for (int t = qq; t < kThreads; t += Q) s += reinterpret_cast<const float*>(&s_red[which * kThreads + t])[j];
-    part[which * p.C4 + c] = s;
+    part[which * p.C4 + c] = quad_sum(reinterpret_cast<const float*>(s_red), 4, 4 * kThreads * which, kThreads, Q, c >> 2, c & 3);
   }
 }
 #endif

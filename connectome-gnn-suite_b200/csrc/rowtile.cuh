@@ -121,6 +121,29 @@ __device__ __forceinline__ float4 bn_bwd4(const BnBwdDev& bn, const BnQuad& b, f
   for (int j = 0; j < 4; ++j) d[j] = bn.train ? bn_bwd_dz(b.k[j], tv[j], d[j]) : b.k[j].bsc * d[j];
   return make_float4(d[0], d[1], d[2], d[3]);
 }
+// dz of the quad of the layer output z from the upstream gradient up: dropout / ReLU backward of the output activation,
+// then BatchNorm backward; RELU_MASK: then the layer's own ReLU (GraphSAGE, z = relu(.))
+template <bool RELU_MASK>
+__device__ __forceinline__ float4 dz4(const Act& act_out, const ChanQuad& cq, const BnBwdDev& bn, const BnQuad& bq, float4 z, float4 up,
+                                      const RowKey& rk, uint32_t row) {
+  float4 dz = bn_bwd4(bn, bq, z, act_bwd4(act_out, cq, z, up, rk, row));
+  if (RELU_MASK) {
+    if (!(z.x > 0.0f)) dz.x = 0.0f;
+    if (!(z.y > 0.0f)) dz.y = 0.0f;
+    if (!(z.z > 0.0f)) dz.z = 0.0f;
+    if (!(z.w > 0.0f)) dz.w = 0.0f;
+  }
+  return dz;
+}
+// mean / rstd of the BatchNorm of the layer below for the quad c0.. (zero unless `want` and c < C), for bn_sums_add
+__device__ __forceinline__ void bn_stats_quad(float (&mean)[4], float (&rstd)[4], const float* m, const float* r, int c0, int C, bool want) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const bool ok = want && c0 + j < C;
+    mean[j] = ok ? m[c0 + j] : 0.0f;
+    rstd[j] = ok ? r[c0 + j] : 0.0f;
+  }
+}
 
 // 4 channels c0.. of row `row` of a dense [rows, C] tensor; VEC: one 16-byte load, else bounded scalar loads
 template <bool VEC>
@@ -142,6 +165,13 @@ __device__ __forceinline__ void st_quad(float* __restrict__ base, long long row,
   if (c0 + 1 < C) d[1] = v.y;
   if (c0 + 2 < C) d[2] = v.z;
   if (c0 + 3 < C) d[3] = v.w;
+}
+// the upstream gradient of every row of subject g (n rows) under a mean pool: the quad c0.. of demb[g] / (n + 1e-8)
+template <bool VEC>
+__device__ __forceinline__ float4 pooled_quad(const float* __restrict__ demb, long long g, int C, int c0, int n) {
+  const float inv_n = pool_bwd_scale(n);
+  const float4 e = ld_quad<VEC>(demb, g, C, c0);
+  return make_float4(e.x * inv_n, e.y * inv_n, e.z * inv_n, e.w * inv_n);
 }
 __device__ __forceinline__ float4 mask_quad(float4 v, int c0, int C) {   // zero the channels >= C
   if (c0 + 0 >= C) v.x = 0.0f;

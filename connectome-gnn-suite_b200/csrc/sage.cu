@@ -241,7 +241,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
     const long long nb = cur.x;
     const int n = cur.y, eb = cur.z, m = cur.w;
     const bool csr_here = p.csr_smem && m <= p.max_edges;
-    const float inv_n = 1.0f / ((float)n + 1e-8f);
+    const float inv_n = pool_bwd_scale(n);
     if (K == K4) cp_async_words(s_u, p.t_in + nb * K, n * K);
     if (csr_here) stage_csr_async(s_csr, p.max_nodes, p.max_edges, p.in_rowptr, p.in_col, p.in_w, p.wsum, nb, n, eb, m);
     cp_async_commit();
@@ -381,11 +381,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_a(SageBwdArgs p) {
     if (ch < H4) s_red[warp * H4 + ch] = acc_db[j];
   }
   __syncthreads();
-  for (int c = tid; c < H4; c += kThreads) {
-    float s = 0.0f;
-    for (int w = 0; w < kWarps; ++w) s += s_red[w * H4 + c];
-    part[p.o_pdb + c] = s;
-  }
+  for (int c = tid; c < H4; c += kThreads) part[p.o_pdb + c] = warp_rows_sum(s_red, H4, c);
 }
 
 struct SageBwdBArgs {
@@ -463,9 +459,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_b(SageBwdBArgs p) {
           p.du_in[grow * K + ch] = acc[j];
           if (p.want_prev) {
             const float dyp = act_bwd(p.act_in, aff_in, t0[j], s_ci[ch], s_ci[K4 + ch], rh, ch, acc[j]);
-            const float xh = (t0[j] - s_ci[2 * K4 + ch]) * s_ci[3 * K4 + ch];
-            ps1[j] += dyp;
-            ps2[j] = fmaf(dyp, xh, ps2[j]);
+            bn_sums_add(ps1[j], ps2[j], dyp, t0[j], s_ci[2 * K4 + ch], s_ci[3 * K4 + ch]);
           }
         }
       }
@@ -481,11 +475,7 @@ __global__ void __launch_bounds__(kThreads) k_sage_bwd_b(SageBwdBArgs p) {
     }
     __syncthreads();
     float* part = p.partials + (size_t)blockIdx.x * 2 * K4;
-    for (int c = tid; c < 2 * K4; c += kThreads) {
-      float s = 0.0f;
-      for (int w = 0; w < kWarps; ++w) s += s_red[w * 2 * K4 + c];
-      part[c] = s;
-    }
+    for (int c = tid; c < 2 * K4; c += kThreads) part[c] = warp_rows_sum(s_red, 2 * K4, c);
   }
 }
 

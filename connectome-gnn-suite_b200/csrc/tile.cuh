@@ -1,5 +1,5 @@
 // tile.cuh - building blocks shared by the GCN / GraphSAGE layer kernels: per-channel constant staging, the output
-// gradient of the backward kernels, Welford statistics epilogue, CSR rows in shared memory.
+// gradient of the backward kernels, per-CTA reductions, Welford statistics epilogue, CSR rows in shared memory.
 #pragma once
 #include "common.cuh"
 
@@ -37,6 +37,21 @@ __device__ __forceinline__ float staged_dz(const Act& act_out, const BnBwdDev& b
   if (!bn.has) return dy;
   if (!bn.train) return s[DZ_BSC * H4 + c] * dy;
   return bn_bwd_dz(BnCoef{s[DZ_MEAN * H4 + c], s[DZ_RSTD * H4 + c], s[DZ_BSC * H4 + c], s[DZ_S1N * H4 + c], s[DZ_S2N * H4 + c]}, t, dy);
+}
+
+// The per-CTA reductions of per-thread partial sums, each in one fixed order.
+// Element j of channel quad q summed over the threads th = q, q + Q, q + 2Q, ... < nt that own that quad:
+// rec[th * stride + off + j].
+__device__ __forceinline__ float quad_sum(const float* rec, int stride, int off, int nt, int Q, int q, int j) {
+  float s = 0.0f;
+  for (int th = q; th < nt; th += Q) s += rec[th * stride + off + j];
+  return s;
+}
+// Column c of a lane-per-channel record summed over the warps 0, 1, ..., kWarps - 1: s_red[w * ld + c].
+__device__ __forceinline__ float warp_rows_sum(const float* s_red, int ld, int c) {
+  float s = 0.0f;
+  for (int w = 0; w < kWarps; ++w) s += s_red[w * ld + c];
+  return s;
 }
 
 // Per-warp running Welford state for HC channels per lane (channel = lane + 32*j).

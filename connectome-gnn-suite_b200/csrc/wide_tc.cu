@@ -107,14 +107,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) bias4[J][j] = p.bias ? p.bias[J * W_SLAB + 4 * qs + j] : 0.0f;
   const bool want_stats = p.partials != nullptr;
-  Welford wf[W_PASSES][4];
-  int cnt[W_PASSES];
+  QuadWelford wf[W_PASSES];
 #pragma unroll
-  for (int J = 0; J < W_PASSES; ++J) {
-    cnt[J] = 0;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) wf[J][j].init();
-  }
+  for (int J = 0; J < W_PASSES; ++J) wf[J].init();
 
   float4 pa[2];
   auto load_a = [&](long long tt, int kk) {
@@ -158,11 +153,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
         x.x += bias4[J][0]; x.y += bias4[J][1]; x.z += bias4[J][2]; x.w += bias4[J][3];
         if (p.relu) { x.x = fmaxf(x.x, 0.0f); x.y = fmaxf(x.y, 0.0f); x.z = fmaxf(x.z, 0.0f); x.w = fmaxf(x.w, 0.0f); }
         *reinterpret_cast<float4*>(p.out + (pend_r0 + r) * WN + J * W_SLAB + 4 * qs) = x;
-        if (want_stats) {
-          cnt[J] += 1;
-          const float inv = fast_rcp((float)cnt[J]);
-          wf[J][0].push(x.x, inv); wf[J][1].push(x.y, inv); wf[J][2].push(x.z, inv); wf[J][3].push(x.w, inv);
-        }
+        if (want_stats) wf[J].push(x);
       }
     }
   };
@@ -226,31 +217,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xw(WideXwArgs p) {
   if (p.partials) {
     float* rec = reinterpret_cast<float*>(base);   // [W_PASSES][kThreads][9] over stage 0 (every MMA has completed)
 #pragma unroll
-    for (int J = 0; J < W_PASSES; ++J) {
-      float* r = rec + ((size_t)J * kThreads + tid) * 9;
-      r[0] = (float)cnt[J];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) { r[1 + j] = wf[J][j].mean; r[5 + j] = wf[J][j].m2; }
-    }
+    for (int J = 0; J < W_PASSES; ++J) wf[J].deposit(rec + ((size_t)J * kThreads + tid) * 9);
     __syncthreads();
-    double* out = p.partials + (size_t)blockIdx.x * (1 + 2 * WN);
-    for (int c = tid; c < WN; c += kThreads) {
-      const int J = c / W_SLAB, q = (c % W_SLAB) >> 2, j = c & 3;
-      double n = 0.0, mean = 0.0, m2 = 0.0;
-      for (int th = q; th < kThreads; th += W_SLAB / 4) {
-        const float* r = rec + ((size_t)J * kThreads + th) * 9;
-        const double nb = (double)r[0];
-        if (nb <= 0.0) continue;
-        const double mb = (double)r[1 + j], qb = (double)r[5 + j];
-        const double nt = n + nb, delta = mb - mean;
-        mean += delta * (nb / nt);
-        m2 += qb + delta * delta * (n * nb / nt);
-        n = nt;
-      }
-      out[1 + c] = mean;
-      out[1 + WN + c] = m2;
-      if (c == 0) out[0] = n;
-    }
+    cta_write_quad_stats(rec, kThreads, W_SLAB / 4, WN, tid, p.partials + (size_t)blockIdx.x * (1 + 2 * WN));
   }
   tc::fence_before_sync();
   __syncthreads();
@@ -298,11 +267,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
 
   const bool want_prev = p.prev_partials != nullptr;
   float pmean[4], prstd[4], ps1[4] = {0.f, 0.f, 0.f, 0.f}, ps2[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    pmean[j] = want_prev ? p.prev_mean[4 * q + j] : 0.0f;
-    prstd[j] = want_prev ? p.prev_rstd[4 * q + j] : 0.0f;
-  }
+  rt::bn_stats_quad(pmean, prstd, p.prev_mean, p.prev_rstd, 4 * q, WN, want_prev);
 
   const long long nchunks = (p.rows + XR - 1) / XR;
   float4 dp[2], tu[2], dd[2];
@@ -337,10 +302,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
           const float4 dy = rt::act_bwd4(p.act_in, cq, tu[i], dd[i], rk, (uint32_t)row);
           const float tv[4] = {tu[i].x, tu[i].y, tu[i].z, tu[i].w}, dv[4] = {dy.x, dy.y, dy.z, dy.w};
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            ps1[j] += dv[j];
-            ps2[j] = fmaf(dv[j], (tv[j] - pmean[j]) * prstd[j], ps2[j]);
-          }
+          for (int j = 0; j < 4; ++j) bn_sums_add(ps1[j], ps2[j], dv[j], tv[j], pmean[j], prstd[j]);
         }
       }
       tc::split4(u, h, l);
@@ -397,10 +359,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wide_xty(WideXtyArgs p) {
     __syncthreads();
     for (int c2 = tid; c2 < 2 * WN; c2 += kThreads) {
       const int which = c2 / WN, ch = c2 - which * WN;
-      const int qq = ch >> 2, j = ch & 3;
-      float sacc = 0.0f;
-      for (int th = qq; th < kThreads; th += WN / 4) sacc += red[th * 8 + which * 4 + j];
-      p.prev_partials[(size_t)blockIdx.x * 2 * WN + c2] = sacc;
+      p.prev_partials[(size_t)blockIdx.x * 2 * WN + c2] = quad_sum(red, 8, which * 4, kThreads, WN / 4, ch >> 2, ch & 3);
     }
   }
   tc::fence_before_sync();
@@ -437,9 +396,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_wide_dz(WideDzArgs p) {
         if (p.du) uv[i] = rt::ld_quad<true>(p.du, row, WN, 4 * q);
         else {
           const int g = p.row_graph[row];
-          const float inv_n = 1.0f / ((float)meta[g].y + 1e-8f);
-          const float4 e = rt::ld_quad<true>(p.demb, g, WN, 4 * q);
-          uv[i] = make_float4(e.x * inv_n, e.y * inv_n, e.z * inv_n, e.w * inv_n);
+          uv[i] = rt::pooled_quad<true>(p.demb, g, WN, 4 * q, meta[g].y);
         }
       }
     }
@@ -447,24 +404,14 @@ __global__ void __launch_bounds__(kThreads, 2) k_wide_dz(WideDzArgs p) {
     for (int i = 0; i < 2; ++i) {
       const long long row = row0 + 8 * i;
       if (row >= p.rows) continue;
-      const float4 dy = rt::act_bwd4(p.act_out, cq, zv[i], uv[i], rk, (uint32_t)row);
-      float4 dz = rt::bn_bwd4(p.bn, bq, zv[i], dy);
-      if (!(zv[i].x > 0.0f)) dz.x = 0.0f;
-      if (!(zv[i].y > 0.0f)) dz.y = 0.0f;
-      if (!(zv[i].z > 0.0f)) dz.z = 0.0f;
-      if (!(zv[i].w > 0.0f)) dz.w = 0.0f;
+      const float4 dz = rt::dz4<true>(p.act_out, cq, p.bn, bq, zv[i], uv[i], rk, (uint32_t)row);
       cs[0] += dz.x; cs[1] += dz.y; cs[2] += dz.z; cs[3] += dz.w;
       rt::st_quad<true>(p.dz, row, WN, 4 * q, dz);
     }
   }
   s_red[tid] = make_float4(cs[0], cs[1], cs[2], cs[3]);
   __syncthreads();
-  if (tid < WN) {
-    const int qq = tid >> 2, j = tid & 3;
-    float s = 0.0f;
-    for (int t = qq; t < kThreads; t += WN / 4) s += reinterpret_cast<const float*>(&s_red[t])[j];
-    p.partials[(size_t)blockIdx.x * WN + tid] = s;
-  }
+  if (tid < WN) p.partials[(size_t)blockIdx.x * WN + tid] = quad_sum(reinterpret_cast<const float*>(s_red), 4, 0, kThreads, WN / 4, tid >> 2, tid & 3);
 }
 
 bool al16(const void* p) { return (((uintptr_t)p) & 15u) == 0; }
