@@ -6,6 +6,14 @@ fused eval) also run under -m "not gpu"; on a B200 every case runs, and each one
 kernels it was written for are the ones that ran - a change to the dispatch cannot silently move coverage.
 test_dispatch_table prints the table of case -> kernels.
 
+Every undirected batch has A^ = A^T, equal in- and out-degrees and the same neighbours in the by-destination and the
+by-source aggregation blobs: a kernel that aggregates in the wrong direction passes on it.  The "-directed" cases repeat
+the kernel paths on one-way multigraphs (directed_graphs, |A^ - A^T| / |A^| > 0.3 asserted), with the aggregation blobs
+written by the collate kernel, by k_build_agg after a device collate or a host-assembled COO batch, or by both (a
+subject over the collate kernel's staging cap).  The "-salt" cases run the layer kernels' dropout with device salt words
+at row offsets 2^32 - 100 and 3 * 2^32 - 50, rows crossing the 2^32 boundary inside one CTA.  test_dispatch_table also
+asserts that the directed cases reach DIRECTED_REQUIRED and the salted cases SALTED_REQUIRED.
+
 Element bar: |got - ref| <= C_ULPS * 2^-23 * mag, mag = the same computation on absolute values (contract_ref.py).
 Model-level cases on ingested (real-density) connectomes compare with the oracle (oracle/port.py) by the rule
 dp_parity uses: per tensor <= max(1e-5, 4 x the fp32 oracle's own distance from the fp64 evaluation), measured in
@@ -16,6 +24,20 @@ Value mutations of the kernel sources that these cases catch on the simulator (a
   k_gcn_fwd without the self-loop term when the CSR is read from L2   gcn-fwd-ingest360-first
   GraphSAGE w_sum + 1e-8 -> w_sum + 0 (isolated nodes)           sage-fwd-generic-n385 (tensor-core edition on a B200)
   BatchNorm backward s2 / count -> s1 / count (k_gcn_bwd)        gcn-bwd-generic-H20
+  k_gcn_bwd launched on the by-destination CSR (in_rowptr / in_col / in_wn for the out_* arrays, gcn.cu)
+                                                                 gcn-bwd-gemm-n385-directed (gcn-bwd-generic-H20-directed on a B200)
+  k_build_agg fills each blob from the other direction's lists (rp, col and weights: dir == 0 -> dir == 1, agg.cu)
+                                                                 gcn-fwd-engine-n129-directed (on a B200 too)
+  k_gcn_fwd_ws hashes row grow instead of row_base + grow        gcn-fwd-engine-n384-salt
+  k_gcn_fwd without act_salt(p.act)                              gcn-fwd-generic-H20-salt
+  k_gcn_bwd's prev-sums mask hashes row grow instead of row_base + grow   gcn-bwd-generic-H20-salt
+  (the last three together: those three cases and gcn-fwd-engine-n129-wrap3-p0.9)
+Mutations of device-only kernels, one B200 run each (first case to fail):
+  every k_gather<GCN_BWD> launch reads agg_in (gcn.cu, wide_tc.cu), decoded as a by-destination blob (agg.cu kPre)
+                                                                 gcn-bwd-gemm-middle-directed
+  k_sage_fwd_gemm's narrow-K operand path hashes row instead of row_base + row (gemm_tc.cu)
+                                                                 sage-fwd-gemm-d9-hidden-salt
+  k_sage_bwd_gemm without act_salt(p.act_out); act_salt(p.act_in)  sage-bwd-gemm-middle-salt
 
 Real-density dispatch (360-region ingested subjects, q = 0.90, ~26k directed edges per subject; the table of
 test_dispatch_table on a B200): GCN runs every layer, forward and backward, on k_gcn_fwd / k_gcn_bwd with the CSR read
@@ -55,6 +77,56 @@ def rand_graphs(sizes, F, seed, isolated=True, deg=8):
     return out
 
 
+def directed_graphs(sizes, F, seed, heavy=1, deg=8):
+    """One-way multigraphs with independent edge weights, skewed so that the direction matters: sources are drawn from
+    the lower two thirds of a subject's ids (mostly the lowest), destinations from the upper two thirds (mostly the
+    highest).  The first third are out-degree hubs that no edge enters, the last third in-degree hubs that no edge
+    leaves.  Every subject also gets self-loops and repeated (src, dst) pairs of other weights; the last node of a
+    subject of > 2 nodes has no edge.  Subject 0 has `heavy` times the edges of the others."""
+    from connectome_gnn.graph import ConnectomeGraph
+    rng = np.random.default_rng(seed)
+    out = []
+    for s, n in enumerate(sizes):
+        hi = n - 1 if n > 2 else n
+        m = deg * n * (heavy if s == 0 else 1)
+        span = max(1, (2 * hi) // 3)
+        src = (span * rng.random(m) ** 2).astype(np.int64)
+        dst = hi - 1 - (span * rng.random(m) ** 2).astype(np.int64)
+        k = max(1, m // 16)
+        loops, rep = rng.integers(0, hi, k), rng.integers(0, m, k)
+        ei = np.stack([np.concatenate([src, loops, src[rep]]), np.concatenate([dst, loops, dst[rep]])])
+        w = rng.random(ei.shape[1]).astype(np.float32) + 0.05
+        x = rng.normal(size=(n, F)).astype(np.float32)
+        out.append(ConnectomeGraph(torch.from_numpy(x), torch.from_numpy(ei), torch.from_numpy(w),
+                                   torch.tensor(int(rng.integers(0, 2)))))
+    asym = asymmetry(out)
+    assert asym > 0.3, f"the directed batch is nearly symmetric: |A^ - A^T| / |A^| = {asym:.2f}"
+    return out
+
+
+def asymmetry(graphs):
+    """|A^ - A^T|_F / |A^|_F of the batch's GCN operator A^ = D^-1/2 (A + I) D^-1/2 (A[dst, src], D^ over sources)."""
+    num = den = 0.0
+    for gr in graphs:
+        n = gr.num_nodes
+        src, dst = gr.edge_index.numpy()
+        a = np.eye(n)
+        np.add.at(a, (dst, src), gr.edge_weight.numpy().astype(np.float64))
+        dinv = 1.0 / np.sqrt(a.sum(0))
+        a = dinv[:, None] * a * dinv[None, :]
+        num += float(((a - a.T) ** 2).sum())
+        den += float((a ** 2).sum())
+    return np.sqrt(num / den)
+
+
+def host_coo(graphs):
+    """(edge_index, edge_weight, ptr) of a list of subjects, concatenated on the host: what the reference is built from."""
+    sizes = np.array([gr.num_nodes for gr in graphs], dtype=np.int64)
+    ptr = np.concatenate([[0], np.cumsum(sizes)])
+    ei = torch.cat([gr.edge_index + int(ptr[s]) for s, gr in enumerate(graphs)], 1)
+    return ei, torch.cat([gr.edge_weight for gr in graphs]), torch.from_numpy(ptr)
+
+
 def ingested(S, N, kind="dense", q=0.90, seed=5):
     """The README's real-data recipe on the device: packed arena of S subjects (1 feature per node)."""
     import ingest_ref
@@ -74,11 +146,36 @@ def packed_graphs(p):
     return out
 
 
-def batch_of(spec):
-    """(batch, contract_ref.Graph) of a graph spec: ("rand", sizes, F, seed) or ("ingest", S, N, kind, q)."""
-    from connectome_gnn.graph import SubjectStore, collate_graphs
+def batch_of(spec, kind=None):
+    """(batch, contract_ref.Graph) of a graph spec: ("rand", sizes, F, seed), ("ingest", S, N, kind, q) or
+    ("directed", sizes, F, seed, blobs).  `blobs` is where the batch's aggregation blobs of model family `kind` come from:
+      "lazy"      collate_graphs; k_build_agg at the first layer call
+      "emit"      a lean SubjectStore.collate(prepare_for=kind): k_collate_graph writes them
+      "full"      the same with lean=False (every subject small enough to be staged)
+      "coo"       a ConnectomeBatch assembled from host tensors: cgnn_csr_from_coo, then k_build_agg
+      "overflow"  subject 0 has 4x the edges, beyond the collate kernel's staging cap: a lean=False collate emits the
+                  blobs of the others and k_build_agg those of subject 0 alone
+    The reference of a directed batch is built from the host lists, not from what the collate kernel wrote."""
+    from connectome_gnn.graph import ConnectomeBatch, SubjectStore, collate_graphs, pack_graphs
     if spec[0] == "rand":
         b = collate_graphs(rand_graphs(spec[1], spec[2], spec[3]))
+    elif spec[0] == "directed":
+        _, sizes, F, seed, blobs = spec
+        gs = directed_graphs(sizes, F, seed, heavy=4 if blobs == "overflow" else 1)
+        ei, w, ptr = host_coo(gs)
+        dev = _DEV["device"]
+        if blobs == "lazy":
+            b = collate_graphs(gs)
+        elif blobs == "coo":
+            x = torch.cat([gr.node_features for gr in gs])
+            batch = torch.repeat_interleave(torch.arange(len(gs)), ptr[1:] - ptr[:-1])
+            labels = torch.stack([gr.label for gr in gs])
+            b = ConnectomeBatch(x.to(dev), ei.to(dev), w.to(dev), batch.to(dev), labels.to(dev), ptr.to(dev))
+            b.ensure_csr()
+        else:
+            assert kind is not None and blobs in ("emit", "full", "overflow"), blobs
+            b = SubjectStore(pack_graphs(gs), dev).collate(np.arange(len(gs)), prepare_for=kind, lean=blobs == "emit")
+        return b, cr.Graph(ei, w, ptr)
     else:
         p = ingested(*spec[1:])
         b = SubjectStore(p, _DEV["device"]).collate(np.arange(spec[1]))
@@ -115,13 +212,15 @@ def worst(rs):
 
 
 # ---- runners: each returns the worst error ratio of the case ----------------------------------------------------------
-def run_layer_fwd(eng, kind, d_in, H, graph, hidden=True, p_drop=0.3, seed=0):
+def run_layer_fwd(eng, kind, d_in, H, graph, hidden=True, p_drop=0.3, row_base=0, salt=None, seed=0):
+    """One forward call.  hidden: the input is a stored activation loaded through BatchNorm affine, (GCN) ReLU and
+    dropout, whose local row 0 is global row `row_base`, salted with the device words `salt`; else the node features."""
     dev = _DEV["device"]
-    b, g = batch_of(graph)
+    b, g = batch_of(graph, kind)
     gen = torch.Generator().manual_seed(seed)
     rows = b.num_nodes
     if hidden:
-        t, a = hidden_input(rows, d_in, gen, kind == "gcn", p_drop)
+        t, a = hidden_input(rows, d_in, gen, kind == "gcn", p_drop, row_base=row_base, salt=salt)
         t = t.to(dev)
     else:                                  # a first layer reads the node features as they are
         assert b.node_features.shape[1] == d_in
@@ -143,21 +242,23 @@ def run_layer_fwd(eng, kind, d_in, H, graph, hidden=True, p_drop=0.3, seed=0):
     return worst(rs)
 
 
-def run_layer_bwd(eng, kind, d_in, H, graph, first=False, pooled=False, bn="train", sums64=True, p_out=0.3, p_in=0.3,
-                  seed=0):
-    """One backward call.  first: the input needs no gradient (no du_in, no prev sums), the node features as input;
-    pooled: the top layer (upstream = demb [B, H]); bn: "train" / "eval" / None; sums64: the double sums are handed in
-    (and the fp32 sums are a decoy the kernel must not read)."""
+def run_layer_bwd(eng, kind, d_in, H, graph, first=False, hidden=None, pooled=False, bn="train", sums64=True, p_out=0.3,
+                  p_in=0.3, row_base=0, salt=None, seed=0):
+    """One backward call.  first: the input needs no gradient (no du_in, no prev sums); hidden (default: not first): the
+    input is a stored activation with its own BatchNorm affine, ReLU and dropout, else the node features; pooled: the top
+    layer (upstream = demb [B, H]); bn: "train" / "eval" / None; sums64: the double sums are handed in (and the fp32
+    sums are a decoy the kernel must not read).  Both dropouts (input and output) start at global row `row_base` and are
+    salted with the device words `salt`."""
     from connectome_gnn._engine import BnBwd
     dev = _DEV["device"]
-    b, g = batch_of(graph)
+    b, g = batch_of(graph, kind)
     gen = torch.Generator().manual_seed(seed)
     rows, B = b.num_nodes, b.num_graphs
-    if first:
+    if not (not first if hidden is None else hidden):
         t, a_in = b.node_features.contiguous(), None
         assert t.shape[1] == d_in
     else:
-        t, a_in = hidden_input(rows, d_in, gen, kind == "gcn", p_in, site=1)
+        t, a_in = hidden_input(rows, d_in, gen, kind == "gcn", p_in, site=1, row_base=row_base, salt=salt)
         t = t.to(dev)
     act_in_d, act_in_r = acts(a_in, dev)
     W = (torch.randn(H, d_in * (2 if kind == "sage" else 1), generator=gen) / np.sqrt(d_in)).to(dev)
@@ -165,7 +266,7 @@ def run_layer_bwd(eng, kind, d_in, H, graph, first=False, pooled=False, bn="trai
     if kind == "sage":   # the aggregate the forward stored (and with it the tensor-core path of the backward)
         _, _, agg = eng.layer_fwd(kind, t, act_in_d, W, torch.zeros(H, device=dev), b.csr, b.ptr, B, False)
     # this layer's output and its BatchNorm + (GCN) ReLU + dropout
-    zt, a_out = hidden_input(rows, H, gen, kind == "gcn", p_out, site=2)
+    zt, a_out = hidden_input(rows, H, gen, kind == "gcn", p_out, site=2, row_base=row_base, salt=salt)
     if kind == "sage":
         zt = torch.clamp(torch.randn(rows, H, generator=gen), min=0.0)   # a ReLU output, exact zeros included
     z = zt.to(dev)
@@ -311,10 +412,11 @@ def _eval_params(L, F, K, gen, M=32, H=64):
     return layers, head
 
 
-def run_eval_fused(eng, L, F, K, sizes=(84, 30, 130, 57, 1, 200), seed=0):
-    """cgnn_eval_fused_fwd against the eval-mode network in float64; K > 8 must decline (None: the caller falls back)."""
+def run_eval_fused(eng, L, F, K, sizes=(84, 30, 130, 57, 1, 200), blobs=None, seed=0):
+    """cgnn_eval_fused_fwd against the eval-mode network in float64; K > 8 must decline (None: the caller falls back).
+    blobs: a directed batch whose aggregation blobs come from there (batch_of), else an undirected one."""
     dev = _DEV["device"]
-    b, g = batch_of(("rand", sizes, F, 40 + L))
+    b, g = batch_of(("rand", sizes, F, 40 + L) if blobs is None else ("directed", sizes, F, 40 + L, blobs), "gcn")
     gen = torch.Generator().manual_seed(seed)
     layers, head = _eval_params(L, F, K, gen)
     to = lambda q: q.to(dev) if isinstance(q, torch.Tensor) else q
@@ -328,11 +430,12 @@ def run_eval_fused(eng, L, F, K, sizes=(84, 30, 130, 57, 1, 200), seed=0):
     return worst([cr.check(out[0], emb, embm, "fused emb"), cr.check(out[1], logits, lm, "fused logits")])
 
 
-def run_fwd_pool(eng, sizes, seed=0):
-    """cgnn_gcn_layer_fwd_pool (eval, hidden 64): emb = mean_rows relu(bn(z)); a subject of > 384 rows -> None."""
+def run_fwd_pool(eng, sizes, blobs=None, seed=0):
+    """cgnn_gcn_layer_fwd_pool (eval, hidden 64): emb = mean_rows relu(bn(z)); a subject of > 384 rows -> None.
+    blobs: as run_eval_fused."""
     from connectome_gnn._engine import Act
     dev = _DEV["device"]
-    b, g = batch_of(("rand", sizes, 3, 60))
+    b, g = batch_of(("rand", sizes, 3, 60) if blobs is None else ("directed", sizes, 3, 60, blobs), "gcn")
     gen = torch.Generator().manual_seed(seed)
     rows = b.num_nodes
     t, a = hidden_input(rows, 64, gen, True, 0.0)
@@ -356,10 +459,25 @@ def run_fwd_pool(eng, sizes, seed=0):
 R84 = ("rand", (84, 84, 84, 84), 64, 1)
 SMALL16 = ("rand", (20,) * 16, 64, 2)
 CASES, EMU_CASES = [], []
+DIRECTED, SALTED = set(), set()     # ids of the cases on directed batches / with salted dropout keys
+BLOBS_BUILT = ("lazy", "coo", "overflow")     # batch_of modes in which k_build_agg writes (some) aggregation blobs
 
 
-def case(cid, fn, kw, emu, expect=(), forbid=()):
-    CASES.append(pytest.param(fn, kw, set(expect), set(forbid), id=cid))
+def case(cid, fn, kw, emu, expect=(), forbid=(), salted=False):
+    """A directed case also names its collate kernel (k_collate_graph, never the pair kernel) and requires or forbids
+    k_build_agg by where its blobs come from; `salted` marks a case whose dropout keys take device salt words (a `salt`
+    argument marks it too)."""
+    expect, forbid = set(expect), set(forbid)
+    graph = kw.get("graph", ("",))
+    blobs = graph[4] if graph[0] == "directed" else kw.get("blobs")
+    if blobs is not None:
+        DIRECTED.add(cid)
+        expect.add("k_collate_graph")
+        forbid.add("k_collate_pairs")
+        (expect if blobs in BLOBS_BUILT else forbid).add("k_build_agg")
+    if salted or kw.get("salt") is not None:
+        SALTED.add(cid)
+    CASES.append(pytest.param(fn, kw, expect, forbid, id=cid))
     if emu:
         EMU_CASES.append(pytest.param(fn, kw, id=cid))
 
@@ -469,7 +587,7 @@ for K in (2, 3, 8, 9, 64):
         for B, p in ((1, 0.0), (4097, 0.3)):
             small = M <= 64 and K <= 8
             case(f"head-K{K}-M{M}-B{B}-p{p}", run_head, dict(B=B, C=64, M=M, K=K, p_drop=p), B == 1 or (K, M) == (9, 32),
-                 ["k_head_fwd_small" if small else "k_head_fwd", "k_head_bwd", "k_ce_fwd", "k_ce_bwd"])
+                 ["k_head_fwd_small" if small else "k_head_fwd", "k_head_bwd", "k_ce_fwd", "k_ce_bwd"], salted=p > 0)
 case("bn-bookkeeping", run_bn_bookkeeping, {}, True, [])
 # -- eval-mode network in one kernel, and the pooled last layer
 for L in (2, 3, 4):
@@ -481,12 +599,118 @@ for sizes in ((1,), (2, 1), (9, 8, 127), (128, 129, 1), (383, 384)):
     case(f"fwd-pool-n{max(sizes)}", run_fwd_pool, dict(sizes=sizes), max(sizes) in (9, 129), ["k_gcn_fwd_ws<true>"])
 case("fwd-pool-n385-declines", run_fwd_pool, dict(sizes=(385, 3)), True, [])
 
+# -- directed twins: one-way edges, A^ != A^T, in-degree != out-degree, agg_in != agg_out.  Every mode of batch_of
+#    appears on several kernel paths; the simulator runs the twins of the cases it runs above
+MODES = ("emit", "lazy", "coo", "overflow")
+D = lambda sizes, F, seed, blobs: ("directed", sizes, F, seed, blobs)
+for n, blobs in ((9, "emit"), (129, "lazy"), (384, "coo")):
+    case(f"gcn-fwd-engine-n{n}-directed", run_layer_fwd, dict(kind="gcn", d_in=64, H=64, graph=D((n, max(1, n // 3), n), 64, n, blobs)),
+         True, ["k_gcn_fwd_ws<false>"])
+case("gcn-fwd-engine-16-per-unit-directed", run_layer_fwd, dict(kind="gcn", d_in=64, H=64, graph=D((20,) * 16, 64, 2, "emit")),
+     True, ["k_gcn_fwd_ws<false>"])
+for i, (kind, d_in, H) in enumerate((k, d, h) for k in ("gcn", "sage") for d in (1, 5, 8) for h in (32, 256)):
+    case(f"{kind}-fwd-first-d{d_in}-H{H}-directed", run_layer_fwd,
+         dict(kind=kind, d_in=d_in, H=H, graph=D((84, 30, 1), d_in, 5, MODES[i % 4]), hidden=False), False, ["k_first_fwd"])
+case("sage-fwd-gemm-d64-directed", run_layer_fwd, dict(kind="sage", d_in=64, H=64, graph=D((84,) * 4, 64, 1, "full")), False,
+     ["k_gather<0>", "k_sage_fwd_gemm"])
+case("sage-fwd-gemm-n384-directed", run_layer_fwd, dict(kind="sage", d_in=64, H=64, graph=D((384, 3), 64, 9, "lazy")), False,
+     ["k_gather<0>", "k_sage_fwd_gemm"])
+case("sage-fwd-generic-n385-directed", run_layer_fwd, dict(kind="sage", d_in=64, H=64, graph=D((385, 20), 64, 4, "coo")), True,
+     ["k_gather<0>", "k_sage_fwd_gemm"])
+for kind, blobs in (("gcn", "emit"), ("sage", "overflow")):
+    case(f"{kind}-fwd-wide256-directed", run_layer_fwd, dict(kind=kind, d_in=256, H=256, graph=D((84, 30, 1), 256, 7, blobs)),
+         False, ["k_gather<3>", "k_wide_xw"] if kind == "gcn" else ["k_wide_xw"])
+for kind, blobs in (("gcn", "coo"), ("sage", "emit")):
+    case(f"{kind}-fwd-generic-H20-directed", run_layer_fwd, dict(kind=kind, d_in=64, H=20, graph=D((84, 30, 1), 64, 8, blobs)),
+         True, ["k_gcn_fwd" if kind == "gcn" else "k_sage_fwd"])
+for kind in ("gcn", "sage"):
+    gemm = "k_gcn_bwd_gemm" if kind == "gcn" else "k_sage_bwd_gemm"
+    generic = ["k_gcn_bwd"] if kind == "gcn" else ["k_sage_bwd_a", "k_sage_bwd_b"]
+    gather_bwd = "k_gather<1>" if kind == "gcn" else "k_gather<2>"
+    wide = ["k_gather<1>", "k_wide_xty", "k_wide_xw"] if kind == "gcn" else ["k_gather<2>", "k_wide_dz", "k_wide_xty"]
+    case(f"{kind}-bwd-gemm-middle-directed", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=D((84,) * 4, 64, 1, "emit")),
+         False, [gemm, gather_bwd])
+    case(f"{kind}-bwd-gemm-top-directed", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=D((84,) * 4, 64, 1, "overflow"),
+                                                              pooled=True), False, [gemm])
+    case(f"{kind}-bwd-gemm-n385-directed", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=D((385, 20), 64, 4, "lazy")), True,
+         [gemm, gather_bwd])
+    case(f"{kind}-bwd-first-d1-directed", run_layer_bwd, dict(kind=kind, d_in=1, H=64, graph=D((84, 30, 1), 1, 12, "coo"),
+                                                              first=True), False, ["k_first_bwd"])
+    case(f"{kind}-bwd-first-d5-H256-top-directed", run_layer_bwd,
+         dict(kind=kind, d_in=5, H=256, graph=D((84, 30, 1), 5, 12, "emit"), first=True, pooled=True), False, ["k_first_bwd"])
+    case(f"{kind}-bwd-wide256-directed", run_layer_bwd, dict(kind=kind, d_in=256, H=256, graph=D((84, 30, 1), 256, 13, "lazy")),
+         False, wide)
+    case(f"{kind}-bwd-wide256-top-directed", run_layer_bwd, dict(kind=kind, d_in=256, H=256, graph=D((84, 30, 1), 256, 13, "coo"),
+                                                                 pooled=True, bn="eval"), False, wide)
+    case(f"{kind}-bwd-generic-H20-directed", run_layer_bwd, dict(kind=kind, d_in=64, H=20, graph=D((84, 30, 1), 64, 14, "emit")),
+         True, generic)
+    case(f"{kind}-bwd-generic-d96-directed", run_layer_bwd, dict(kind=kind, d_in=96, H=64, graph=D((84, 30, 1), 96, 14, "overflow"),
+                                                                 pooled=True), True, generic)
+for sizes, blobs in (((128, 129, 1), "emit"), ((9, 8, 127), "overflow"), ((383, 384), "lazy")):
+    case(f"fwd-pool-n{max(sizes)}-directed", run_fwd_pool, dict(sizes=sizes, blobs=blobs), max(sizes) in (9, 129),
+         ["k_gcn_fwd_ws<true>"])
+for i, (L, F, K) in enumerate((l, f, k) for l in (2, 4) for f in (1, 8) for k in (2, 8)):
+    case(f"eval-fused-L{L}-F{F}-K{K}-directed", run_eval_fused, dict(L=L, F=F, K=K, blobs=MODES[i % 4]), False, ["k_gcn_eval_fused"])
+case("eval-fused-L3-F5-K8-directed", run_eval_fused, dict(L=3, F=5, K=8, blobs="emit"), True, ["k_gcn_eval_fused"])
+
+# -- salted dropout keys in the layer kernels, at row offsets whose rows cross a 2^32 boundary of the global row id inside
+#    one CTA's range (every batch has > 100 rows); the second offset has the high word 2, neither 0 nor 1
+WRAP3 = 3 * 2 ** 32 - 50
+SALT = [0x9E3779B9, 0x7F4A7C15]
+SALT3 = [0xA5A5F00D, 0x0000C0DE]
+S = lambda rb, salt, p=0.3: dict(row_base=rb, salt=salt, p_drop=p)
+SB = lambda rb, salt: dict(row_base=rb, salt=salt)
+case("gcn-fwd-engine-n384-salt", run_layer_fwd, dict(kind="gcn", d_in=64, H=64, graph=("rand", (384, 128, 384), 64, 384),
+                                                     **S(ROW_BASE_WRAP, SALT)), True, ["k_gcn_fwd_ws<false>"])
+case("gcn-fwd-engine-n129-wrap3-p0.9", run_layer_fwd, dict(kind="gcn", d_in=64, H=64, graph=("rand", (129, 43, 129), 64, 129),
+                                                           **S(WRAP3, SALT3, 0.9)), True, ["k_gcn_fwd_ws<false>"])
+for kind in ("gcn", "sage"):
+    case(f"{kind}-fwd-generic-H20-salt", run_layer_fwd, dict(kind=kind, d_in=64, H=20, graph=("rand", (84, 30, 1), 64, 8),
+                                                             **S(ROW_BASE_WRAP, SALT)), True, ["k_gcn_fwd" if kind == "gcn" else "k_sage_fwd"])
+    case(f"{kind}-fwd-first-d5-H64-hidden-salt", run_layer_fwd, dict(kind=kind, d_in=5, H=64, graph=("rand", (84, 30, 1), 5, 5),
+                                                                     **S(WRAP3, SALT3)), False, ["k_first_fwd"])
+    case(f"{kind}-fwd-wide256-salt", run_layer_fwd, dict(kind=kind, d_in=256, H=256, graph=("rand", (84, 30, 1), 256, 7),
+                                                         **S(ROW_BASE_WRAP, SALT)), False,
+         ["k_gather<3>", "k_wide_xw"] if kind == "gcn" else ["k_wide_xw"])
+    gemm = "k_gcn_bwd_gemm" if kind == "gcn" else "k_sage_bwd_gemm"
+    generic = ["k_gcn_bwd"] if kind == "gcn" else ["k_sage_bwd_a", "k_sage_bwd_b"]
+    gather_bwd = "k_gather<1>" if kind == "gcn" else "k_gather<2>"
+    wide = ["k_gather<1>", "k_wide_xty", "k_wide_xw"] if kind == "gcn" else ["k_gather<2>", "k_wide_dz", "k_wide_xty"]
+    case(f"{kind}-bwd-gemm-middle-salt", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=R84, **SB(ROW_BASE_WRAP, SALT)), False,
+         [gemm, gather_bwd])
+    case(f"{kind}-bwd-gemm-n385-wrap3-salt", run_layer_bwd, dict(kind=kind, d_in=64, H=64, graph=("rand", (385, 20), 64, 4),
+                                                                 **SB(WRAP3, SALT3)), False, [gemm, gather_bwd])
+    case(f"{kind}-bwd-generic-H20-salt", run_layer_bwd, dict(kind=kind, d_in=64, H=20, graph=("rand", (84, 30, 1), 64, 14),
+                                                             **SB(ROW_BASE_WRAP, SALT)), True, generic)
+    case(f"{kind}-bwd-first-d5-H64-hidden-salt", run_layer_bwd, dict(kind=kind, d_in=5, H=64, graph=("rand", (84, 30, 1), 5, 12),
+                                                                     first=True, hidden=True, **SB(WRAP3, SALT3)), False,
+         ["k_first_bwd"])
+    case(f"{kind}-bwd-wide256-salt", run_layer_bwd, dict(kind=kind, d_in=256, H=256, graph=("rand", (84, 30, 1), 256, 13),
+                                                         **SB(ROW_BASE_WRAP, SALT)), False, wide)
+case("sage-fwd-gemm-d64-salt", run_layer_fwd, dict(kind="sage", d_in=64, H=64, graph=R84, **S(WRAP3, SALT3)), False,
+     ["k_gather<0>", "k_sage_fwd_gemm"])
+# nine input channels: k_sage_fwd_gemm applies the input's dropout itself (the narrow-K operand path)
+case("sage-fwd-gemm-d9-hidden-salt", run_layer_fwd, dict(kind="sage", d_in=9, H=64, graph=("rand", (84, 30), 9, 6),
+                                                         **S(ROW_BASE_WRAP, SALT)), False, ["k_sage_fwd_gemm"])
+case("pool-sums-C64-wrap3-salt", run_pool_and_sums, dict(C=64, graph=("rand", (360,), 64, 15), row_base=WRAP3, salt=SALT3), True,
+     ["k_pool_fwd_quad", "k_bn_bwd_sums_quad"])
+
 # every one of these must be reached by at least one case on a B200
 REQUIRED = {"k_gcn_fwd_ws<true>", "k_gcn_fwd_ws<false>", "k_first_fwd", "k_first_bwd", "k_gather<0>", "k_gather<1>",
             "k_gather<2>", "k_gather<3>", "k_sage_fwd_gemm", "k_gcn_bwd_gemm", "k_sage_bwd_gemm", "k_wide_xw", "k_wide_xty",
             "k_wide_dz", "k_gcn_fwd", "k_gcn_bwd", "k_sage_fwd", "k_sage_bwd_a", "k_sage_bwd_b", "k_gcn_eval_fused",
             "k_pool_fwd", "k_pool_fwd_quad", "k_head_fwd", "k_head_fwd_small", "k_head_bwd", "k_ce_fwd", "k_ce_bwd",
             "k_bn_bwd_sums", "k_bn_bwd_sums_quad", "k_build_agg"}
+# ... these by a directed case (every layer kernel, the blob builder and the collate kernel that emits blobs)
+DIRECTED_REQUIRED = {"k_gcn_fwd_ws<true>", "k_gcn_fwd_ws<false>", "k_first_fwd", "k_first_bwd", "k_gather<0>", "k_gather<1>",
+                     "k_gather<2>", "k_gather<3>", "k_sage_fwd_gemm", "k_gcn_bwd_gemm", "k_sage_bwd_gemm", "k_wide_xw",
+                     "k_wide_xty", "k_wide_dz", "k_gcn_fwd", "k_gcn_bwd", "k_sage_fwd", "k_sage_bwd_a", "k_sage_bwd_b",
+                     "k_gcn_eval_fused", "k_build_agg", "k_collate_graph"}
+# ... and these by a salted case: every kernel that folds the device salt into its dropout keys (act_salt)
+SALTED_REQUIRED = {"k_gather<0>", "k_gather<1>", "k_gather<2>", "k_gather<3>", "k_gcn_fwd_ws<false>", "k_first_fwd",
+                   "k_first_bwd", "k_gcn_fwd", "k_gcn_bwd", "k_sage_fwd_gemm", "k_gcn_bwd_gemm", "k_sage_bwd_gemm", "k_pool_fwd",
+                   "k_pool_fwd_quad", "k_head_fwd", "k_head_fwd_small", "k_bn_bwd_sums", "k_bn_bwd_sums_quad", "k_sage_fwd",
+                   "k_sage_bwd_a", "k_sage_bwd_b", "k_wide_xty", "k_wide_dz"}
 
 _DEV = {"device": "cpu"}
 
@@ -561,8 +785,9 @@ def test_head_rejects_more_than_64_classes_b200():
 
 @pytest.mark.gpu
 def test_dispatch_table():
-    """Prints case -> kernels (and worst error ratio) and asserts every kernel of REQUIRED was reached.  Cases that did not
-    run in this session (deselected) are run here."""
+    """Prints case -> kernels (and worst error ratio) and asserts every kernel of REQUIRED was reached, every kernel of
+    DIRECTED_REQUIRED by a directed case and every kernel of SALTED_REQUIRED by a salted one.  Cases that did not run in
+    this session (deselected) are run here."""
     for p in CASES:
         if p.id not in _SEEN:
             fn, kw, _, _ = p.values
@@ -571,14 +796,18 @@ def test_dispatch_table():
     print("\ncase | worst error (x 2^-23 x mag) | kernels")
     for cid, (names, r) in _SEEN.items():
         print(f"{cid} | {r:.2f} | {' '.join(sorted(n for n in names if n.startswith('k_')))}")
-    seen = set().union(*(n for n, _ in _SEEN.values()))
-    assert REQUIRED <= seen, f"never reached: {sorted(REQUIRED - seen)}"
+    for what, ids in (("directed", DIRECTED), ("salted", SALTED)):
+        print(f"worst error of the {what} cases: {max(_SEEN[c][1] for c in ids):.2f}")
+    reached = lambda ids: set().union(*(n for c, (n, _) in _SEEN.items() if c in ids))
+    assert REQUIRED <= reached(_SEEN), f"never reached: {sorted(REQUIRED - reached(_SEEN))}"
+    assert DIRECTED_REQUIRED <= reached(DIRECTED), f"no directed case reached: {sorted(DIRECTED_REQUIRED - reached(DIRECTED))}"
+    assert SALTED_REQUIRED <= reached(SALTED), f"no salted case reached: {sorted(SALTED_REQUIRED - reached(SALTED))}"
 
 
 # ---- model level: ingested (real-density) and synthetic subjects against the oracle -----------------------------------
 def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hidden=64, seed=0):
     """A training step (logits, loss, every gradient, running statistics) and eval logits against parity.oracle_reference.
-    source: ("ingest", S, N, kind, q) or ("synthetic", S, N).  With one all-positive feature per node the fp32 oracle
+    source: ("ingest", S, N, kind, q), ("synthetic", S, N) or ("directed", sizes, F, seed) (directed_graphs).  With one all-positive feature per node the fp32 oracle
     itself sits above 1e-5 from fp64 on some tensors (BatchNorm means of nearly constant columns): bars below 1e-5 are
     scaled by the oracle's own distance, measured here.  Logits and loss at 1e-5.  (The "ties" recipe at 84 regions keeps
     no edge at all: a batch without edges, which once failed to collate.)"""
@@ -590,6 +819,11 @@ def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hi
     if source[0] == "ingest":
         p = ingested(*source[1:])
         graphs = packed_graphs(p)
+    elif source[0] == "directed":
+        graphs = directed_graphs(*source[1:])
+        for i, gr in enumerate(graphs):
+            gr.label = torch.tensor(i % K)
+        p = pack_graphs(graphs)
     else:
         from connectome_gnn.synthetic import generate_dataset
         graphs = generate_dataset(num_subjects=source[1], num_regions=source[2], seed=source[1] + source[2])
@@ -673,6 +907,9 @@ for kind in ("gcn", "sage"):
     for K in (3, 9, 64):
         model_case(f"{kind}-synthetic-K{K}", dict(kind=kind, source=("synthetic", 12, 40), K=K), K == 9)
     model_case(f"{kind}-synthetic-1-layer", dict(kind=kind, source=("synthetic", 6, 84), layers=1), True)
+    for fe in ("auto", False):       # one-way edges through every layer of the model, lean batches
+        model_case(f"{kind}-directed-fused_{fe}", dict(kind=kind, source=("directed", (84, 60, 84, 30, 84, 9), 5, 21),
+                                                       fused_eval=fe), kind == "gcn" and fe == "auto")
 
 
 @pytest.mark.parametrize("kw", EMU_MODEL_CASES)
