@@ -8,7 +8,7 @@
 //
 //   layer 1          gather warps: a_i = sum_e w^_e x_src(e) in the F (<= 8) input channels, z = a W1^T + b1 (FMAs)
 //   layers 2..L      P = u W_l^T on the tensor core (3 x TF32, A operand in tensor memory), drained into the P tile,
-//                    then z_i = sum_e w^_e P_src(e) + b_l by the gather warps - the pipeline of engine.cu, except that
+//                    then z_i = sum_e w^_e P_src(e) + b_l by the gather warps - the roles of engine.cuh, except that
 //                    the rows reach the converters through a shared-memory ring written by the PREVIOUS layer's
 //                    epilogue (u = relu(scale z + shift)) instead of by TMA
 //   readout + head   per-warp partial sums in a fixed order (the result does not depend on how subjects are batched),
@@ -35,19 +35,15 @@ struct Args {
   const float* affine;                       // [L][2][64] scale, shift of the eval-mode BatchNorm after every layer
   int L;
   const float* W0; const float* b0; const float* Wc; const float* bc; int M, K;   // head
-  const int32_t* blob; const int32_t* meta; long long B, units;
-  int spu, blob_cap_bytes, nblob;
+  UnitPlan plan;
   float* emb; float* logits;
   int o_ring, o_p, o_blob, o_x, o_pool, o_const, o_head, o_tab;   // byte offsets from the 1024-aligned base (W buffer at 0)
-  __host__ __device__ UnitSrc src() const { return UnitSrc{meta, B, spu, blob_cap_bytes}; }
 };
 
 struct EvalBarriers {
   uint64_t w_full, w_free;
   uint64_t ring_full[2], ring_free[2];
-  uint64_t a_full[2], a_free[2];
-  uint64_t d_full[kMaxTiles], d_free[kMaxTiles];
-  uint64_t blob_full[2], blob_free[2];
+  PipeBars pipe;
 };
 
 struct PrepArgs {
@@ -62,13 +58,8 @@ struct PrepArgs {
 __global__ void __launch_bounds__(256) k_eval_prep(PrepArgs p) {
   const int b = blockIdx.x, tid = threadIdx.x;
   if (b < p.L - 1) {
-    const float* W = p.W[b + 1];
     unsigned char* hi = p.wimg + (size_t)b * kWImgBytes;
-    unsigned char* lo = hi + 2 * kC * 128;
-    for (int idx = tid; idx < kC * (kC / 4); idx += blockDim.x) {
-      const int n = idx / (kC / 4), k = (idx - n * (kC / 4)) * 4;
-      tc::store_split4(hi, lo, n, k, kC, *reinterpret_cast<const float4*>(W + n * kC + k));
-    }
+    stage_w_split(hi, hi + 2 * kC * 128, p.W[b + 1], tid, blockDim.x);
     return;
   }
   for (int idx = tid; idx < p.L * kC; idx += blockDim.x) {
@@ -105,7 +96,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
   float* s_hb = s_w1 + kC * kFeat;                              // [L - 1][64]
   float* s_aff = s_hb + (kMaxLayers - 1) * kC;                  // [L][2][64]
   float* s_head = reinterpret_cast<float*>(base + p.o_head);    // W0 [M][64], b0 [M], Wc [K][M], bc [K], then [16 warps][64 + M]
-  int* s_tab = reinterpret_cast<int*>(base + p.o_tab);          // [2][kTabInts]
+  UnitTab* s_tab = reinterpret_cast<UnitTab*>(base + p.o_tab);  // [2]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int L = p.L, NH = p.L - 1;
 
@@ -113,9 +104,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
   if (tid == 0) {
     tc::mbar_init(&bars.w_full, 1); tc::mbar_init(&bars.w_free, 1);
     for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.ring_full[i], kGathWarps); tc::mbar_init(&bars.ring_free[i], 4 * 32); }
-    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.a_full[i], 4 * 32); tc::mbar_init(&bars.a_free[i], 1); }
-    for (int i = 0; i < kMaxTiles; ++i) { tc::mbar_init(&bars.d_full[i], 1); tc::mbar_init(&bars.d_free[i], kGathWarps); }
-    for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars.blob_full[i], 1); tc::mbar_init(&bars.blob_free[i], kGathWarps); }
+    init_pipe_bars(bars.pipe);
     tc::fence_mbar_init();
   }
   for (int c = tid; c < kC; c += kNT) s_b1[c] = p.b1 ? p.b1[c] : 0.0f;
@@ -143,7 +132,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
         tc::bulk_load(w_hi, p.wimg, kWImgBytes, &bars.w_full);
       } else {
         uint32_t wq = 0;
-        for (long long u = blockIdx.x; u < p.units; u += gridDim.x)
+        for (long long u = blockIdx.x; u < p.plan.units; u += gridDim.x)
           for (int hl = 0; hl < NH; ++hl, ++wq) {
             tc::mbar_wait(&bars.w_free, (wq & 1u) ^ 1u);    // the previous layer's MMAs no longer read the buffer
             tc::mbar_arrive_expect_tx(&bars.w_full, kWImgBytes);
@@ -153,44 +142,18 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
     }
   } else if (warp == kWarpBlob) {
     // ================================ blob loader ==================================================================
-    if (lane == 0) {
-      uint32_t ucount = 0;
-      for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
-        const Unit un = unit_geom(p.src(), u);
-        const uint32_t b = ucount % (uint32_t)p.nblob, use = ucount / (uint32_t)p.nblob;
-        tc::mbar_wait(&bars.blob_free[b], (use & 1u) ^ 1u);
-        tc::mbar_arrive_expect_tx(&bars.blob_full[b], (uint32_t)un.blob_bytes);
-        tc::bulk_load(s_blob + (size_t)b * p.blob_cap_bytes, p.blob + un.blob_word0, (uint32_t)un.blob_bytes, &bars.blob_full[b]);
-      }
-    }
+    if (lane == 0) blob_producer(p.plan, bars.pipe, s_blob);
   } else if (warp == kWarpMma) {
     // ================================ MMA issuer ===================================================================
     if (lane == 0 && NH >= 1) {
       const uint32_t idesc = tc::idesc_tf32(kTR, kC);
       const uint64_t b_hi = tc::smem_desc_sw128(tc::smem_u32(w_hi)), b_lo = tc::smem_desc_sw128(tc::smem_u32(w_lo));
       uint32_t tq = 0, wq = 0, uses[kMaxTiles] = {0, 0, 0};
-      for (long long u = blockIdx.x; u < p.units; u += gridDim.x) {
-        const Unit un = unit_geom(p.src(), u);
+      for (long long u = blockIdx.x; u < p.plan.units; u += gridDim.x) {
+        const Unit un = unit_geom(p.plan, u);
         for (int hl = 0; hl < NH; ++hl) {
           if (NH > 1 || wq == 0) { tc::mbar_wait(&bars.w_full, wq & 1u); ++wq; }
-          for (int t = 0; t < un.tiles; ++t, ++tq) {
-            tc::mbar_wait(&bars.d_free[t], (uses[t] & 1u) ^ 1u);
-            ++uses[t];
-            const uint32_t d = tmem + kColD + (uint32_t)(kC * t);
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              tc::mbar_wait(&bars.a_full[h], tq & 1u);
-              tc::fence_after_sync();
-#pragma unroll
-              for (int ks = 0; ks < 4; ++ks) {
-                const uint64_t bo = (uint64_t)((h * kC * 128 + ks * 32) >> 4);
-                const uint32_t ac = (uint32_t)(32 * h + 8 * ks);
-                tc::mma_tf32x3_ts(d, tmem + kColAHi + ac, tmem + kColALo + ac, b_hi + bo, b_lo + bo, idesc, (h | ks) ? 1u : 0u);
-              }
-              tc::mma_commit(&bars.a_free[h]);
-            }
-            tc::mma_commit(&bars.d_full[t]);
-          }
+          for (int t = 0; t < un.tiles; ++t, ++tq) mma_tile(bars.pipe, tmem, t, uses[t], tq, idesc, b_hi, b_lo);
           if (NH > 1) tc::mma_commit(&bars.w_free);     // fires when this layer's last MMA has read the weights
         }
       }
@@ -202,34 +165,15 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
     const unsigned char* slot = s_ring + h * kStageBytes;
     const uint32_t lane_addr = tmem + ((uint32_t)(32 * q) << 16);
     uint32_t tq = 0;
-    for (long long u = blockIdx.x; u < p.units; u += gridDim.x) {
-      const Unit un = unit_geom(p.src(), u);
+    for (long long u = blockIdx.x; u < p.plan.units; u += gridDim.x) {
+      const Unit un = unit_geom(p.plan, u);
       for (int hl = 0; hl < NH; ++hl)
         for (int t = 0; t < un.tiles; ++t, ++tq) {
           tc::mbar_wait(&bars.ring_full[h], tq & 1u);
           float4 v[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const float4*>(slot + tc::box_chunk_offset(row, j));
+          load_box_row(slot, row, v);
           tc::mbar_arrive(&bars.ring_free[h]);
-          tc::mbar_wait(&bars.a_free[h], (tq & 1u) ^ 1u);
-          tc::fence_after_sync();
-#pragma unroll
-          for (int part = 0; part < 2; ++part) {
-            float hi[16], lo[16];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              float4 h, l;
-              tc::split4(v[4 * part + j], h, l);
-              hi[4 * j + 0] = h.x; hi[4 * j + 1] = h.y; hi[4 * j + 2] = h.z; hi[4 * j + 3] = h.w;
-              lo[4 * j + 0] = l.x; lo[4 * j + 1] = l.y; lo[4 * j + 2] = l.z; lo[4 * j + 3] = l.w;
-            }
-            const uint32_t col = (uint32_t)(32 * h + 16 * part);
-            tc::tmem_st<16>(lane_addr + kColAHi + col, hi);
-            tc::tmem_st<16>(lane_addr + kColALo + col, lo);
-          }
-          tc::tmem_st_wait();
-          tc::fence_before_sync();
-          tc::mbar_arrive(&bars.a_full[h]);
+          store_a_row(bars.pipe, lane_addr, h, tq, v);
         }
     }
   } else if (warp >= kGathWarp0) {
@@ -242,73 +186,29 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
     const float4 b1q = *reinterpret_cast<const float4*>(s_b1 + 4 * cl);
     uint32_t ucount = 0, rq = 0, uses[kMaxTiles] = {0, 0, 0};   // rq: ring tiles written so far (all warps count alike)
 
-    auto build_table = [&](long long u, int* tab) {
-      const Unit un = unit_geom(p.src(), u);
-      const int4* meta = reinterpret_cast<const int4*>(p.meta);
-      int4 m = make_int4(0, 0, 0, 0);
-      if (lane < un.nsub) m = meta[un.g0 + lane];
-      const int n = lane < un.nsub ? m.y : 0;
-      int pincl = (n + 7) & ~7;
-      for (int o = 1; o < 32; o <<= 1) {
-        const int a = __shfl_up_sync(kFull, pincl, o);
-        if (lane >= o) pincl += a;
-      }
-      if (lane < un.nsub) {
-        int* e = tab + 8 + 8 * lane;
-        e[0] = (int)(m.x - un.row0);
-        e[1] = pincl - ((n + 7) & ~7);
-        e[2] = n;
-        e[3] = (int)(agg_base_words(m.x, m.z, un.g0 + lane) - un.blob_word0);
-      }
-      if (lane == 0) {
-        tab[0] = un.rows; tab[1] = un.nsub; tab[3] = un.tiles;
-        tab[4] = (int)(un.row0 & 0xffffffffll); tab[5] = (int)(un.row0 >> 32);
-        tab[6] = (int)(un.g0 & 0xffffffffll); tab[7] = (int)(un.g0 >> 32);
-      }
-    };
-    if (gw == 0 && (long long)blockIdx.x < p.units) build_table(blockIdx.x, s_tab);
+    if (gw == 0 && (long long)blockIdx.x < p.plan.units) build_unit_tab(p.plan, blockIdx.x, s_tab, lane);
     tc::named_sync(1, kGathThreads);
 
-    for (long long u = blockIdx.x; u < p.units; u += gridDim.x, ++ucount) {
-      const int* tab = s_tab + (ucount & 1u) * kTabInts;
-      const int rows = tab[0], nsub = tab[1], tiles = tab[3];
-      const long long row0 = (long long)(uint32_t)tab[4] | ((long long)tab[5] << 32);
-      const long long g0 = (long long)(uint32_t)tab[6] | ((long long)tab[7] << 32);
+    for (long long u = blockIdx.x; u < p.plan.units; u += gridDim.x, ++ucount) {
+      const UnitTab& tab = s_tab[ucount & 1u];
+      const int rows = tab.rows, nsub = tab.nsub, tiles = tab.tiles;
+      const long long row0 = tab.row0, g0 = tab.g0;
       // ---- the unit's node features: [rows][8], zero padded --------------------------------------------------------
       for (int idx = gt; idx < rows * kFeat; idx += kGathThreads) {
         const int r = idx >> 3, k = idx & 7;
         s_x[idx] = k < p.F ? p.x[(row0 + r) * p.F + k] : 0.0f;
       }
-      const uint32_t b = ucount % (uint32_t)p.nblob;
-      tc::mbar_wait(&bars.blob_full[b], (ucount / (uint32_t)p.nblob) & 1u);
-      if (gw == 0 && u + gridDim.x < p.units) build_table(u + gridDim.x, s_tab + ((ucount + 1) & 1u) * kTabInts);
+      const uint32_t b = ucount % (uint32_t)p.plan.nblob;
+      tc::mbar_wait(&bars.pipe.blob_full[b], (ucount / (uint32_t)p.plan.nblob) & 1u);
+      if (gw == 0 && u + gridDim.x < p.plan.units) build_unit_tab(p.plan, u + gridDim.x, &s_tab[(ucount + 1) & 1u], lane);
       tc::named_sync(1, kGathThreads);
-      const int32_t* blob = reinterpret_cast<const int32_t*>(s_blob + (size_t)b * p.blob_cap_bytes);
+      const int32_t* blob = reinterpret_cast<const int32_t*>(s_blob + (size_t)b * p.plan.blob_cap_bytes);
 
       for (int l = 0; l < L; ++l) {          // l = 0: the narrow first layer; l >= 1: hidden layer over the P tile
         const bool last = l == L - 1;
         if (l >= 1) {
           // ---- drain this layer's projected tiles, tensor memory -> P ------------------------------------------------
-          for (int t = 0; t < tiles; ++t) {
-            tc::mbar_wait(&bars.d_full[t], uses[t] & 1u);
-            ++uses[t];
-            tc::fence_after_sync();
-            float v[16];
-            tc::tmem_ld<16>(tmem + ((uint32_t)(32 * q) << 16) + kColD + (uint32_t)(kC * t + 16 * cg), v);
-            tc::tmem_ld_wait();
-            const int drow = t * kTR + 32 * q + lane;
-            if (drow < rows) {
-              int j = 0;
-              while (j + 1 < nsub && drow >= tab[8 + 8 * (j + 1)]) ++j;
-              const int i = drow - tab[8 + 8 * j], prow = tab[8 + 8 * j + 1] + i;
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                *reinterpret_cast<float4*>(s_p + p_chunk_offset(prow, i, 4 * cg + k)) = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
-            }
-            tc::fence_before_sync();
-            __syncwarp();
-            if (lane == 0) tc::mbar_arrive(&bars.d_free[t]);
-          }
+          drain_tiles(bars.pipe, tab, tmem, q, cg, lane, s_p, uses);
         } else {
           // ---- first layer: P = x W1^T with plain FMAs (F <= 8 input channels), written like a drained tile ------------
           // (reference models.py:111 projects first as well; the gather below is the one every layer shares)
@@ -316,10 +216,10 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
 #pragma unroll
           for (int k = 0; k < kFeat; ++k) wq[k] = *reinterpret_cast<const float4*>(s_w1 + k * kC + 4 * cl);
           for (int j = 0; j < nsub; ++j) {
-            const int* e = tab + 8 + 8 * j;
-            const int n = e[2];
+            const SubRec& e = tab.sub[j];
+            const int n = e.rows;
             for (int i = 2 * gw + half; i < n; i += 2 * kGathWarps) {
-              const float* xr = s_x + (size_t)(e[0] + i) * kFeat;
+              const float* xr = s_x + (size_t)(e.row + i) * kFeat;
               const float4 xa = *reinterpret_cast<const float4*>(xr), xb = *reinterpret_cast<const float4*>(xr + 4);
               const float xv[kFeat] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
               float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -328,7 +228,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
                 o.x = fmaf(xv[k], wq[k].x, o.x); o.y = fmaf(xv[k], wq[k].y, o.y);
                 o.z = fmaf(xv[k], wq[k].z, o.z); o.w = fmaf(xv[k], wq[k].w, o.w);
               }
-              *reinterpret_cast<float4*>(s_p + p_chunk_offset(e[1] + i, i, cl)) = o;
+              *reinterpret_cast<float4*>(s_p + p_chunk_offset(e.prow + i, i, cl)) = o;
             }
           }
         }
@@ -350,46 +250,16 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
           }
         };
         for (int j = 0; j < nsub; ++j) {
-          const int* e = tab + 8 + 8 * j;
-          const int n = e[2];
-          const int4* desc = reinterpret_cast<const int4*>(blob + e[3]);
-          const int4* rec2 = reinterpret_cast<const int4*>(blob + e[3] + 4 * n);
+          const SubRec& e = tab.sub[j];
+          const int n = e.rows;
+          const int4* desc = reinterpret_cast<const int4*>(blob + e.blob);
           float4 pool = make_float4(0.f, 0.f, 0.f, 0.f);
           for (int lp = gw; 2 * lp < n; lp += kGathWarps) {       // subject-local pairs: the same warp for the same row in any batch
             const int i = 2 * lp + half;
             const bool valid = i < n;
             int4 d = make_int4(0, 0, 0, 0);
             if (valid) d = desc[i];
-            const int len = d.y - d.x;
-            const int lmax = max(len, __shfl_xor_sync(kFull, len, 16));
-            const int4* rp = rec2 + (d.x >> 1);
-            float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-            {
-              const int lmin = min(len, __shfl_xor_sync(kFull, len, 16));
-              const unsigned char* pbase = s_p + (size_t)e[1] * 256;
-              int k = 0;
-#pragma unroll 1
-              for (; k + 4 <= lmin; k += 4, rp += 2) {
-                const int4 r = rp[0], s = rp[1];
-                const float4 v0 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)r.x ^ lane_const));
-                const float4 v1 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)r.z ^ lane_const));
-                const float4 v2 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)s.x ^ lane_const));
-                const float4 v3 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)s.z ^ lane_const));
-                fma_quad(a, v0, __int_as_float(r.y));
-                fma_quad(a, v1, __int_as_float(r.w));
-                fma_quad(a, v2, __int_as_float(s.y));
-                fma_quad(a, v3, __int_as_float(s.w));
-              }
-#pragma unroll 1
-              for (; k < lmax; k += 2, ++rp) {
-                int4 r = make_int4(0, 0, 0, 0);
-                if (k < len) r = *rp;
-                const float4 v0 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)r.x ^ lane_const));
-                const float4 v1 = *reinterpret_cast<const float4*>(pbase + ((uint32_t)r.z ^ lane_const));
-                fma_quad(a, v0, __int_as_float(r.y));
-                fma_quad(a, v1, __int_as_float(r.w));
-              }
-            }
+            const float4 a = gather_row(d, desc + n, s_p + (size_t)e.prow * 256, lane_const);
             // z = a + b; u = relu(scale z + shift)   (GCN: conv -> BatchNorm -> ReLU, reference models.py:207-209)
             float4 uo;
             uo.x = fmaxf(fmaf(a.x + bq.x, scq.x, shq.x), 0.0f);
@@ -400,7 +270,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
               if (valid) { pool.x += uo.x; pool.y += uo.y; pool.z += uo.z; pool.w += uo.w; }
             } else {
               // the row goes to the converters through the ring, in the layout a TMA box would have
-              const int ur = e[0] + (valid ? i : (n - 1));               // row of the unit
+              const int ur = e.row + (valid ? i : (n - 1));               // row of the unit
               const int t_mine = ur >> 7;
               const int t0 = __shfl_sync(kFull, t_mine, 0), t1 = __shfl_sync(kFull, t_mine, 16);
               const int hh = cl >> 3, jc = cl & 7, rr = ur & 127;
@@ -413,11 +283,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
               }
             }
           }
-          if (last) {     // this warp's share of the subject's readout: the two rows of the pair in a fixed order
-            pool.x += __shfl_xor_sync(kFull, pool.x, 16); pool.y += __shfl_xor_sync(kFull, pool.y, 16);
-            pool.z += __shfl_xor_sync(kFull, pool.z, 16); pool.w += __shfl_xor_sync(kFull, pool.w, 16);
-            if (half == 0) *reinterpret_cast<float4*>(s_pool + ((size_t)j * kGathWarps + gw) * kC + 4 * cl) = pool;
-          }
+          if (last) pool_put(s_pool, j, gw, lane, pool);
         }
         if (!last) {
           advance_to(tiles - 1);
@@ -430,7 +296,7 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
         }
       }
       __syncwarp();
-      if (lane == 0) tc::mbar_arrive(&bars.blob_free[b]);
+      if (lane == 0) tc::mbar_arrive(&bars.pipe.blob_free[b]);
       tc::named_sync(1, kGathThreads);              // the readout partials are complete; P, x and the blob are free
 
       // ---- mean-pool readout and MLP head: one warp per subject ------------------------------------------------------
@@ -438,11 +304,9 @@ __global__ void __launch_bounds__(kNT, 1) k_gcn_eval_fused(Args p) {
         const float* w0 = s_head; const float* b0 = w0 + M * kC; const float* wc = b0 + M; const float* bc = wc + K * M;
         float* my = s_head + M * kC + M + K * M + K + (size_t)gw * (kC + M);    // [64] emb, [M] hidden
         for (int j = gw; j < nsub; j += kGathWarps) {
-          const float inv = 1.0f / ((float)tab[8 + 8 * j + 2] + 1e-8f);          // reference models.py:40-47: sum / (count + 1e-8)
+          const float inv = 1.0f / ((float)tab.sub[j].rows + 1e-8f);          // reference models.py:40-47: sum / (count + 1e-8)
           for (int c = lane; c < kC; c += 32) {
-            float s = 0.0f;
-            for (int w = 0; w < kGathWarps; ++w) s += s_pool[((size_t)j * kGathWarps + w) * kC + c];
-            const float v = s * inv;
+            const float v = pool_sum(s_pool, j, c) * inv;
             my[c] = v;
             if (p.emb) p.emb[(g0 + j) * kC + c] = v;
           }
@@ -508,18 +372,13 @@ int launch_eval_fused(int kind, const float* x, int F, const cgnn_eval_layer_t* 
   a.x = x; a.F = F; a.W1 = layers[0].W; a.b1 = layers[0].bias;
   a.wimg = pa.wimg; a.hbias = pa.hbias; a.affine = pa.affine; a.L = L;
   a.W0 = W0; a.b0 = b0; a.Wc = Wc; a.bc = bc; a.M = M; a.K = K;
-  a.blob = csr->agg_in; a.meta = csr->graph_meta; a.B = num_graphs;
+  a.plan.blob = csr->agg_in; a.plan.meta = csr->graph_meta; a.plan.B = num_graphs;
   a.emb = emb; a.logits = logits;
-  int spu = kMaxUnitRows / max_nodes;
-  if (spu > kMaxSub) spu = kMaxSub;
-  {   // small batches: fewer subjects per unit so that the units cover the SMs (the launch is latency-bound there)
-    const long long fill = (num_graphs + dev.sm_count - 1) / dev.sm_count;
-    if ((long long)spu > fill) spu = (int)(fill < 1 ? 1 : fill);
-  }
+  int spu = plan_spu(max_nodes, num_graphs, dev.sm_count);
   size_t smem = 0;
   for (; spu >= 1; --spu) {         // the largest number of subjects per unit whose tiles, records and readout partials fit
     const int p_rows = spu * ((max_nodes + 7) & ~7);
-    const size_t blob_cap = (size_t)(((long long)spu * (agg_copy_words(max_nodes, max_edges) + 8) + 3) & ~3ll) * 4;
+    const size_t blob_cap = plan_blob_cap(spu, max_nodes, max_edges);
     size_t off = kWImgBytes;
     a.o_ring = (int)off; off += 2 * kStageBytes;
     a.o_p = (int)off; off += (size_t)p_rows * 256;
@@ -530,22 +389,22 @@ int launch_eval_fused(int kind, const float* x, int F, const cgnn_eval_layer_t* 
     a.o_const = (int)off; off += (size_t)(kC + kC * kFeat + (kMaxLayers - 1) * kC + kMaxLayers * 2 * kC) * 4;
     a.o_head = (int)off; off += (size_t)(M * kC + M + K * M + K + kGathWarps * (kC + M)) * 4;
     off = (off + 15) & ~(size_t)15;
-    a.o_tab = (int)off; off += (size_t)2 * kTabInts * 4;
+    a.o_tab = (int)off; off += 2 * sizeof(UnitTab);
     off = (off + 15) & ~(size_t)15;
     a.o_blob = (int)off;
     const size_t limit = (size_t)dev.smem_optin - kStaticSmem;     // the kernel's static shared memory counts too
     int nblob = 2;
     if (off + 2 * blob_cap + 1024 > limit) nblob = 1;
     if (off + (size_t)nblob * blob_cap + 1024 > limit) continue;
-    a.nblob = nblob; a.blob_cap_bytes = (int)blob_cap;
+    a.plan.nblob = nblob; a.plan.blob_cap_bytes = (int)blob_cap;
     smem = off + (size_t)nblob * blob_cap + 1024;
     break;
   }
   if (spu < 1) return -1;
-  a.spu = spu;
-  a.units = (num_graphs + spu - 1) / spu;
+  a.plan.spu = spu;
+  a.plan.units = (num_graphs + spu - 1) / spu;
   long long grid = dev.sm_count;
-  if (grid > a.units) grid = a.units;
+  if (grid > a.plan.units) grid = a.plan.units;
   if (grid < 1) return -1;
   {
     auto kp = evf::k_eval_prep;
