@@ -159,6 +159,8 @@ def encode(kind: str, params: dict, batch: dict, training: bool = False, dropout
 
 def forward(kind: str, params: dict, batch: dict, training: bool = False, dropout: float = 0.0,
             masks: Optional[list] = None) -> torch.Tensor:
+    """Class logits.  ``masks`` replaces the dropout draws: one ``[rows, H]`` multiplier per layer, then ``[B, M]`` for
+    the head, each already scaled by 1 / (1 - p)."""
     emb = encode(kind, params, batch, training, dropout, masks)
     h = F.relu(F.linear(emb, params["classifier.0.weight"], params["classifier.0.bias"]))
     h = _dropout(h, dropout, training, None if masks is None else masks[-1])
@@ -198,10 +200,11 @@ def trainable(params: dict) -> list[str]:
     return [k for k in params if not k.endswith(("running_mean", "running_var", "num_batches_tracked"))]
 
 
-def loss_and_grads(kind: str, params: dict, batch: dict, training: bool = True, dropout: float = 0.0):
-    """Mean cross-entropy (train.py:39,49) and d loss / d param for every trainable tensor."""
+def loss_and_grads(kind: str, params: dict, batch: dict, training: bool = True, dropout: float = 0.0,
+                   masks: Optional[list] = None):
+    """Mean cross-entropy (train.py:39,49) and d loss / d param for every trainable tensor.  ``masks``: as ``forward``."""
     leaves = {k: (v.detach().clone().requires_grad_(True) if k in trainable(params) else v) for k, v in params.items()}
-    logits = forward(kind, leaves, batch, training, dropout)
+    logits = forward(kind, leaves, batch, training, dropout, masks)
     loss = F.cross_entropy(logits, batch["labels"])
     names = trainable(params)
     grads = torch.autograd.grad(loss, [leaves[k] for k in names])

@@ -98,6 +98,37 @@ class Act:
         return t * sc + sh, (t * sc).abs() + sh.abs()
 
 
+def model_masks(L, H, M, rows, B, p, seed, row_base, graph_base, salt=None, sites=None):
+    """The keep multipliers (float64, 0 or keep_scale) of one training step of a classifier, in oracle/port.py's order:
+    layer l's output [rows, H] from site l (models._EncodeFn), the head's hidden units [B, M] from HEAD_SITE with one row
+    per graph (models._HeadFn).  `sites` replaces the layer sites (the negative controls)."""
+    sites = range(L) if sites is None else sites
+    out = [Act(p_drop=p, seed=seed, site=s, row_base=row_base, salt=salt).mask_and_scale(rows, H) for s in sites]
+    return out + [Act(p_drop=p, seed=seed, site=HEAD_SITE, row_base=graph_base, salt=salt).mask_and_scale(B, M)]
+
+
+M64 = 0xFFFFFFFFFFFFFFFF
+
+
+def step_salt(seed, step):
+    """The salt words (low, high) k_step_tick (optim.cu) leaves in state[2] at step `step`: splitmix64 of (seed, step)."""
+    x = (seed * 0x9E3779B97F4A7C15 + step * 0xBF58476D1CE4E5B9) & M64
+    x ^= x >> 30
+    x = (x * 0xBF58476D1CE4E5B9) & M64
+    x ^= x >> 27
+    x = (x * 0x94D049BB133111EB) & M64
+    x ^= x >> 31
+    return [x & 0xFFFFFFFF, x >> 32]
+
+
+def draw_seed(initial_seed, offset):
+    """The seed models._draw_seed cuts from a CUDA generator with this initial seed at this philox offset."""
+    x = (initial_seed * 0x9E3779B97F4A7C15 + (offset // 4 + 1) * 0xBF58476D1CE4E5B9) & M64
+    x ^= x >> 31
+    x = (x * 0x94D049BB133111EB) & M64
+    return (x ^ (x >> 29)) & 0x3FFFFFFFFFFFFFFF
+
+
 def act_fwd(act, t):
     """u = act(t) (and its magnitude); the keep mask / ReLU mask multiplier for the backward."""
     y, mag = act.pre(t)

@@ -150,8 +150,10 @@ class _float64:
         torch.set_default_dtype(self.old)
 
 
-def oracle_reference(kind, params, graphs):
-    """(fp64 truth, fp32 oracle at 8 threads) as fixture-style dicts for the package to be compared with."""
+def oracle_reference(kind, params, graphs, dropout=0.0, masks=None):
+    """(fp64 truth, fp32 oracle at 8 threads) as fixture-style dicts for the package to be compared with.  The training
+    step runs with dropout `dropout` and, when given, the keep masks `masks` (port.forward's; made in float64 and cast
+    to each run's precision, which they survive exactly: 0 or 1 / (1 - p) in fp32).  The eval outputs never drop."""
     from oracle import port
     ob = port.collate(graphs)
     out = {}
@@ -169,7 +171,8 @@ def oracle_reference(kind, params, graphs):
                     a[f"{kind}.eval.emb"] = port.encode(kind, dict(p), b).numpy()
                     a[f"{kind}.eval.logits"] = port.forward(kind, dict(p), b).numpy()
                 p2 = {k: v.clone() for k, v in p.items()}
-                logits, loss, grads = port.loss_and_grads(kind, p2, b, training=True, dropout=0.0)
+                mk = None if masks is None else [m.to(cast) for m in masks]
+                logits, loss, grads = port.loss_and_grads(kind, p2, b, training=True, dropout=dropout, masks=mk)
         finally:
             torch.set_num_threads(old_threads)
         a[f"{kind}.train.logits"], a[f"{kind}.train.loss"] = logits.numpy(), loss.numpy()

@@ -805,33 +805,28 @@ def test_dispatch_table():
 
 
 # ---- model level: ingested (real-density) and synthetic subjects against the oracle -----------------------------------
-def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hidden=64, seed=0):
-    """A training step (logits, loss, every gradient, running statistics) and eval logits against parity.oracle_reference.
-    source: ("ingest", S, N, kind, q), ("synthetic", S, N) or ("directed", sizes, F, seed) (directed_graphs).  With one all-positive feature per node the fp32 oracle
-    itself sits above 1e-5 from fp64 on some tensors (BatchNorm means of nearly constant columns): bars below 1e-5 are
-    scaled by the oracle's own distance, measured here.  Logits and loss at 1e-5.  (The "ties" recipe at 84 regions keeps
-    no edge at all: a batch without edges, which once failed to collate.)"""
-    import parity
+def model_inputs(dev, kind, source, K=2, layers=3, hidden=64, seed=0):
+    """(subjects, their SubjectStore, oracle parameters) of a model-level case.  source: ("ingest", S, N, kind, q),
+    ("synthetic", S, N), ("directed", sizes, F, seed) (directed_graphs) or ("rand", sizes, F, seed) (rand_graphs); all
+    but ingested subjects are labelled i % K.  The parameters have non-trivial BatchNorm affine and running statistics."""
     from connectome_gnn.graph import SubjectStore, pack_graphs
-    from connectome_gnn.train import CrossEntropyLoss
     from oracle import port
     _DEV["device"] = dev
     if source[0] == "ingest":
         p = ingested(*source[1:])
         graphs = packed_graphs(p)
-    elif source[0] == "directed":
-        graphs = directed_graphs(*source[1:])
-        for i, gr in enumerate(graphs):
-            gr.label = torch.tensor(i % K)
-        p = pack_graphs(graphs)
     else:
-        from connectome_gnn.synthetic import generate_dataset
-        graphs = generate_dataset(num_subjects=source[1], num_regions=source[2], seed=source[1] + source[2])
+        if source[0] == "directed":
+            graphs = directed_graphs(*source[1:])
+        elif source[0] == "rand":
+            graphs = rand_graphs(*source[1:])
+        else:
+            from connectome_gnn.synthetic import generate_dataset
+            graphs = generate_dataset(num_subjects=source[1], num_regions=source[2], seed=source[1] + source[2])
         for i, gr in enumerate(graphs):
             gr.label = torch.tensor(i % K)
         p = pack_graphs(graphs)
     store = SubjectStore(p, dev)
-    ids = np.arange(len(graphs))
     g = torch.Generator().manual_seed(seed)
     g2 = torch.Generator().manual_seed(seed + 1)
     params = port.init_params(kind, graphs[0].num_features, hidden, K, layers, generator=g)
@@ -842,6 +837,19 @@ def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hi
             params[k] = 0.05 * torch.randn(params[k].shape, generator=g2)
         if k.endswith("running_var"):
             params[k] = 1.0 + 0.2 * torch.rand(params[k].shape, generator=g2)
+    return graphs, store, params
+
+
+def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hidden=64, seed=0):
+    """A training step (logits, loss, every gradient, running statistics) and eval logits against parity.oracle_reference,
+    on the subjects of model_inputs.  With one all-positive feature per node the fp32 oracle itself sits above 1e-5 from
+    fp64 on some tensors (BatchNorm means of nearly constant columns): bars below 1e-5 are scaled by the oracle's own
+    distance, measured here (step_errors).  (The "ties" recipe at 84 regions keeps no edge at all: a batch without edges,
+    which once failed to collate.)"""
+    import parity
+    from connectome_gnn.train import CrossEntropyLoss
+    graphs, store, params = model_inputs(dev, kind, source, K, layers, hidden, seed)
+    ids = np.arange(len(graphs))
     refs = parity.oracle_reference(kind, params, graphs)
     a, a32 = refs["f64"], refs["f32"]
     m = parity.make_model(kind, a32, dev)
@@ -855,34 +863,53 @@ def run_model(dev, kind, source, fused_eval="auto", K=2, lean=True, layers=3, hi
     logits = m(b)
     loss = CrossEntropyLoss()(logits, b.labels)
     loss.backward()
-    helpers.assert_close(logits, a[f"{kind}.train.logits"], "train logits")
-    helpers.assert_close(loss, a[f"{kind}.train.loss"], "train loss")
-    # all gradients together: max(1e-5, 10 x the fp32 oracle's distance) as parity.check_against_oracle has it; each tensor
-    # within the per-tensor band of parity.py (1e-4), or 4 x the oracle's own distance where that is larger.  Measured:
-    # the first-layer GCN weight gradient at 360 dense regions is 6.4e-5 (B200) / 8.6e-5 (simulator) from fp64 where the
-    # fp32 oracle is at 1.6e-5 - a sum over 1080 rows of one all-positive feature cancels to 1e-3 of its magnitude, and
-    # the layer-level cases above hold that very kernel (k_gcn_bwd) to 5 x 2^-23 of the magnitude.
+    got = dict(logits=logits, loss=loss, grads={k: q.grad for k, q in m.named_parameters()},
+               after={k: v for k, v in m.state_dict().items() if "running" in k})
+    errs = step_errors(kind, got, a, a32)
+    over = {what: r for what, r in errs.items() if not r <= 1.0}
+    assert not over, f"error / bar over 1: {over}"
+    return max(errs.values())
+
+
+def step_errors(kind, got, a, a32, ref=None):
+    """run_model's comparison of one training step with the oracle, as {what: error / bar} (over 1 fails).  got: logits
+    (or None), loss, grads {parameter name: tensor}, after {running-statistics key: tensor}.  The bars come from the fp64
+    and fp32 oracle runs (a, a32); the errors are measured from `ref` (default a: a negative control passes an fp64 run
+    with other dropout masks).  Logits and loss at 1e-5.  All gradients together: max(1e-5, 10 x the fp32 oracle's
+    distance) as parity.check_against_oracle has it; each tensor within the per-tensor band of parity.py (1e-4), or 4 x the
+    oracle's own distance where that is larger.  Measured: the first-layer GCN weight gradient at 360 dense regions is
+    6.4e-5 (B200) / 8.6e-5 (simulator) from fp64 where the fp32 oracle is at 1.6e-5 - a sum over 1080 rows of one
+    all-positive feature cancels to 1e-3 of its magnitude, and the layer-level cases above hold that very kernel (k_gcn_bwd)
+    to 5 x 2^-23 of the magnitude."""
     import parity
-    names = [k for k, _ in m.named_parameters()]
+    ref = a if ref is None else ref
+
+    def rel(g, r):
+        g = torch.as_tensor(g).detach().cpu().double()
+        return helpers.max_rel(g, r) if bool(torch.isfinite(g).all()) else float("inf")
+    out = {}
+    if got.get("logits") is not None:
+        out["train logits"] = rel(got["logits"], ref[f"{kind}.train.logits"]) / helpers.REL_TOL
+    out["train loss"] = rel(got["loss"], ref[f"{kind}.train.loss"]) / helpers.REL_TOL
+    names = list(got["grads"])
     cat = lambda src: torch.cat([torch.as_tensor(src[f"{kind}.train.grad.{k}"]).reshape(-1).double() for k in names])
-    got_all = torch.cat([q.grad.reshape(-1) for _, q in m.named_parameters()])
     noise_all = helpers.max_rel(cat(a32), cat(a))
-    helpers.assert_close(got_all, cat(a), f"all gradients (fp32 oracle at {noise_all:.1e})", tol=max(helpers.REL_TOL, 10 * noise_all))
+    bar_all = max(helpers.REL_TOL, 10 * noise_all)
+    got_all = torch.cat([got["grads"][k].detach().cpu().reshape(-1) for k in names])
+    out[f"all gradients (fp32 oracle at {noise_all:.1e})"] = rel(got_all, cat(ref)) / bar_all
     scale = float(cat(a).abs().max())
-    worst_bar = 0.0
-    tensors = [(f"grad {k}", q.grad, f"{kind}.train.grad.{k}") for k, q in m.named_parameters()]
-    tensors += [(k, v, f"{kind}.train.after.{k}") for k, v in m.state_dict().items() if "running" in k]
-    for what, got, key in tensors:
+    tensors = [(f"grad {k}", got["grads"][k], f"{kind}.train.grad.{k}") for k in names]
+    tensors += [(k, v, f"{kind}.train.after.{k}") for k, v in got["after"].items()]
+    for what, g, key in tensors:
         noise = helpers.max_rel(a32[key], a[key])
         bar = max(helpers.REL_TOL, 4 * noise) if what.startswith("running") else max(parity.PER_TENSOR_TOL, 4 * noise)
-        worst_bar = max(worst_bar, bar)
         if kind == "gcn" and what.startswith("grad convs.") and what.endswith(".bias"):
             # analytically zero (the bias feeds BatchNorm): round-off only, held to the global gradient scale
-            err = float((got.detach().cpu().double() - torch.as_tensor(a[key]).double()).abs().max())
-            assert err <= max(helpers.REL_TOL, 10 * noise_all) * scale, (what, err, scale)
+            err = float((torch.as_tensor(g).detach().cpu().double() - torch.as_tensor(ref[key]).double()).abs().max())
+            out[what] = err / (bar_all * scale) if np.isfinite(err) else float("inf")
         else:
-            helpers.assert_close(got, a[key], f"{what} (fp32 oracle at {noise:.1e})", tol=bar)
-    return worst_bar
+            out[f"{what} (fp32 oracle at {noise:.1e})"] = rel(g, ref[key]) / bar
+    return out
 
 
 MODEL_CASES, EMU_MODEL_CASES = [], []
